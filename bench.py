@@ -2,7 +2,7 @@
 """
 bench.py — PPO-AF post-rollout update path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--workload c4|c3|c5|c1] [--impl ours|reference]
+    python bench.py --gpus N --steps K --warmup W [--workload c4|c3|c5|c1] [--impl ours|reference] [--dump-outputs DIR]
     (N > 1: launched by torch.distributed.run, one rank per GPU, NCCL)
 
 Metric (BASELINE.json): "PPO update env-steps/sec at 1/2/4/8 B200; GAE+norm GB/s vs HBM peak".
@@ -53,6 +53,9 @@ WORKLOADS = {
                actor_hidden=128, critic_hidden=128, act="leaky_relu", dist_range=1.0, lr=2e-3, B=256, epochs=10,
                max_ts_per_ep=32, shared_critic=False),
 }
+
+STATUS_KEYS = ("actor loss", "critic loss", "kl avg", "weighted entropy")   # order of status.npy (--dump-outputs)
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def peaks():
@@ -199,6 +202,20 @@ class HotPath:
     def d2h_bytes(self):
         return 64 * self.w["epochs"]
 
+    def outputs(self):
+        """What a caller of `step` receives from its last call: the status scalars, the trained actor / critic parameters,
+        the dataset's advantages, rewards-to-go and values, and the value normaliser's running statistics."""
+        sd = self.state.status_dict["pol"]
+        out = {"status": np.array([sd[k] for k in STATUS_KEYS], dtype=np.float64)}
+        for net in ("actor", "critic"):
+            for k, v in getattr(self.pol, net).state_dict().items():
+                out[f"{net}.{k}"] = v.detach().float().cpu().numpy()
+        ds = self.pol.dataset
+        for k in ("advantages", "rewards_to_go", "values"):
+            out[k] = getattr(ds, k).float().cpu().numpy()
+        out["value_normalizer"] = self.state.value_normalizers["pol"].running_stats.state.double().cpu().numpy()
+        return out
+
     def launches_per_step(self):
         """Kernels of libppoaf_b200.so launched per step (torch's own fills / copies are not counted)."""
         world = torch.distributed.get_world_size() if torch.distributed.is_initialized() else 1
@@ -259,6 +276,17 @@ def kernel_shares(hp):
         return {"total_us": total, "kernels": top}
     except Exception:
         return None
+
+
+def dump_outputs(outputs, out_dir):
+    """One `<name>.npy` per output array (float32 / float64), so that two builds can be compared array by array."""
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in outputs.items():
+        assert arr.dtype in (np.float32, np.float64), (name, arr.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
 
 
 def time_steps(fn, steps, warmup, flush):
@@ -449,16 +477,15 @@ def run_reference_arm(args, w):
     if rank != 0:
         return
     R = max(int(args.gpus), 1)
+    steps = args.steps
     if reference_available():
         from oracle import ref_bench
-        steps = max(1, min(args.steps, 5 // R if R > 1 else 5))  # bounded: a CPU step takes ~8 s x R on a 16-core host (the ranks share the cores)
         wu = 1 if args.warmup > 0 else 0
         res = ref_bench.run(w, n_ranks=R, steps=steps, warmup=wu, epochs_timed=1)
         v, secs = res["value"], res["per_step_s"]
         note = ("unmodified reference on the host cores: value = ranks x shard env-steps / slowest rank's step time; "
                 f"{steps} timed step(s) after {wu} warm-up step(s)")
     else:
-        steps = args.steps
         for _ in range(args.warmup):
             cpu_reference_sample(w, sample_minibatches=2)
         vals, tot = [], 0.0
@@ -487,7 +514,15 @@ def main():
     ap.add_argument("--workload", default="c4", choices=sorted(WORKLOADS))
     ap.add_argument("--no-microbench", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (status scalars, trained parameters, advantages, "
+                         "rewards-to-go, values, value-normaliser state) as DIR/<name>.npy; inputs are seeded, so two "
+                         "builds run with the same arguments can be compared array by array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the device path computed; the reference arm has none")
     w = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference_arm(args, w)
@@ -510,6 +545,8 @@ def main():
     sampler.start()
     ms = time_steps(lambda: hp.step(False), args.steps, args.warmup, flush)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:                      # before the passes below train the policy further
+        dump_outputs(hp.outputs(), args.dump_outputs)
     ms_e2e = time_steps(lambda: hp.step(True), args.steps, args.warmup, flush)
     h2d_ms = float(np.mean([a.elapsed_time(b) for a, b in hp.h2d_events[-args.steps:]]))   # the ring copy alone, per step
 

@@ -3,15 +3,17 @@ The drop-in boundary (SURVEY.md §8b, INTEGRATION.md): the UNMODIFIED reference 
 INTEGRATION.md edits.
 
 CPU (no GPU needed): every member the reference `PPO` touches on a policy object exists on the B200 `PPOPolicy`
-with a compatible signature — checked against the reference SOURCE (regex over ppo.py) and the reference CLASS
-(inspect.signature), so a missing member fails here instead of inside `PPO.__init__` on the GPU box.
+with a compatible signature — checked against the reference's static surface recorded in
+tests/golden/reference_surface.json (the members a regex over its ppo.py finds, the parameter names of its policy
+methods and of generate_policy), so a missing member fails here instead of inside `PPO.__init__` on the GPU.
 GPU: the real `PPO.__init__ -> rollout() -> learn()` for two iterations on a toy environment, once stock on the CPU and
 once with the four edits applied by monkey-patching, must report the same status dictionary.
 
-The reference tree is /root/reference in the build container and the git-ignored copy oracle/_ref on the GPU box
-(oracle/build_ref.py); without either these tests skip.
+The tests that execute the reference need its source tree (PPOAF_REFERENCE_ROOT, or the git-ignored copy oracle/_ref
+made by oracle/build_ref.py) and skip without it; with it, the static tests also check the record against the tree.
 """
 import inspect
+import json
 import os
 import re
 import sys
@@ -25,7 +27,12 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 sys.path.insert(0, GOLDEN)
 import ref_harness  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not ref_harness.available(), reason="reference tree (or its oracle/_ref copy) not present")
+requires_reference = pytest.mark.skipif(
+    not ref_harness.available(),
+    reason="runs the original LLNL/ppo_and_friends: set PPOAF_REFERENCE_ROOT to its source tree (or copy it to oracle/_ref "
+           "with oracle/build_ref.py)")
+with open(os.path.join(GOLDEN, "reference_surface.json")) as _fh:
+    SURFACE = json.load(_fh)
 
 # members of the reference policy that belong to subsystems outside the accelerated path (SURVEY.md §8: ICM, LSTM, MAT)
 OUT_OF_SCOPE = {"icm_lr", "intr_reward_weight", "get_agent_shared_intrinsic_rewards", "get_intrinsic_reward", "icm_model",
@@ -47,13 +54,20 @@ def _b200_policy():
                      actor_kw_args={"activation": torch.nn.LeakyReLU()}, critic_kw_args={"activation": torch.nn.LeakyReLU()})
 
 
+def _param_names(fn):
+    return [p.name for p in inspect.signature(fn).parameters.values() if p.kind != p.VAR_KEYWORD]
+
+
 def test_every_policy_member_the_reference_trainer_touches_exists():
-    ref_ppo, _ = _reference()
-    src = open(os.path.join(ref_harness.REFERENCE_ROOT, "ppo.py")).read()
-    used = set(re.findall(r"self\.policies\[[^\]]+\]\.([A-Za-z_][A-Za-z_0-9]*)", src))
-    used |= set(re.findall(r"\bpolicy\.([A-Za-z_][A-Za-z_0-9]*)", src))
+    used = set(SURFACE["trainer_policy_members"])
+    if ref_harness.available():
+        _reference()
+        src = open(os.path.join(ref_harness.REFERENCE_ROOT, "ppo.py")).read()
+        live = set(re.findall(r"self\.policies\[[^\]]+\]\.([A-Za-z_][A-Za-z_0-9]*)", src))
+        live |= set(re.findall(r"\bpolicy\.([A-Za-z_][A-Za-z_0-9]*)", src))
+        assert live - OUT_OF_SCOPE <= used, sorted(live - OUT_OF_SCOPE - used)
     assert {"have_step_constraints", "have_reset_constraints", "seed", "freeze", "get_inference_actions",
-            "apply_step_constraints", "add_episode_info", "end_episodes", "finalize_dataset"} <= used   # the regex sees them
+            "apply_step_constraints", "add_episode_info", "end_episodes", "finalize_dataset"} <= used
     pol = _b200_policy()
     missing = sorted(m for m in used - OUT_OF_SCOPE - SET_BY_FINALIZE if not hasattr(pol, m))
     assert not missing, f"PPOPolicy lacks members the reference PPO uses: {missing}"
@@ -64,32 +78,32 @@ def test_every_policy_member_the_reference_trainer_touches_exists():
 
 
 def test_policy_method_signatures_match_the_reference_class():
-    _, RefPolicy = _reference()
     from ppo_and_friends_b200.policies.ppo_policy import PPOPolicy
-    methods = ["register_agent", "finalize", "seed", "initialize_episodes", "initialize_dataset", "add_episode_info",
-               "end_episodes", "finalize_dataset", "clear_dataset", "get_rollout_actions", "get_inference_actions",
-               "evaluate", "get_critic_values", "update_learning_rate", "get_bs_clip_range", "apply_step_constraints",
-               "apply_reset_constraints", "save", "load", "direct_load", "eval", "train", "freeze", "unfreeze",
-               "update_weights"]
-    for name in methods:
-        ref_sig = inspect.signature(getattr(RefPolicy, name))
-        our_sig = inspect.signature(getattr(PPOPolicy, name))
-        ref_p = [p for p in ref_sig.parameters.values() if p.kind not in (p.VAR_KEYWORD,)]
-        our_p = [p for p in our_sig.parameters.values() if p.kind not in (p.VAR_KEYWORD,)]
-        assert [p.name for p in our_p] == [p.name for p in ref_p], (name, str(our_sig), str(ref_sig))
+    ref_methods, ref_ctor = SURFACE["policy_method_params"], set(SURFACE["policy_ctor_params"])
+    assert len(ref_methods) == 25
+    if ref_harness.available():
+        _, RefPolicy = _reference()
+        for name, params in ref_methods.items():
+            assert _param_names(getattr(RefPolicy, name)) == params, name
+        assert set(inspect.signature(RefPolicy.__init__).parameters) <= ref_ctor
+    for name, params in ref_methods.items():
+        assert _param_names(getattr(PPOPolicy, name)) == params, (name, str(inspect.signature(getattr(PPOPolicy, name))))
     # constructor: every keyword a runner file may pass is accepted under the same name
-    ref_ctor = inspect.signature(RefPolicy.__init__).parameters
     our_ctor = inspect.signature(PPOPolicy.__init__).parameters
-    assert set(ref_ctor) - {"kw_args"} <= set(our_ctor), sorted(set(ref_ctor) - set(our_ctor))
+    assert ref_ctor - {"kw_args"} <= set(our_ctor), sorted(ref_ctor - set(our_ctor))
 
 
 def test_generate_policy_hook_matches_reference_signature_and_rejects_other_classes():
-    _reference()
-    from ppo_and_friends.policies.utils import generate_policy as ref_generate
-    from ppo_and_friends.policies.mat_policy import MATPolicy
     from ppo_and_friends_b200.policies.utils import generate_policy
     from ppo_and_friends_b200.spaces import Box, Discrete
-    assert list(inspect.signature(generate_policy).parameters) == list(inspect.signature(ref_generate).parameters)
+    if ref_harness.available():
+        _reference()
+        from ppo_and_friends.policies.utils import generate_policy as ref_generate
+        assert list(inspect.signature(ref_generate).parameters) == SURFACE["generate_policy_params"]
+    assert list(inspect.signature(generate_policy).parameters) == SURFACE["generate_policy_params"]
+
+    class MATPolicy:            # stands in for the reference's policies/mat_policy.py class: rejected by name
+        pass
     box = Box(-np.inf, np.inf, (4,))
     pol = generate_policy(policy_name="p", policy_class=None, actor_observation_space=box, critic_observation_space=box,
                           action_space=Discrete(3), test_mode=False, envs_per_proc=1)
@@ -140,6 +154,7 @@ def _status(ppo):
     return {k: float(sd[k]) for k in keys}, dict(ppo.status_dict["global status"])
 
 
+@requires_reference
 @pytest.mark.gpu
 @pytest.mark.parametrize("continuous", [False, True])
 def test_unmodified_reference_trainer_runs_on_the_b200_path(monkeypatch, continuous):
@@ -171,6 +186,7 @@ def test_unmodified_reference_trainer_runs_on_the_b200_path(monkeypatch, continu
             np.testing.assert_allclose(v.cpu().numpy(), ref_sd[k].detach().numpy(), rtol=2e-3, atol=2e-5, err_msg=f"{n}/{k}")
 
 
+@requires_reference
 def test_reference_cpu_arm_runs_with_two_ranks_over_gloo():
     """bench.py's CPU arm: the unmodified reference in two worker processes, its mpi4py calls (mpi_avg_gradients,
     RunningMeanStd's allgather, broadcast_model_parameters) carried by gloo through the COMM_WORLD stand-in."""
@@ -185,6 +201,7 @@ def test_reference_cpu_arm_runs_with_two_ranks_over_gloo():
     assert two["threads_per_rank"] <= max(one["threads_per_rank"] // 2, 1)          # set_torch_threads: threads / num_procs
     assert one["value"] > 0 and two["value"] > 0
 
+@requires_reference
 @pytest.mark.timeout(600)
 def test_reference_cpu_arm_under_a_torchrun_environment(monkeypatch):
     """`bench.py --impl reference --gpus N` is launched by torchrun for N > 1: rank 0 spawns the gloo workers with the

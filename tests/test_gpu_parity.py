@@ -724,3 +724,40 @@ def test_checkpoint_resume_from_reference_state_matches_reference_epoch(tmp_path
     vn.load_info(str(out))
     assert np.allclose(vn.running_stats.mean, before[0]) and np.allclose(vn.running_stats.variance, before[1])
     assert vn.running_stats.count == before[2]
+
+
+# ----------------------------------------------------------------------------------------- bench.py --dump-outputs
+def test_bench_dump_outputs_are_what_the_last_timed_step_returned(tmp_path):
+    """`bench.py --dump-outputs`, run as a program, writes what its last timed step of the launch chain left to the
+    caller, before the e2e and fused passes train the policy further: the status scalars, every actor / critic parameter,
+    the dataset's advantages / rewards-to-go / values and the value normaliser's state.  The same seeded workload stepped
+    warm-up + steps times in this process must give every one of those arrays bit for bit."""
+    import os
+    import subprocess
+    import sys
+    import bench
+    root = os.path.dirname(os.path.abspath(bench.__file__))
+    out = tmp_path / "dump"
+    warmup, steps = 3, 2
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "c1", "--steps", str(steps),
+                        "--warmup", str(warmup), "--no-microbench", "--no-cpu-baseline", "--dump-outputs", str(out)],
+                       cwd=root, capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    w = bench.WORKLOADS["c1"]
+    ro, pol = bench.build_workload(w, 0, "cuda:0")
+    hp = bench.HotPath(w, ro, pol)
+    for _ in range(warmup + steps):
+        hp.step(False)
+    torch.cuda.synchronize()
+    sd = hp.state.status_dict["pol"]
+    want = {"status": np.array([sd[k] for k in ("actor loss", "critic loss", "kl avg", "weighted entropy")])}
+    for net in ("actor", "critic"):
+        for k, v in getattr(pol, net).state_dict().items():
+            want[f"{net}.{k}"] = v.cpu().numpy()
+    for k in ("advantages", "rewards_to_go", "values"):
+        want[k] = getattr(pol.dataset, k).cpu().numpy()
+    want["value_normalizer"] = hp.state.value_normalizers["pol"].running_stats.state.cpu().numpy()
+    assert sorted(os.listdir(out)) == sorted(n + ".npy" for n in want)
+    for n, ref in want.items():
+        got = np.load(out / (n + ".npy"))
+        assert got.dtype == ref.dtype and np.array_equal(got, ref), n

@@ -376,3 +376,13 @@ def test_ctypes_structs_match_the_c_header(tmp_path):
     want = [C.sizeof(_lib.MlpDesc), C.sizeof(_lib.UpdateCfg), C.sizeof(_lib.UpdateBufs), _lib.UpdateBufs.n_flat.offset,
             _lib.UpdateBufs.batch.offset, _lib.UpdateBufs.n_mirror.offset, _lib.UpdateBufs.mirror_delta.offset]
     assert got == want, (got, want)
+
+
+def test_bench_rejects_arguments_it_would_not_honour(tmp_path):
+    """`--steps` is the number of timed steps (no fewer than one), and `--dump-outputs` has nothing to write for the
+    reference arm: both are refused before any work starts."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "dump")]):
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), *args], capture_output=True, text=True)
+        assert r.returncode == 2 and "error:" in r.stderr, (args, r.stderr[-500:])
+    assert not (tmp_path / "dump").exists()
