@@ -32,8 +32,13 @@ extern "C" {
 
 /* activation ids (hidden layers of FeedForwardNetwork, networks/utils.py:160-183) */
 enum { PPOAF_ACT_IDENTITY = 0, PPOAF_ACT_RELU = 1, PPOAF_ACT_LEAKY_RELU = 2, PPOAF_ACT_TANH = 3 };
-/* action heads (networks/distributions.py) */
-enum { PPOAF_HEAD_GAUSSIAN_TANH = 0, PPOAF_HEAD_CATEGORICAL = 1 };
+/* action heads (networks/distributions.py).  PPOAF_HEAD_MULTI_CATEGORICAL (MultiDiscrete action spaces,
+ * MultiCategoricalDistribution :272-438) is a restatement, not pinned by a reference golden: softmax over the whole
+ * actor output row, then one torch Categorical(probs) per section of the row (renormalised, clamped to [eps, 1-eps]);
+ * log-prob and entropy are the sums over the sections.  The sections are described by a 64-bit table of section
+ * ends (bit c set: actor output c is the last of its section), so the row holds at most 64 outputs; nvec must be
+ * 1-D with start = 0 and every entry >= 1. */
+enum { PPOAF_HEAD_GAUSSIAN_TANH = 0, PPOAF_HEAD_CATEGORICAL = 1, PPOAF_HEAD_MULTI_CATEGORICAL = 2 };
 
 int         ppoaf_abi_version(void);
 const char* ppoaf_last_error(void);
@@ -146,7 +151,8 @@ enum {
 typedef struct {
     ppoaf_mlp_desc actor, critic;
     int32_t head;                 /* PPOAF_HEAD_*                                                    */
-    int32_t act_dim;              /* stored action width: Da (Gaussian) or 1 (Categorical index)    */
+    int32_t act_dim;              /* stored action width: Da (Gaussian), 1 (Categorical index) or the
+                                     number of sections (Multi-categorical, one int64 index each)   */
     int32_t use_huber;            /* nn.HuberLoss(delta=10) instead of MSE (ppo.py:2416-2419)       */
     int32_t normalize_adv;        /* ppo.py:2325-2333                                               */
     int32_t normalize_values;     /* ppo.py:2299-2303                                               */
@@ -154,7 +160,10 @@ typedef struct {
     int32_t world_size;           /* ranks whose gradients the caller all-reduces between grads/apply */
     int32_t reserved[1];
     float   min_std;              /* GaussianDistribution min_std (networks/distributions.py:453)   */
-    float   reserved_f[3];
+    uint32_t section_ends[2];     /* Multi-categorical section table, 64-bit mask (lo, hi): bit c set =
+                                     actor output c ends a section.  Nonzero, highest bit = outputs - 1,
+                                     popcount = act_dim.  Read by no other head (leave it zero).      */
+    float   reserved_f[1];
 } ppoaf_update_cfg;
 
 /* Flat parameter layout (shared by params / grads / Adam m / Adam v): for each net, for each
@@ -258,6 +267,22 @@ int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t pred_dim, 
 int ppoaf_head_sample(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std, float min_std,
                       const float* noise, const float* dist_min, const float* dist_max, int32_t act_dim,
                       int32_t n_rows, void* raw_action_out, void* action_out, float* log_prob_out, void* stream);
+
+/* The multi-categorical head (PPOAF_HEAD_MULTI_CATEGORICAL) on its own; (section_ends_lo, section_ends_hi) is the
+ * section table of ppoaf_update_cfg.section_ends, n_sections its popcount.
+ * _evaluate: log-prob of actions_i64 [n_rows, n_sections] (index inside each section) and entropy, from the actor's
+ *   logits actor_out [n_rows, pred_dim] (PPOPolicy.evaluate).
+ * _sample: rollout-time sampling from probs [n_rows, pred_dim] (ppoaf_mlp_forward with softmax_out = 1).  `noise` holds
+ *   the host generator's Exp(1) draws in the order per-section Categorical sampling consumes them: section after
+ *   section, a contiguous [n_rows, n_k] block each, so section k starting at output o_k reads
+ *   noise[n_rows * o_k + i * n_k + j].  In each section a_k = first argmax(p~_k / q_k) (aten multinomial's one-sample
+ *   path).  Outputs actions_out_i64 [n_rows, n_sections] and the summed log-prob [n_rows]. */
+int ppoaf_multi_categorical_evaluate(const float* actor_out, int32_t pred_dim, uint32_t section_ends_lo,
+                                     uint32_t section_ends_hi, const int64_t* actions_i64, int32_t n_sections,
+                                     int32_t n_rows, float* log_prob_out, float* entropy_out, void* stream);
+int ppoaf_multi_categorical_sample(const float* probs, int32_t pred_dim, uint32_t section_ends_lo,
+                                   uint32_t section_ends_hi, const float* noise, int32_t n_sections, int32_t n_rows,
+                                   int64_t* actions_out_i64, float* log_prob_out, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * P5  Gradient all-reduce over NVLink peer memory FUSED with clip + Adam (R > 1 on one node).

@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(_HERE, "csrc", "libppoaf_b200.so")
 
 MAX_LAYERS = 8
 ACT_IDS = {"identity": 0, "relu": 1, "leaky_relu": 2, "tanh": 3}
-HEAD_GAUSSIAN_TANH, HEAD_CATEGORICAL = 0, 1
+HEAD_GAUSSIAN_TANH, HEAD_CATEGORICAL, HEAD_MULTI_CATEGORICAL = 0, 1, 2
 
 HP = dict(LR=0, ENTROPY_WEIGHT=1, SURR_CLIP=2, GRAD_CLIP=3, KL_WEIGHT=4, VF_CLIP=5, BETA1=6, BETA2=7,
           ADAM_EPS=8, INV_WORLD=9, COUNT=16)
@@ -40,7 +40,7 @@ class UpdateCfg(C.Structure):
     _fields_ = [("actor", MlpDesc), ("critic", MlpDesc), ("head", C.c_int32), ("act_dim", C.c_int32),
                 ("use_huber", C.c_int32), ("normalize_adv", C.c_int32), ("normalize_values", C.c_int32),
                 ("vf_clip_enabled", C.c_int32), ("world_size", C.c_int32), ("reserved", C.c_int32 * 1), ("min_std", C.c_float),
-                ("reserved_f", C.c_float * 3)]
+                ("section_ends", C.c_uint32 * 2), ("reserved_f", C.c_float * 1)]
 
 
 class UpdateBufs(C.Structure):
@@ -88,6 +88,8 @@ _SIGNATURES = {
     "ppoaf_mlp_forward": (C.c_int, [C.POINTER(MlpDesc), _P, _P, _P, C.c_int32, C.c_int, _P, _P, C.c_size_t, _P]),
     "ppoaf_head_evaluate": (C.c_int, [C.c_int32, _P, C.c_int32, _P, C.c_float, _P, C.c_int32, C.c_int32, _P, _P, _P]),
     "ppoaf_head_sample": (C.c_int, [C.c_int32, _P, C.c_int32, _P, C.c_float, _P, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P]),
+    "ppoaf_multi_categorical_evaluate": (C.c_int, [_P, C.c_int32, C.c_uint32, C.c_uint32, _P, C.c_int32, C.c_int32, _P, _P, _P]),
+    "ppoaf_multi_categorical_sample": (C.c_int, [_P, C.c_int32, C.c_uint32, C.c_uint32, _P, C.c_int32, C.c_int32, _P, _P, _P]),
     "ppoaf_nvls_ctrl_bytes": (C.c_size_t, []),
     "ppoaf_nvls_flag_block_bytes": (C.c_size_t, []),
     "ppoaf_nvls_allreduce_adam": (C.c_int, [_P, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int32, C.c_int32, _P, _P, _P,
@@ -152,6 +154,16 @@ def ptr(t):
 def stream_ptr(stream=None):
     s = torch.cuda.current_stream() if stream is None else stream
     return C.c_void_p(s.cuda_stream)
+
+
+def section_ends(nvec):
+    """The multi-categorical section table of ppoaf_update_cfg: bit c set = actor output c ends a section."""
+    mask = 0
+    end = -1
+    for n in nvec:
+        end += int(n)
+        mask |= 1 << end
+    return mask
 
 
 def param_layout(desc, log_std_dim=0):

@@ -1405,6 +1405,7 @@ static int build_plan(const ppoaf_update_cfg* cfg, const ppoaf_update_bufs* b, i
     a.head = cfg->head;
     a.act_dim = cfg->act_dim;
     a.pred_dim = cfg->actor.dims[L];
+    a.section_ends = cfg_section_ends(cfg);
     a.use_huber = cfg->use_huber;
     a.normalize_adv = cfg->normalize_adv;
     a.normalize_values = cfg->normalize_values;
@@ -1484,10 +1485,9 @@ extern "C" size_t ppoaf_ppo_fused_workspace_bytes(const ppoaf_update_cfg* cfg, i
 
 extern "C" int ppoaf_ppo_fused_steps(const ppoaf_update_cfg* cfg, const ppoaf_update_bufs* b, int32_t n_steps, void* stream) {
     PPOAF_CHECK_ARG(cfg != nullptr && b != nullptr, "ppoaf_ppo_fused_steps: null argument");
-    if (check_mlp_desc(&cfg->actor, "ppoaf_ppo_fused_steps") || check_mlp_desc(&cfg->critic, "ppoaf_ppo_fused_steps")) return 1;
+    if (check_cfg(cfg, "ppoaf_ppo_fused_steps")) return 1;
     const char* why = fused::unsupported_reason(cfg);
     PPOAF_CHECK_ARG(why == nullptr, "ppoaf_ppo_fused_steps: not supported: %s", why ? why : "");
-    PPOAF_CHECK_ARG(cfg->critic.dims[cfg->critic.n_layers] == 1, "ppoaf_ppo_fused_steps: critic output width must be 1");
     PPOAF_CHECK_ARG(b->batch >= 2 && b->batch <= b->batch_size && b->n_flat > 0 && n_steps >= 1,
                     "ppoaf_ppo_fused_steps: bad batch sizes (one-row minibatches are skipped by the caller)");
     PPOAF_CHECK_ARG(n_steps == 1 || b->batch == b->batch_size, "ppoaf_ppo_fused_steps: several steps need full minibatches");

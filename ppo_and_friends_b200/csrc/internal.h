@@ -63,6 +63,7 @@ struct LossArgs {
     float* partials;             // workspace
     unsigned int* ticket;        // zero-initialised, self-resetting
     int head, act_dim, pred_dim;
+    unsigned long long section_ends;   // PPOAF_HEAD_MULTI_CATEGORICAL: bit c set = actor output c ends a section
     int use_huber, normalize_adv, normalize_values, vf_clip_enabled;
     float min_std;
     // fused head layers (loss_head_fusable): the last Linear of both networks and its dX are computed by the loss
@@ -88,6 +89,13 @@ struct LossArgs {
     int d_actor_ld, d_critic_ld;
 };
 bool loss_head_fusable(int pred_dim, int Ha, int Hc, int vf_clip_enabled);
+// a multi-categorical section table that fits the row: nonzero, last section ends at pred_dim - 1, n_sections ends
+bool section_table_ok(unsigned long long section_ends, int pred_dim, int n_sections);
+inline unsigned long long cfg_section_ends(const ppoaf_update_cfg* cfg) {
+    return (uint64_t(cfg->section_ends[1]) << 32) | cfg->section_ends[0];
+}
+// step.cu: validates an update configuration (networks, head, section table); 0 = ok
+int check_cfg(const ppoaf_update_cfg* cfg, const char* who);
 size_t loss_workspace_bytes(int max_batch, int act_dim);
 int launch_ppo_loss(const LossArgs& a, cudaStream_t s);
 

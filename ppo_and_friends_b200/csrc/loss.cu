@@ -12,6 +12,11 @@
 
 namespace ppoaf {
 
+bool section_table_ok(unsigned long long section_ends, int pred_dim, int n_sections) {
+    return pred_dim >= 1 && pred_dim <= kMaxAct && section_ends != 0 && 63 - __builtin_clzll(section_ends) == pred_dim - 1 &&
+           __builtin_popcountll(section_ends) == n_sections;
+}
+
 bool loss_head_fusable(int pred_dim, int Ha, int Hc, int vf_clip_enabled) {
     auto ok = [](int H) { return H % 4 == 0 && H >= 4 && H <= 4 * kG * kFusedMaxChunks; };
     return pred_dim <= kFusedMaxPred && ok(Ha) && ok(Hc) && !vf_clip_enabled;
@@ -548,5 +553,104 @@ extern "C" int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t
     head_evaluate_kernel<<<(n_rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
         head, actor_out, pred_dim, log_std, min_std, actions, act_dim, n_rows, log_prob_out, entropy_out);
     PPOAF_CHECK_LAUNCH("ppoaf_head_evaluate");
+    return 0;
+}
+
+// ---- the multi-categorical head on its own (PPOAF_HEAD_MULTI_CATEGORICAL): one thread per row, sections in order ----
+namespace ppoaf {
+
+__global__ void multi_categorical_evaluate_kernel(const float* __restrict__ actor_out, int pred_dim,
+                                                  unsigned long long ends, const int64_t* __restrict__ actions,
+                                                  int n_sections, int n_rows, float* __restrict__ lp_out,
+                                                  float* __restrict__ ent_out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_rows) return;
+    const float* pred = actor_out + int64_t(i) * pred_dim;
+    const int64_t* act = actions + int64_t(i) * n_sections;
+    float mx = pred[0];
+    for (int c = 1; c < pred_dim; ++c) mx = fmaxf(mx, pred[c]);
+    float se = 0.f;
+    for (int c = 0; c < pred_dim; ++c) se += expf(pred[c] - mx);
+    float lp = 0.f, h = 0.f;
+    for (int o = 0, k = 0, c = 0; c < pred_dim; ++c) {
+        if (!((ends >> c) & 1ull)) continue;
+        float S = 0.f;                                            // section k = columns o .. c
+        for (int d = o; d <= c; ++d) S += expf(pred[d] - mx) / se;
+        const int a = int(act[k]);
+        for (int d = o; d <= c; ++d) {
+            const float pn = (expf(pred[d] - mx) / se) / S;
+            const float l = logf(fminf(fmaxf(pn, kCatEps), 1.f - kCatEps));
+            h += pn * l;
+            if (d - o == a) lp += l;
+        }
+        o = c + 1;
+        ++k;
+    }
+    lp_out[i] = lp;
+    if (ent_out) ent_out[i] = -h;
+}
+
+// probs: the softmax of the whole row; noise: section k's Exp(1) block [n_rows, n_k] starts at n_rows * o_k
+__global__ void multi_categorical_sample_kernel(const float* __restrict__ probs, int pred_dim, unsigned long long ends,
+                                                const float* __restrict__ noise, int n_sections, int n_rows,
+                                                int64_t* __restrict__ act_out, float* __restrict__ lp_out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_rows) return;
+    const float* p = probs + int64_t(i) * pred_dim;
+    float lp = 0.f;
+    for (int o = 0, k = 0, c = 0; c < pred_dim; ++c) {
+        if (!((ends >> c) & 1ull)) continue;
+        const int nk = c - o + 1;
+        const float* q = noise + int64_t(n_rows) * o + int64_t(i) * nk;
+        float S = 0.f;
+        for (int d = 0; d < nk; ++d) S += p[o + d];
+        int best = 0;
+        float best_v = -INFINITY, best_p = 0.f;
+        for (int d = 0; d < nk; ++d) {
+            const float pn = p[o + d] / S;
+            const float v = pn / q[d];
+            if (v > best_v) { best_v = v; best = d; best_p = pn; }        // first maximum, like argmax
+        }
+        act_out[int64_t(i) * n_sections + k] = best;
+        lp += logf(fminf(fmaxf(best_p, kCatEps), 1.f - kCatEps));
+        o = c + 1;
+        ++k;
+    }
+    lp_out[i] = lp;
+}
+
+}  // namespace ppoaf
+
+extern "C" int ppoaf_multi_categorical_evaluate(const float* actor_out, int32_t pred_dim, uint32_t section_ends_lo,
+                                                uint32_t section_ends_hi, const int64_t* actions_i64, int32_t n_sections,
+                                                int32_t n_rows, float* log_prob_out, float* entropy_out, void* stream) {
+    using namespace ppoaf;
+    const unsigned long long ends = (uint64_t(section_ends_hi) << 32) | section_ends_lo;
+    PPOAF_CHECK_ARG(section_table_ok(ends, pred_dim, n_sections),
+                    "ppoaf_multi_categorical_evaluate: bad section table for %d outputs / %d sections (at most %d outputs)",
+                    pred_dim, n_sections, kMaxAct);
+    PPOAF_CHECK_ARG(n_rows >= 0, "ppoaf_multi_categorical_evaluate: n_rows < 0");
+    if (n_rows == 0) return 0;
+    multi_categorical_evaluate_kernel<<<(n_rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
+        actor_out, pred_dim, ends, actions_i64, n_sections, n_rows, log_prob_out, entropy_out);
+    PPOAF_CHECK_LAUNCH("ppoaf_multi_categorical_evaluate");
+    return 0;
+}
+
+extern "C" int ppoaf_multi_categorical_sample(const float* probs, int32_t pred_dim, uint32_t section_ends_lo,
+                                              uint32_t section_ends_hi, const float* noise, int32_t n_sections,
+                                              int32_t n_rows, int64_t* actions_out_i64, float* log_prob_out,
+                                              void* stream) {
+    using namespace ppoaf;
+    const unsigned long long ends = (uint64_t(section_ends_hi) << 32) | section_ends_lo;
+    PPOAF_CHECK_ARG(section_table_ok(ends, pred_dim, n_sections),
+                    "ppoaf_multi_categorical_sample: bad section table for %d outputs / %d sections (at most %d outputs)",
+                    pred_dim, n_sections, kMaxAct);
+    PPOAF_CHECK_ARG(n_rows >= 0, "ppoaf_multi_categorical_sample: n_rows < 0");
+    if (n_rows == 0) return 0;
+    PPOAF_CHECK_ARG(noise != nullptr, "ppoaf_multi_categorical_sample: noise is required");
+    multi_categorical_sample_kernel<<<(n_rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
+        probs, pred_dim, ends, noise, n_sections, n_rows, actions_out_i64, log_prob_out);
+    PPOAF_CHECK_LAUNCH("ppoaf_multi_categorical_sample");
     return 0;
 }

@@ -51,6 +51,54 @@ __device__ __forceinline__ float group_max(float v) {
     return v;
 }
 
+// Multi-categorical section table (bit c set: column c ends a section).  For a column c < 64: first column of its
+// section, last column of its section (-1 past the last section) and the section's index.
+__device__ __forceinline__ int section_start(unsigned long long ends, int c) {
+    const unsigned long long below = ends & ((1ull << c) - 1ull);
+    return below ? 64 - __clzll((long long)below) : 0;
+}
+__device__ __forceinline__ int section_end(unsigned long long ends, int c) { return __ffsll((long long)(ends >> c << c)) - 1; }
+__device__ __forceinline__ int section_index(unsigned long long ends, int c) { return __popcll(ends & ((1ull << c) - 1ull)); }
+
+// Per-section sums over the kG lanes of one sample: out[k] = sum of v over the section that column gl + k kG belongs
+// to (st / en: first / last column of that section).  A segmented inclusive scan of each half of the row (a lane adds
+// its neighbour's partial sum only while that neighbour lies in the same section), the second half continuing the
+// section column 31 leaves open, then every lane reads the scan at its section's last column.  A table of one section
+// takes the Categorical head's whole-row sum instead (same order), so MultiDiscrete([n]) reproduces Discrete(n) exactly.
+__device__ __forceinline__ void section_sum(const float (&v)[kPerLane], const int (&st)[kPerLane],
+                                            const int (&en)[kPerLane], int gl, bool one_section,
+                                            float (&out)[kPerLane]) {
+    if (one_section) {
+        float t = 0.f;
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) t += v[k];
+        t = group_sum(t);
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) out[k] = t;
+        return;
+    }
+    float x[kPerLane];
+#pragma unroll
+    for (int k = 0; k < kPerLane; ++k) x[k] = v[k];
+#pragma unroll
+    for (int o = 1; o < kG; o <<= 1) {
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) {
+            const float y = __shfl_up_sync(kFull, x[k], o);
+            if (gl >= o && gl - o + k * kG >= st[k]) x[k] += y;
+        }
+    }
+    static_assert(kPerLane == 2, "the carry below joins two halves of the row");
+    const float carry = __shfl_sync(kFull, x[0], kG - 1);
+    if (st[1] < kG) x[1] += carry;
+#pragma unroll
+    for (int k = 0; k < kPerLane; ++k) {
+        const int e = en[k] < 0 ? 0 : en[k];
+        const float lo = __shfl_sync(kFull, x[0], e & (kG - 1)), hi = __shfl_sync(kFull, x[1], e & (kG - 1));
+        out[k] = e >= kG ? hi : lo;
+    }
+}
+
 // Action-head part of the loss for one sample shared by the 32 lanes of a warp (lane gl owns dims gl, gl + 32):
 // log-prob, entropy, ratio, clipped surrogate and their gradients w.r.t. the head outputs (written to dpred, and
 // to sdp when the head layer itself is fused) and w.r.t. std (dsd).  Lane 0 receives the sample's scalars in sc.
@@ -113,6 +161,99 @@ __device__ __forceinline__ void actor_head_loss(const LossArgs& a, bool gaussian
                 if constexpr (FUSED) sdp[d] = gd;
                 // dlp/dsd = z^2/sd^3 - 1/sd ; dH/dsd = 1/sd
                 dsd[k] = g_lp * on[k] * ((z[k] * z[k]) / (var * sd) - 1.f / sd) + g_ent * one[k] * (1.f / sd);
+            }
+        }
+    } else if (a.head == PPOAF_HEAD_MULTI_CATEGORICAL) {
+        // softmax over the whole row (as for Categorical), then one Categorical(probs) per section: the Categorical
+        // arithmetic with the renormaliser S and the sum of G p taken per section (section_sum)
+        const unsigned long long ends = a.section_ends;
+        const bool one_section = (ends & (ends - 1ull)) == 0ull;
+        const int n = a.pred_dim;
+        const int64_t* acts = reinterpret_cast<const int64_t*>(a.raw_actions) + j * a.act_dim;
+        float p[kPerLane], pn[kPerLane], lg[kPerLane];
+        int st[kPerLane], en[kPerLane];
+        bool hit[kPerLane];
+        float mx = -INFINITY;
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) {
+            const int c = gl + k * kG;
+            st[k] = section_start(ends, c);
+            en[k] = section_end(ends, c);
+            p[k] = (c < n) ? pred[c] : -INFINITY;
+            hit[k] = live && c < n && c - st[k] == int(acts[section_index(ends, c)]);
+            if (c < n) bad_value = fmaxf(bad_value, isnan(p[k]) ? 1.f : 0.f);
+            mx = fmaxf(mx, p[k]);
+        }
+        mx = group_max(mx);
+        float se = 0.f;
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) {
+            const int c = gl + k * kG;
+            p[k] = (c < n) ? expf(p[k] - mx) : 0.f;
+            se += p[k];
+        }
+        se = group_sum(se);
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) p[k] = p[k] / se;
+        float S[kPerLane];
+        section_sum(p, st, en, gl, one_section, S);
+        float h = 0.f, lpa = 0.f;
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) {
+            const int c = gl + k * kG;
+            pn[k] = lg[k] = 0.f;
+            if (c < n) {
+                pn[k] = p[k] / S[k];
+                lg[k] = logf(fminf(fmaxf(pn[k], kCatEps), 1.f - kCatEps));
+                h += pn[k] * lg[k];
+                if (hit[k]) lpa += lg[k];
+            }
+        }
+        lp = group_sum(lpa);                                                    // sums over the sections
+        ent = -group_sum(h);
+        const float ratio = expf(lp - lp_old);
+        const float s1 = ratio * adv, s2 = fminf(fmaxf(ratio, clip_lo), clip_hi) * adv;
+        const float g_lp = (s1 <= s2) ? -adv * ratio * inv_b : 0.f;
+        const float g_ent = -w_ent * inv_b;
+        if (gl == 0 && live) {
+            sc[LS_ACTOR] = -fminf(s1, s2);
+            sc[LS_KL] = lp_old - lp;
+            sc[LS_ENTROPY] = ent;
+            sc[LS_BAD_RATIO] = (isnan(ratio) || isinf(ratio)) ? 1.f : 0.f;
+        }
+        // G_c = dL/d pn_c ; pn = p / S_k ; p = softmax(z)
+        float G[kPerLane], gp[kPerLane];
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) {
+            const int c = gl + k * kG;
+            G[k] = gp[k] = 0.f;
+            if (c < n) {
+                const float q = fminf(fmaxf(pn[k], kCatEps), 1.f - kCatEps);
+                const float mask = (pn[k] >= kCatEps && pn[k] <= 1.f - kCatEps) ? 1.f : 0.f;
+                const float dlg = (hit[k] ? g_lp : 0.f) + g_ent * (-pn[k]);
+                G[k] = g_ent * (-lg[k]) + dlg * mask / q;
+                gp[k] = G[k] * p[k];
+            }
+        }
+        float gdotp[kPerLane];
+        section_sum(gp, st, en, gl, one_section, gdotp);
+        float dpdotp = 0.f;
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) {
+            const int c = gl + k * kG;
+            if (c < n) {
+                G[k] = G[k] / S[k] - gdotp[k] / (S[k] * S[k]);                  // dL/dp_c
+                dpdotp += G[k] * p[k];
+            }
+        }
+        dpdotp = group_sum(dpdotp);
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) {
+            const int c = gl + k * kG;
+            if (c < n && live) {
+                const float gd = p[k] * (G[k] - dpdotp);
+                dpred[c] = gd;
+                if constexpr (FUSED) sdp[c] = gd;
             }
         }
     } else {

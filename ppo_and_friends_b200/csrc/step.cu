@@ -96,14 +96,19 @@ static void carve(const ppoaf_update_cfg* cfg, int max_batch, char* base, StepSc
     out->total = off;
 }
 
-static int check_cfg(const ppoaf_update_cfg* cfg, const char* who) {
+int check_cfg(const ppoaf_update_cfg* cfg, const char* who) {
     PPOAF_CHECK_ARG(cfg != nullptr, "%s: null cfg", who);
     if (check_mlp_desc(&cfg->actor, who) || check_mlp_desc(&cfg->critic, who)) return 1;
     PPOAF_CHECK_ARG(cfg->critic.dims[cfg->critic.n_layers] == 1, "%s: critic output width must be 1", who);
-    PPOAF_CHECK_ARG(cfg->head == PPOAF_HEAD_GAUSSIAN_TANH || cfg->head == PPOAF_HEAD_CATEGORICAL, "%s: unknown head", who);
+    PPOAF_CHECK_ARG(cfg->head == PPOAF_HEAD_GAUSSIAN_TANH || cfg->head == PPOAF_HEAD_CATEGORICAL ||
+                    cfg->head == PPOAF_HEAD_MULTI_CATEGORICAL, "%s: unknown head", who);
     if (cfg->head == PPOAF_HEAD_GAUSSIAN_TANH)
         PPOAF_CHECK_ARG(cfg->actor.dims[cfg->actor.n_layers] == cfg->act_dim,
                         "%s: Gaussian actor output width must equal act_dim", who);
+    else if (cfg->head == PPOAF_HEAD_MULTI_CATEGORICAL)
+        PPOAF_CHECK_ARG(section_table_ok(cfg_section_ends(cfg), cfg->actor.dims[cfg->actor.n_layers], cfg->act_dim),
+                        "%s: bad multi-categorical section table (must be nonzero, its highest set bit must be the last "
+                        "actor output, at most 64 outputs, and it must have act_dim = %d bits)", who, cfg->act_dim);
     else
         PPOAF_CHECK_ARG(cfg->act_dim == 1, "%s: Categorical actions are stored as one int64 index", who);
     return 0;
@@ -246,6 +251,7 @@ extern "C" int ppoaf_ppo_minibatch_grads(const ppoaf_update_cfg* cfg, const ppoa
     a.head = cfg->head;
     a.act_dim = cfg->act_dim;
     a.pred_dim = cfg->actor.dims[L[0]];
+    a.section_ends = cfg_section_ends(cfg);
     a.use_huber = cfg->use_huber;
     a.normalize_adv = cfg->normalize_adv;
     a.normalize_values = cfg->normalize_values;

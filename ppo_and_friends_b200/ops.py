@@ -163,6 +163,29 @@ def head_sample(head, actor_out, log_std, noise, min_std=0.01, dist_min=None, di
     return raw, act, lp
 
 
+def multi_categorical_evaluate(actor_out, section_ends, actions, want_entropy=True):
+    """(log_prob, entropy) [n] of int64 actions [n, n_sections] under the multi-categorical head on logits actor_out."""
+    n, pred = actor_out.shape
+    lp = torch.empty(n, dtype=torch.float32, device=actor_out.device)
+    ent = torch.empty(n, dtype=torch.float32, device=actor_out.device) if want_entropy else None
+    check(load().ppoaf_multi_categorical_evaluate(ptr(actor_out), pred, section_ends & 0xFFFFFFFF, section_ends >> 32,
+                                                  ptr(actions), actions.shape[1], n, ptr(lp), ptr(ent), stream_ptr()),
+          "ppoaf_multi_categorical_evaluate")
+    return lp, ent
+
+
+def multi_categorical_sample(probs, section_ends, noise, n_sections):
+    """(int64 actions [n, n_sections], log_prob [n]) from softmax probs and host-drawn Exp(1) noise laid out section after
+    section (see ppoaf_multi_categorical_sample)."""
+    n, pred = probs.shape
+    act = torch.empty((n, n_sections), dtype=torch.int64, device=probs.device)
+    lp = torch.empty(n, dtype=torch.float32, device=probs.device)
+    check(load().ppoaf_multi_categorical_sample(ptr(probs), pred, section_ends & 0xFFFFFFFF, section_ends >> 32, ptr(noise),
+                                                int(n_sections), n, ptr(act), ptr(lp), stream_ptr()),
+          "ppoaf_multi_categorical_sample")
+    return act, lp
+
+
 def clip_adam_step(params, grads, m, v, adam_step, hparams, n_actor, n_critic):
     lib = load()
     ws = _workspace("adam", 1 << 16, params.device)

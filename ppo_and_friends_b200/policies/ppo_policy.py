@@ -14,7 +14,10 @@ Changed on purpose: there are no per-segment EpisodeInfo objects and no autograd
 into a packed device ring, segments into a table, and `update_weights(actor_loss, critic_loss)` has
 no counterpart because the losses never exist as tensors — the fused step in ppo.py
 (`ppo_batch_train`) replaces `PPO._ppo_batch_train` + `evaluate` + `update_weights` as one unit.
-Out of scope (raise): LSTM networks, ICM, MAT, Bernoulli/MultiCategorical/Mixed action heads.
+MultiDiscrete action spaces take a multi-categorical head (reference MultiCategoricalDistribution,
+networks/distributions.py:272-438, restated: softmax over the whole actor output, one Categorical per section, log-prob
+and entropy summed over the sections); `nvec` must be 1-D with `start` = 0, every entry >= 1 and sum(nvec) <= 64.
+Out of scope (raise): LSTM networks, ICM, MAT, Bernoulli/Mixed action heads.
 """
 import os
 
@@ -112,9 +115,9 @@ class PPOPolicy:
         self.action_dtype = space_dtype_str(action_space)
         if self.action_dtype == "unknown":
             abort(f"ERROR: unknown action type: {type(action_space)} with dtype {getattr(action_space, 'dtype', None)}.")
-        if self.action_dtype not in ("continuous", "discrete"):
+        if self.action_dtype not in ("continuous", "discrete", "multi-discrete"):
             abort(f"ERROR: {self.action_dtype} action heads are outside the B200 update path "
-                  "(Gaussian and Categorical only, SURVEY.md §2 row 8).")
+                  "(Gaussian, Categorical and MultiCategorical only, SURVEY.md §2 row 8).")
         rank_print("{} policy using {} actions.".format(self.name, self.action_dtype))
 
         self.have_bootstrap_clip = bootstrap_clip is not None
@@ -126,6 +129,22 @@ class PPOPolicy:
         if self.action_dtype == "discrete":
             self.action_dim = 1
             self.action_pred_size = int(action_space.n)
+        elif self.action_dtype == "multi-discrete":
+            nvec = np.asarray(action_space.nvec)
+            start = getattr(action_space, "start", None)
+            if nvec.ndim != 1 or nvec.size == 0:
+                abort(f"ERROR: MultiDiscrete nvec must be a non-empty 1-D array on the B200 path, got shape {nvec.shape}.")
+            if start is not None and np.any(np.asarray(start) != 0):
+                abort("ERROR: MultiDiscrete spaces with a nonzero start are outside the B200 update path.")
+            if np.any(nvec < 1):
+                abort(f"ERROR: every MultiDiscrete nvec entry must be >= 1, got {nvec.tolist()}.")
+            if int(nvec.sum()) > 64:
+                abort(f"ERROR: MultiDiscrete sum(nvec) = {int(nvec.sum())} exceeds the 64 actor outputs the "
+                      "multi-categorical head supports.")
+            self.nvec = [int(n) for n in nvec]
+            self.action_dim = len(self.nvec)
+            self.action_pred_size = sum(self.nvec)
+            self.section_ends = _lib.section_ends(self.nvec)
         else:
             self.action_dim = _flat_dim(action_space)
             self.action_pred_size = self.action_dim
@@ -207,7 +226,8 @@ class PPOPolicy:
 
     @property
     def head(self):
-        return _lib.HEAD_GAUSSIAN_TANH if self.action_dtype == "continuous" else _lib.HEAD_CATEGORICAL
+        return {"continuous": _lib.HEAD_GAUSSIAN_TANH, "discrete": _lib.HEAD_CATEGORICAL,
+                "multi-discrete": _lib.HEAD_MULTI_CATEGORICAL}[self.action_dtype]
 
     def to(self, device):
         self.device = torch.device(device)
@@ -224,7 +244,7 @@ class PPOPolicy:
         if self._ring is None or self._ring.E != E or self._ring.A != len(self.agent_ids):
             self._ring = RolloutRing(self.device, E, len(self.agent_ids), _flat_dim(self.actor_obs_space),
                                      _flat_dim(self.critic_obs_space), self.action_dim,
-                                     self.action_dtype == "discrete",
+                                     self.action_dtype != "continuous",
                                      capacity_steps=max(64, getattr(self, "rollout_steps_hint", 64)))
         self._ring.reset()
         if self.dataset is not None:
@@ -322,6 +342,10 @@ class PPOPolicy:
         values = self.critic(batch_critic_obs).reshape(-1)
         pred = self.actor(batch_obs)
         acts = batch_actions if torch.is_tensor(batch_actions) else torch.as_tensor(np.asarray(batch_actions))
+        if self.action_dtype == "multi-discrete":
+            acts = acts.to(self.device, torch.int64).reshape(pred.shape[0], -1).contiguous()
+            lp, ent = ops.multi_categorical_evaluate(pred, self.section_ends, acts)
+            return values, lp, ent
         if self.action_dtype == "continuous":
             acts = acts.to(self.device, torch.float32).reshape(pred.shape[0], -1).contiguous()
             log_std = self.actor.state_dict()["distribution.log_std"]
@@ -337,8 +361,9 @@ class PPOPolicy:
         (reference policies/ppo_policy.py:729-794).  The actor forward, the std scaling, the tanh squashing / range
         mapping and the log-prob run on the device; the random draws come from torch's global CPU generator in exactly
         the order the reference's CPU sampling consumes them (Normal.sample -> normal_(0, 1) of shape [n, act_dim];
-        Categorical.sample -> exponential_(1) of shape [n, n_actions]), so a seeded run reproduces the reference's
-        actions.  Returns numpy raw_action / action and a CPU log_prob tensor, like the reference.
+        Categorical.sample -> exponential_(1) of shape [n, n_actions]; MultiDiscrete: one Categorical.sample per section,
+        in section order), so a seeded run reproduces the reference's actions.  Returns numpy raw_action / action and a
+        CPU log_prob tensor, like the reference.
         """
         obs = np.asarray(obs) if not torch.is_tensor(obs) else obs
         if len(obs.shape) < 2:
@@ -348,7 +373,12 @@ class PPOPolicy:
         n = t_obs.shape[0]
         discrete = self.action_dtype != "continuous"
         action_pred = self.actor(t_obs, softmax_out=discrete)
-        if discrete:
+        if self.action_dtype == "multi-discrete":
+            noise = torch.cat([torch.empty(n, k, dtype=torch.float32).exponential_(1).reshape(-1) for k in self.nvec])
+            act, lp = ops.multi_categorical_sample(action_pred, self.section_ends,
+                                                   noise.to(self.device, non_blocking=True), len(self.nvec))
+            raw = act
+        elif discrete:
             noise = torch.empty(n, self.action_pred_size, dtype=torch.float32).exponential_(1)
             log_std = dist_min = dist_max = None
         else:
@@ -357,8 +387,9 @@ class PPOPolicy:
             rescale = bool((self.dist_min != -1.0).any() or (self.dist_max != 1.0).any())
             dist_min = self._dist_dev("min") if rescale else None
             dist_max = self._dist_dev("max") if rescale else None
-        raw, act, lp = ops.head_sample(self.head, action_pred, log_std, noise.to(self.device, non_blocking=True),
-                                       self.min_std, dist_min, dist_max, act_dim=1 if discrete else self.action_dim)
+        if self.action_dtype != "multi-discrete":
+            raw, act, lp = ops.head_sample(self.head, action_pred, log_std, noise.to(self.device, non_blocking=True),
+                                           self.min_std, dist_min, dist_max, act_dim=1 if discrete else self.action_dim)
         # the reference aborts on NaN observations / predictions (:758-775); one check of the results covers both
         bad = torch.isnan(t_obs).any() | torch.isnan(action_pred).any()
         # ONE device->host transfer and one sync per call: the three results and the NaN flag travel as one byte buffer
@@ -383,8 +414,9 @@ class PPOPolicy:
     def get_inference_actions(self, obs, deterministic):
         """
         Environment actions only, for `ppoaf test` (reference policies/ppo_policy.py:796-888; ppo.py:972, 1023).
-        deterministic: tanh(mean) mapped to the action range (Gaussian, networks/distributions.py:596-631) or the arg-max
-        class (Categorical, :251-269); otherwise a sample drawn with the rollout protocol.
+        deterministic: tanh(mean) mapped to the action range (Gaussian, networks/distributions.py:596-631), the arg-max
+        class (Categorical, :251-269) or the arg-max class of every section ([n, n_sections], MultiDiscrete); otherwise a
+        sample drawn with the rollout protocol.
         """
         obs = np.asarray(obs) if not torch.is_tensor(obs) else obs
         if len(obs.shape) < 2:
@@ -395,6 +427,8 @@ class PPOPolicy:
         t_obs = torch.as_tensor(obs, dtype=torch.float32).to(self.device).reshape(obs.shape[0], -1).contiguous()
         discrete = self.action_dtype != "continuous"
         action_pred = self.actor(t_obs, softmax_out=discrete)
+        if self.action_dtype == "multi-discrete":
+            return torch.stack([s.argmax(dim=-1) for s in action_pred.split(self.nvec, dim=1)], dim=1).cpu()
         if discrete:
             return torch.argmax(action_pred, dim=-1).cpu()
         n = t_obs.shape[0]

@@ -73,6 +73,8 @@ class UpdateEngine:
         cfg.vf_clip_enabled = int(policy.vf_clip is not None)
         cfg.min_std = policy.min_std
         cfg.world_size = mpi_utils.get_num_procs()
+        if policy.head == _lib.HEAD_MULTI_CATEGORICAL:
+            cfg.section_ends[0], cfg.section_ends[1] = policy.section_ends & 0xFFFFFFFF, policy.section_ends >> 32
         self.cfg = cfg
         dev = self.device
         self.hparams_host = torch.zeros(HP["COUNT"], dtype=torch.float64, pin_memory=True)

@@ -1,6 +1,6 @@
 """
-Minimal Box / Discrete stand-ins with the attributes the update path reads from gymnasium spaces
-(`shape`, `dtype`, `low`, `high`, `n`).  gymnasium is not part of this image; real gymnasium
+Minimal Box / Discrete / MultiDiscrete stand-ins with the attributes the update path reads from gymnasium spaces
+(`shape`, `dtype`, `low`, `high`, `n`, `nvec`, `start`).  gymnasium is not part of this image; real gymnasium
 spaces work unchanged because the policy only duck-types these attributes.
 """
 import numpy as np
@@ -20,4 +20,12 @@ class Discrete:
         self.n = int(n)
         self.start = start
         self.shape = ()
+        self.dtype = np.dtype(np.int64)
+
+
+class MultiDiscrete:
+    def __init__(self, nvec, start=None):
+        self.nvec = np.asarray(nvec, dtype=np.int64)
+        self.start = None if start is None else np.asarray(start, dtype=np.int64)
+        self.shape = self.nvec.shape
         self.dtype = np.dtype(np.int64)
