@@ -589,45 +589,35 @@ __device__ __forceinline__ void ftile(const GemmProblem& g, int tile, int64_t id
     }
 }
 
+static_assert(kLossThreads == kStageThreads, "the staging warps run the shared loss code (loss_common.cuh)");
+struct StageBarrier { __device__ __forceinline__ void operator()() const { bar_stage(); } };
+
 // Head weights of both networks -> shared memory.  They were written by the ADAM phase of the previous step (several grid
 // barriers ago), so the staging warps run this BEFORE the grid barrier that opens the LOSS phase: the L2 loads overlap the
 // wait for the slowest CTA of the last hidden layer.
 __device__ __forceinline__ void loss_stage_heads(const LossArgs& a, float* s_dyn, float* s_sd, float* s_dsd) {
     const int tid = threadIdx.x;
-    const bool gaussian = a.head == PPOAF_HEAD_GAUSSIAN_TANH;
-    const int prows = (a.pred_dim + kPB - 1) / kPB * kPB;
-    const int ldw = a.Ha + 4;
-    float* s_wa = s_dyn;                                             // [prows][ldw]
-    float* s_wc = s_wa + prows * ldw;                                // [Hc]
-    float* s_b = s_wc + a.Hc;                                        // [pred + 1]
-    {
-        const int qa = a.Ha / 4;
-        for (int t = tid; t < prows * qa; t += kStageThreads) {
-            const int row = t / qa, c4 = t - row * qa;
-            const float4 w = row < a.pred_dim ? __ldcg(reinterpret_cast<const float4*>(a.W_actor + int64_t(row) * a.Ha + 4 * c4))
-                                              : make_float4(0.f, 0.f, 0.f, 0.f);
-            *reinterpret_cast<float4*>(s_wa + row * ldw + 4 * c4) = w;
-        }
-        for (int t = tid; t < a.Hc / 4; t += kStageThreads)
-            *reinterpret_cast<float4*>(s_wc + 4 * t) = __ldcg(reinterpret_cast<const float4*>(a.W_critic + 4 * t));
-        if (tid < a.pred_dim) s_b[tid] = __ldcg(a.b_actor + tid);
-        if (tid == 0) s_b[a.pred_dim] = __ldcg(a.b_critic);
-        if (gaussian && tid < a.act_dim) {
-            const float ls = __ldcg(a.log_std + tid);
-            const float sp = softplus_torch(ls);
-            s_sd[tid] = fmaxf(sp, a.min_std);
-            const float sig = ls > 20.f ? 1.f : 1.f / (1.f + expf(-ls));
-            s_dsd[tid] = sp > a.min_std ? sig : (sp == a.min_std ? 0.5f * sig : 0.f);
-        }
+    const HeadSmem hs(a, s_dyn);
+    const int qa = a.Ha / 4;
+    for (int t = tid; t < hs.prows * qa; t += kStageThreads) {
+        const int row = t / qa, c4 = t - row * qa;
+        const float4 w = row < a.pred_dim ? __ldcg(reinterpret_cast<const float4*>(a.W_actor + int64_t(row) * a.Ha + 4 * c4))
+                                          : make_float4(0.f, 0.f, 0.f, 0.f);
+        *reinterpret_cast<float4*>(hs.wa + row * hs.ldw + 4 * c4) = w;
     }
+    for (int t = tid; t < a.Hc / 4; t += kStageThreads)
+        *reinterpret_cast<float4*>(hs.wc + 4 * t) = __ldcg(reinterpret_cast<const float4*>(a.W_critic + 4 * t));
+    if (tid < a.pred_dim) hs.b[tid] = __ldcg(a.b_actor + tid);
+    if (tid == 0) hs.b[a.pred_dim] = __ldcg(a.b_critic);
+    if (a.head == PPOAF_HEAD_GAUSSIAN_TANH && tid < a.act_dim) s_sd[tid] = std_of_log_std(__ldcg(a.log_std + tid), a.min_std, s_dsd[tid]);
 }
 
 // ---------------------------------------------------------------------------------------------------------
 // LOSS phase: one warp per sample, samples dealt round-robin over CTAs so that every SM holds 3-4 of a 512-row
 // minibatch.  Head layers, loss and the heads' dX as in ppo_loss_kernel<true> (loss.cu); the per-CTA partial sums are
 // folded by the last CTA at the start of the next phase (loss_finalize).
-__device__ __forceinline__ void loss_phase(const LossArgs& a, int cur, float* s_dyn, float* s_sd, float* s_dsd,
-                                           double (*s_red)[kPartialStride], long long* dbg) {
+__device__ __forceinline__ void loss_phase(const LossArgs& a, int cur, float* s_dyn, float* s_sd, double (*s_red)[kPartialStride],
+                                           long long* dbg) {
     if (dbg) dbg[0] = clock64();
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int gl = lane;
@@ -635,13 +625,7 @@ __device__ __forceinline__ void loss_phase(const LossArgs& a, int cur, float* s_
     const float w_ent = float(a.hparams[PPOAF_HP_ENTROPY_WEIGHT]);
     const float clip_lo = float(1.0 - a.hparams[PPOAF_HP_SURR_CLIP]), clip_hi = float(1.0 + a.hparams[PPOAF_HP_SURR_CLIP]);
     const bool gaussian = a.head == PPOAF_HEAD_GAUSSIAN_TANH;
-    const int prows = (a.pred_dim + kPB - 1) / kPB * kPB;
-    const int ldw = a.Ha + 4;
-    float* s_wa = s_dyn;                                             // [prows][ldw]
-    float* s_wc = s_wa + prows * ldw;                                // [Hc]
-    float* s_b = s_wc + a.Hc;                                        // [pred + 1]
-    float* s_pred = s_b + ((a.pred_dim + 1 + 3) & ~3);               // [8 warps][kFusedPredLd]
-    float* s_dpred = s_pred + (kStageThreads / 32) * kFusedPredLd;
+    const HeadSmem hs(a, s_dyn);
 
     float adv_mu = 0.f, adv_sd = 1.f, val_mu = 0.f, val_sd = 1.f;    // this minibatch's normalisation constants
     if (a.normalize_adv) { adv_mu = a.mb_adv_stats[2 * cur]; adv_sd = a.mb_adv_stats[2 * cur + 1]; }
@@ -689,57 +673,14 @@ __device__ __forceinline__ void loss_phase(const LossArgs& a, int cur, float* s_
         if (a.normalize_values) target = (target - val_mu) / val_sd;
         if (dbg) dbg[2] = clock64();
 
-        // ---- head layers, forward ----
-        float v_fused = 0.f;
-        float acc[kFusedMaxPred];
-#pragma unroll
-        for (int d = 0; d < kFusedMaxPred; ++d) acc[d] = 0.f;
-#pragma unroll
-        for (int c = 0; c < kFusedMaxChunks; ++c) {
-            const int col = 4 * (gl + kG * c);
-            if (col < a.Ha) {
-#pragma unroll
-                for (int db = 0; db < kFusedMaxPred / kPB; ++db) {
-                    if (db * kPB < a.pred_dim) {
-                        float4 w[kPB];
-#pragma unroll
-                        for (int e = 0; e < kPB; ++e) w[e] = *reinterpret_cast<const float4*>(s_wa + (db * kPB + e) * ldw + col);
-#pragma unroll
-                        for (int e = 0; e < kPB; ++e)
-                            acc[db * kPB + e] = fmaf(ha[c].x, w[e].x, fmaf(ha[c].y, w[e].y, fmaf(ha[c].z, w[e].z,
-                                                fmaf(ha[c].w, w[e].w, acc[db * kPB + e]))));
-                    }
-                }
-            }
-            if (col < a.Hc) {
-                const float4 w = *reinterpret_cast<const float4*>(s_wc + col);
-                v_fused = fmaf(hc[c].x, w.x, fmaf(hc[c].y, w.y, fmaf(hc[c].z, w.z, fmaf(hc[c].w, w.w, v_fused))));
-            }
-        }
-        float v32[32];
-#pragma unroll
-        for (int d = 0; d < 32; ++d) v32[d] = d < kFusedMaxPred ? acc[d] : (d == kFusedMaxPred ? v_fused : 0.f);
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const bool up = (lane & o) != 0;
-#pragma unroll
-            for (int k = 0; k < o; ++k) {
-                const float send = up ? v32[k] : v32[k + o];
-                const float keep = up ? v32[k + o] : v32[k];
-                v32[k] = keep + __shfl_xor_sync(kFull, send, o);
-            }
-        }
-        v_fused = __shfl_sync(kFull, v32[0], kFusedMaxPred) + s_b[a.pred_dim];
-        if (gl < a.pred_dim) s_pred[warp * kFusedPredLd + gl] = v32[0] + s_b[gl];
-        __syncwarp();
+        const float v = head_forward(a, hs, ha, hc, gl, hs.pred + warp * kFusedPredLd);
         if (dbg) dbg[3] = clock64();
-        const float v = v_fused;
         if (gl == 0) a.values[j] = v;                                 // dataset.values[batch_idxs] = values (ppo.py:2340)
         float bad_value = isnan(v) ? 1.f : 0.f;
 
-        const float* pred = s_pred + warp * kFusedPredLd;
+        const float* pred = hs.pred + warp * kFusedPredLd;
         float* dpred = a.d_actor_out + int64_t(i) * (a.d_actor_ld ? a.d_actor_ld : a.pred_dim);
-        float* sdp = s_dpred + warp * kFusedPredLd;
+        float* sdp = hs.dpred + warp * kFusedPredLd;
         actor_head_loss<true>(a, gaussian, true, gl, j, pred, dpred, sdp, s_sd, adv, lp_old, inv_b, w_ent, clip_lo, clip_hi, sc,
                               dsd, bad_value);
 
@@ -752,44 +693,7 @@ __device__ __forceinline__ void loss_phase(const LossArgs& a, int cur, float* s_
         const float bad_any = group_max(bad_value);
         sc[LS_BAD_VALUE] = gl == 0 ? bad_any : 0.f;
 
-        // ---- head layers, backward: dX times the activation derivative of the layer below ----
-        __syncwarp();
-        float dp[kFusedMaxPred];
-#pragma unroll
-        for (int d = 0; d < kFusedMaxPred; ++d) dp[d] = d < a.pred_dim ? sdp[d] : 0.f;
-        const float gv = dv1 * inv_b;
-        float* dza = a.dz_actor + int64_t(i) * a.Ha + 4 * gl;
-        float* dzc = a.dz_critic + int64_t(i) * a.Hc + 4 * gl;
-#pragma unroll
-        for (int c = 0; c < kFusedMaxChunks; ++c) {
-            const int col = 4 * (gl + kG * c);
-            if (col < a.Ha) {
-                float t[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-                for (int db = 0; db < kFusedMaxPred / kPB; ++db) {
-                    if (db * kPB < a.pred_dim) {
-                        float4 w[kPB];
-#pragma unroll
-                        for (int e = 0; e < kPB; ++e) w[e] = *reinterpret_cast<const float4*>(s_wa + (db * kPB + e) * ldw + col);
-#pragma unroll
-                        for (int e = 0; e < kPB; ++e) {
-                            t[0] = fmaf(dp[db * kPB + e], w[e].x, t[0]); t[1] = fmaf(dp[db * kPB + e], w[e].y, t[1]);
-                            t[2] = fmaf(dp[db * kPB + e], w[e].z, t[2]); t[3] = fmaf(dp[db * kPB + e], w[e].w, t[3]);
-                        }
-                    }
-                }
-                const float y[4] = {ha[c].x, ha[c].y, ha[c].z, ha[c].w};
-                act_bwd4(t, y, a.act);
-                *reinterpret_cast<float4*>(dza + 4 * kG * c) = make_float4(t[0], t[1], t[2], t[3]);
-            }
-            if (col < a.Hc) {
-                const float4 w = *reinterpret_cast<const float4*>(s_wc + col);
-                float t[4] = {gv * w.x, gv * w.y, gv * w.z, gv * w.w};
-                const float y[4] = {hc[c].x, hc[c].y, hc[c].z, hc[c].w};
-                act_bwd4(t, y, a.act);
-                *reinterpret_cast<float4*>(dzc + 4 * kG * c) = make_float4(t[0], t[1], t[2], t[3]);
-            }
-        }
+        head_backward(a, hs, ha, hc, sdp, dv1, inv_b, true, gl, i);
         __syncwarp();                                                // s_pred / s_dpred are reused by the next sample
         if (dbg) dbg[5] = clock64();
 #pragma unroll
@@ -798,92 +702,21 @@ __device__ __forceinline__ void loss_phase(const LossArgs& a, int cur, float* s_
         for (int k = 0; k < kPerLane; ++k) tot_dsd[k] += double(dsd[k]);
     }
 
-    // ---- CTA partials (fp64, fixed order) ----
-    if (lane == 0) {
-#pragma unroll
-        for (int k = 0; k < kLossScalars; ++k) s_red[warp][k] = tot_sc[k];
-    }
-#pragma unroll
-    for (int k = 0; k < kPerLane; ++k) s_red[warp][kLossScalars + lane + k * kG] = tot_dsd[k];
-    bar_stage();
-    const int n_vals = kLossScalars + (gaussian ? a.act_dim : 0);
-    double* part = reinterpret_cast<double*>(a.partials);
-    if (tid < n_vals) {
-        double t = 0.0;
-#pragma unroll
-        for (int w = 0; w < kStageThreads / 32; ++w) t += s_red[w][tid];
-        part[size_t(blockIdx.x) * kPartialStride + tid] = t;
-    }
+    loss_cta_partials(tot_sc, tot_dsd, kLossScalars + (gaussian ? a.act_dim : 0), s_red, reinterpret_cast<double*>(a.partials),
+                      StageBarrier{});
     bar_stage();
     if (dbg) dbg[6] = clock64();
 }
 
 // Totals of the loss partials -> d(log_std) (+ its sum of squares) and the epoch statistics.  Run by the staging warps
-// of the last CTA at the start of the phase after LOSS (the partials are visible after the grid barrier).
+// of the last CTA at the start of the phase after LOSS (the partials are visible after the grid barrier).  The fused
+// engine never clips values (loss_head_fusable), so the critic loss is the unclipped one.
 __device__ __forceinline__ void loss_finalize(const LossArgs& a, const float* s_dsd, double (*s_red)[kPartialStride],
                                               double* s_tot, double* s_sq) {
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const bool gaussian = a.head == PPOAF_HEAD_GAUSSIAN_TANH;
-    const int n_vals = kLossScalars + (gaussian ? a.act_dim : 0);
-    const double* part = reinterpret_cast<const double*>(a.partials);
     const float w_ent = float(a.hparams[PPOAF_HP_ENTROPY_WEIGHT]);
-    {
-        constexpr int kSub = kStageThreads / 32, kSlots = (kPartialStride + 31) / 32;
-        double acc3[kSlots];
-#pragma unroll
-        for (int q = 0; q < kSlots; ++q) acc3[q] = 0.0;
-        for (unsigned b = warp; b < gridDim.x; b += kSub) {
-#pragma unroll
-            for (int q = 0; q < kSlots; ++q) {
-                const int vi = lane + 32 * q;
-                if (vi < n_vals) acc3[q] += __ldcg(&part[size_t(b) * kPartialStride + vi]);
-            }
-        }
-#pragma unroll
-        for (int q = 0; q < kSlots; ++q) {
-            const int vi = lane + 32 * q;
-            if (vi < kPartialStride) s_red[warp][vi] = acc3[q];
-        }
-    }
-    bar_stage();
-    double my_sq = 0.0;
-    if (tid < n_vals) {
-        double t = 0.0;
-#pragma unroll
-        for (int w = 0; w < kStageThreads / 32; ++w) t += s_red[w][tid];
-        s_tot[tid] = t;
-        if (tid >= kLossScalars) {
-            const float gls = float(t) * s_dsd[tid - kLossScalars];
-            a.d_log_std[tid - kLossScalars] = gls;
-            for (int q = 0; q < a.n_mirror; ++q)
-                *reinterpret_cast<float*>(reinterpret_cast<char*>(a.d_log_std + (tid - kLossScalars)) + a.mirror_delta[q]) = gls;
-            my_sq = double(gls) * double(gls);
-        }
-    }
-    my_sq = warp_sum(my_sq);
-    if (lane == 0) s_sq[warp] = my_sq;
-    bar_stage();
-    if (tid == 0) {
-        if (a.sq_log_std) {
-            double t = 0.0;
-#pragma unroll
-            for (int k = 0; k < kStageThreads / 32; ++k) t += s_sq[k];
-            *a.sq_log_std = t;
-        }
-        const double nb = double(a.batch);
-        const float actor_mean = float(s_tot[LS_ACTOR] / nb);
-        const float critic_mean = float(s_tot[LS_CRITIC] / nb);
-        double* es = a.epoch_stats;
-        const double e0 = es[PPOAF_ST_ACTOR_LOSS], e1 = es[PPOAF_ST_CRITIC_LOSS], e2 = es[PPOAF_ST_ENTROPY], e3 = es[PPOAF_ST_KL];
-        const double e4 = es[PPOAF_ST_COUNTER], e5 = es[PPOAF_ST_BAD_RATIO], e6 = es[PPOAF_ST_BAD_VALUE];
-        es[PPOAF_ST_ACTOR_LOSS] = e0 + double(actor_mean);
-        es[PPOAF_ST_CRITIC_LOSS] = e1 + double(critic_mean);
-        if (w_ent != 0.f) es[PPOAF_ST_ENTROPY] = e2 + double(float(s_tot[LS_ENTROPY] / nb));
-        es[PPOAF_ST_KL] = e3 + double(float(s_tot[LS_KL] / nb));
-        es[PPOAF_ST_COUNTER] = e4 + 1.0;
-        es[PPOAF_ST_BAD_RATIO] = e5 + s_tot[LS_BAD_RATIO];
-        es[PPOAF_ST_BAD_VALUE] = e6 + s_tot[LS_BAD_VALUE];
-    }
+    loss_fold(a, kLossScalars + (a.head == PPOAF_HEAD_GAUSSIAN_TANH ? a.act_dim : 0), s_dsd, s_red, s_tot, s_sq,
+              StageBarrier{});
+    if (threadIdx.x == 0) add_epoch_stats(a, s_tot, float(s_tot[LS_CRITIC] / double(a.batch)), w_ent);
     bar_stage();
 }
 
@@ -1105,7 +938,7 @@ __global__ void __launch_bounds__(kFThreads, 1) ppo_fused_step_kernel(const __gr
                 if (stp) stp[1] = clock64();
                 if (ph == P.loss_finalize_phase && blockIdx.x == gridDim.x - 1) loss_finalize(P.loss, s_dsd, s_red, s_tot, s_sq);
                 if (d.type == PH_LOSS) {
-                    loss_phase(P.loss, cur, loss_smem, s_sd, s_dsd, s_red, (stp && blockIdx.x == 0) ? P.stamps + 3 * kMaxPhases * 4 + ph * 32 : nullptr);
+                    loss_phase(P.loss, cur, loss_smem, s_sd, s_red, (stp && blockIdx.x == 0) ? P.stamps + 3 * kMaxPhases * 4 + ph * 32 : nullptr);
                     if (step + 1 < P.n_steps) gather_minibatch(P, cur + 1, (step + 1) & 1);   // read again 4 barriers from now
                 } else if (d.type == PH_ADAM) {
                     adam_phase(P, p1, p2, s_scr, s_f, (stp && blockIdx.x == 0) ? P.stamps + 3 * kMaxPhases * 4 + ph * 32 : nullptr);

@@ -91,7 +91,13 @@ struct LossArgs {
 bool loss_head_fusable(int pred_dim, int Ha, int Hc, int vf_clip_enabled);
 // a multi-categorical section table that fits the row: nonzero, last section ends at pred_dim - 1, n_sections ends
 bool section_table_ok(unsigned long long section_ends, int pred_dim, int n_sections);
+// The Categorical head is the table of one section (its callers leave cfg->section_ends zero); rows wider than 64 are
+// refused by the loss launch.
 inline unsigned long long cfg_section_ends(const ppoaf_update_cfg* cfg) {
+    if (cfg->head == PPOAF_HEAD_CATEGORICAL) {
+        const int pred_dim = cfg->actor.dims[cfg->actor.n_layers];
+        return pred_dim <= 64 ? 1ull << (pred_dim - 1) : 0ull;
+    }
     return (uint64_t(cfg->section_ends[1]) << 32) | cfg->section_ends[0];
 }
 // step.cu: validates an update configuration (networks, head, section table); 0 = ok

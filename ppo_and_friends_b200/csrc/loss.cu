@@ -30,18 +30,21 @@ __device__ long long g_loss_stamps[16];
 #define LOSS_STAMP(k) do {} while (0)
 #endif
 
+struct CtaBarrier { __device__ __forceinline__ void operator()() const { __syncthreads(); } };
+
 template <bool FUSED>
 __global__ void __launch_bounds__(kLossThreads) ppo_loss_kernel(const LossArgs a) {
-    extern __shared__ __align__(16) float s_dyn[];      // FUSED: W_actor [pred][Ha+4] | W_critic [Hc] | biases | pred | dpred
+    extern __shared__ __align__(16) float s_dyn[];      // FUSED: HeadSmem
     __shared__ float s_sd[kMaxAct], s_dsd[kMaxAct];
     __shared__ double s_red[kLossThreads / 32][kPartialStride];
     __shared__ double s_tot[kPartialStride];
+    __shared__ double s_sq[kLossThreads / 32];
     __shared__ bool s_last;
 
 #ifdef PPOAF_GEMM_TIMING
     const long long t_entry = clock64();
 #endif
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x;
     const int gl = tid & (kG - 1);                                   // lane inside the sample group
     const int i = blockIdx.x * kSamplesPerBlock + tid / kG;          // sample of this group
     const bool live = i < a.batch;
@@ -54,13 +57,7 @@ __global__ void __launch_bounds__(kLossThreads) ppo_loss_kernel(const LossArgs a
 
     // ---- every global load that does not depend on the cursor is issued first: the hidden activations of this
     // sample and the head weights travel while the cursor -> permutation -> dataset chain resolves ----
-    const int prows = (a.pred_dim + kPB - 1) / kPB * kPB;            // head rows padded to whole blocks of kPB
-    const int ldw = a.Ha + 4;                                        // rows of W_actor land on distinct bank groups
-    float* s_wa = s_dyn;                                             // [prows][ldw]
-    float* s_wc = s_wa + prows * ldw;                                // [Hc]
-    float* s_b = s_wc + a.Hc;                                        // [pred + 1]
-    float* s_pred = s_b + ((a.pred_dim + 1 + 3) & ~3);               // [samples per block][kFusedPredLd]
-    float* s_dpred = s_pred + kSamplesPerBlock * kFusedPredLd;
+    const HeadSmem hs(a, s_dyn);
     // Everything up to pdl_wait() reads only data that no launch of the current step writes (parameters, the
     // dataset, the permutation, the cursor): it overlaps the tail of the previous launch.
     float4 ha[kFusedMaxChunks], hc[kFusedMaxChunks];
@@ -84,14 +81,7 @@ __global__ void __launch_bounds__(kLossThreads) ppo_loss_kernel(const LossArgs a
     if (a.normalize_adv) { adv_mu = a.mb_adv_stats[2 * cur]; adv_sd = a.mb_adv_stats[2 * cur + 1]; }
     if (a.normalize_values) { val_mu = a.mb_val_stats[2 * cur]; val_sd = a.mb_val_stats[2 * cur + 1]; }
 
-    if (gaussian && tid < a.act_dim) {
-        // std = max(softplus(log_std), min_std)  (distributions.py:514-515) and d std / d log_std
-        const float ls = a.log_std[tid];
-        const float sp = softplus_torch(ls);
-        s_sd[tid] = fmaxf(sp, a.min_std);
-        const float sig = ls > 20.f ? 1.f : 1.f / (1.f + expf(-ls));
-        s_dsd[tid] = sp > a.min_std ? sig : (sp == a.min_std ? 0.5f * sig : 0.f);
-    }
+    if (gaussian && tid < a.act_dim) s_sd[tid] = std_of_log_std(a.log_std[tid], a.min_std, s_dsd[tid]);
     float adv = live ? a.advantages[j] : 0.f;
     const float lp_old = live ? a.log_probs[j] : 0.f;
     float target = live ? a.rewards_to_go[j] : 0.f;
@@ -111,12 +101,12 @@ __global__ void __launch_bounds__(kLossThreads) ppo_loss_kernel(const LossArgs a
         for (int k = 0; k < kFusedStageSlots; ++k) {
             const int t = tid + k * kLossThreads;
             const int row = t / qa, c4 = t - row * qa;
-            if (row < prows) *reinterpret_cast<float4*>(s_wa + row * ldw + 4 * c4) = wreg[k];   // padding rows are zero
+            if (row < hs.prows) *reinterpret_cast<float4*>(hs.wa + row * hs.ldw + 4 * c4) = wreg[k];   // padding rows are zero
         }
         for (int t = tid; t < a.Hc / 4; t += kLossThreads)
-            *reinterpret_cast<float4*>(s_wc + 4 * t) = *reinterpret_cast<const float4*>(a.W_critic + 4 * t);
-        if (tid < a.pred_dim) s_b[tid] = a.b_actor[tid];
-        if (tid == 0) s_b[a.pred_dim] = a.b_critic[0];
+            *reinterpret_cast<float4*>(hs.wc + 4 * t) = *reinterpret_cast<const float4*>(a.W_critic + 4 * t);
+        if (tid < a.pred_dim) hs.b[tid] = a.b_actor[tid];
+        if (tid == 0) hs.b[a.pred_dim] = a.b_critic[0];
     }
     if (jn >= 0) {
         // pull the NEXT minibatch's observation rows into L2 while this step's backward pass runs: the first-layer
@@ -133,70 +123,22 @@ __global__ void __launch_bounds__(kLossThreads) ppo_loss_kernel(const LossArgs a
     float sc[kLossScalars];
 #pragma unroll
     for (int k = 0; k < kLossScalars; ++k) sc[k] = 0.f;
-    float dsd[kPerLane];                                             // d loss / d std for dims gl + 8k of this sample
+    float dsd[kPerLane];                                             // d loss / d std for dims gl + 32k of this sample
 #pragma unroll
     for (int k = 0; k < kPerLane; ++k) dsd[k] = 0.f;
 
     if (a.normalize_adv) adv = (adv - adv_mu) / adv_sd;
     if (a.normalize_values) target = (target - val_mu) / val_sd;
-    // ---- fused heads, forward: every lane dots its columns of the hidden activations with all head rows, the 8
-    // lanes of the sample fold their partial sums, and the outputs go to shared memory ----
     float v_fused = 0.f;
-    if constexpr (FUSED) {
-        float acc[kFusedMaxPred];
-#pragma unroll
-        for (int d = 0; d < kFusedMaxPred; ++d) acc[d] = 0.f;
-#pragma unroll
-        for (int c = 0; c < kFusedMaxChunks; ++c) {
-            const int col = 4 * (gl + kG * c);
-            if (col < a.Ha) {
-#pragma unroll
-                for (int db = 0; db < kFusedMaxPred / kPB; ++db) {
-                    if (db * kPB < a.pred_dim) {                     // uniform: whole blocks of independent rows
-                        float4 w[kPB];
-#pragma unroll
-                        for (int e = 0; e < kPB; ++e) w[e] = *reinterpret_cast<const float4*>(s_wa + (db * kPB + e) * ldw + col);
-#pragma unroll
-                        for (int e = 0; e < kPB; ++e)
-                            acc[db * kPB + e] = fmaf(ha[c].x, w[e].x, fmaf(ha[c].y, w[e].y, fmaf(ha[c].z, w[e].z,
-                                                fmaf(ha[c].w, w[e].w, acc[db * kPB + e]))));
-                    }
-                }
-            }
-            if (col < a.Hc) {
-                const float4 w = *reinterpret_cast<const float4*>(s_wc + col);
-                v_fused = fmaf(hc[c].x, w.x, fmaf(hc[c].y, w.y, fmaf(hc[c].z, w.z, fmaf(hc[c].w, w.w, v_fused))));
-            }
-        }
-        LOSS_STAMP(2);
-        // fold over the 32 lanes by recursive halving: at every step a lane keeps half of its values and trades the
-        // other half with its partner, so 32 value slots cost 16+8+4+2+1 shuffles and lane l ends with the total of
-        // slot l (slots 0..23: actor outputs, slot 24: the critic output)
-        float v32[32];
-#pragma unroll
-        for (int d = 0; d < 32; ++d) v32[d] = d < kFusedMaxPred ? acc[d] : (d == kFusedMaxPred ? v_fused : 0.f);
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const bool up = (lane & o) != 0;
-#pragma unroll
-            for (int k = 0; k < o; ++k) {
-                const float send = up ? v32[k] : v32[k + o];
-                const float keep = up ? v32[k + o] : v32[k];
-                v32[k] = keep + __shfl_xor_sync(kFull, send, o);
-            }
-        }
-        v_fused = __shfl_sync(kFull, v32[0], kFusedMaxPred) + s_b[a.pred_dim];
-        if (gl < a.pred_dim) s_pred[smp * kFusedPredLd + gl] = v32[0] + s_b[gl];
-        __syncwarp();                                                // the lanes of a sample share one warp
-    }
+    if constexpr (FUSED) v_fused = head_forward(a, hs, ha, hc, gl, hs.pred + smp * kFusedPredLd);
     LOSS_STAMP(3);
     const float v = FUSED ? (live ? v_fused : 0.f) : (live ? a.critic_out[i] : 0.f);
     if (live && gl == 0) a.values[j] = v;                            // dataset.values[batch_idxs] = values (ppo.py:2340)
     float bad_value = isnan(v) ? 1.f : 0.f;
 
-    const float* pred = FUSED ? s_pred + smp * kFusedPredLd : a.actor_out + int64_t(live ? i : 0) * a.pred_dim;
+    const float* pred = FUSED ? hs.pred + smp * kFusedPredLd : a.actor_out + int64_t(live ? i : 0) * a.pred_dim;
     float* dpred = a.d_actor_out + int64_t(live ? i : 0) * a.pred_dim;
-    float* sdp = s_dpred + smp * kFusedPredLd;                       // FUSED: dL/d(actor out) kept for the head's dX
+    float* sdp = hs.dpred + smp * kFusedPredLd;                      // FUSED: dL/d(actor out) kept for the head's dX
     actor_head_loss<FUSED>(a, gaussian, live, gl, j, pred, dpred, sdp, s_sd, adv, lp_old, inv_b, w_ent, clip_lo, clip_hi,
                            sc, dsd, bad_value);
 
@@ -220,69 +162,13 @@ __global__ void __launch_bounds__(kLossThreads) ppo_loss_kernel(const LossArgs a
     const float bad_any = group_max(bad_value);
     sc[LS_BAD_VALUE] = (live && gl == 0) ? bad_any : 0.f;
 
-    // ---- fused heads, backward: dX of the two head layers times the activation derivative of the layer below ----
-    if constexpr (FUSED) {
-        __syncwarp();
-        float dp[kFusedMaxPred];
-#pragma unroll
-        for (int d = 0; d < kFusedMaxPred; ++d) dp[d] = (d < a.pred_dim && live) ? sdp[d] : 0.f;
-        const float gv = live ? dv1 * inv_b : 0.f;
-        float* dza = a.dz_actor + int64_t(live ? i : 0) * a.Ha + 4 * gl;
-        float* dzc = a.dz_critic + int64_t(live ? i : 0) * a.Hc + 4 * gl;
-#pragma unroll
-        for (int c = 0; c < kFusedMaxChunks; ++c) {
-            const int col = 4 * (gl + kG * c);
-            if (col < a.Ha) {
-                float t[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-                for (int db = 0; db < kFusedMaxPred / kPB; ++db) {
-                    if (db * kPB < a.pred_dim) {                     // padding rows of s_wa are zero
-                        float4 w[kPB];
-#pragma unroll
-                        for (int e = 0; e < kPB; ++e) w[e] = *reinterpret_cast<const float4*>(s_wa + (db * kPB + e) * ldw + col);
-#pragma unroll
-                        for (int e = 0; e < kPB; ++e) {
-                            t[0] = fmaf(dp[db * kPB + e], w[e].x, t[0]); t[1] = fmaf(dp[db * kPB + e], w[e].y, t[1]);
-                            t[2] = fmaf(dp[db * kPB + e], w[e].z, t[2]); t[3] = fmaf(dp[db * kPB + e], w[e].w, t[3]);
-                        }
-                    }
-                }
-                const float y[4] = {ha[c].x, ha[c].y, ha[c].z, ha[c].w};
-                act_bwd4(t, y, a.act);
-                if (live) *reinterpret_cast<float4*>(dza + 4 * kG * c) = make_float4(t[0], t[1], t[2], t[3]);
-            }
-            if (col < a.Hc) {
-                const float4 w = *reinterpret_cast<const float4*>(s_wc + col);
-                float t[4] = {gv * w.x, gv * w.y, gv * w.z, gv * w.w};
-                const float y[4] = {hc[c].x, hc[c].y, hc[c].z, hc[c].w};
-                act_bwd4(t, y, a.act);
-                if (live) *reinterpret_cast<float4*>(dzc + 4 * kG * c) = make_float4(t[0], t[1], t[2], t[3]);
-            }
-        }
-    }
+    if constexpr (FUSED) head_backward(a, hs, ha, hc, sdp, dv1, inv_b, live, gl, live ? i : 0);
 
     LOSS_STAMP(5);
-    // ---------------- CTA reduction (fp64, fixed order) ----------------
-    // one warp per sample: lane 0 holds the sample's scalars, lane l holds d(loss)/d(std) of dims l, l + 32
-    static_assert(kG == 32, "the reduction below assumes one warp per sample");
-    const int n_extra = gaussian ? a.act_dim : 0;
-    if (lane == 0) {
-#pragma unroll
-        for (int k = 0; k < kLossScalars; ++k) s_red[warp][k] = double(sc[k]);
-    }
-    if (gaussian) {
-#pragma unroll
-        for (int k = 0; k < kPerLane; ++k) s_red[warp][kLossScalars + lane + k * kG] = double(dsd[k]);
-    }
-    __syncthreads();
-    const int n_vals = kLossScalars + n_extra;
+    // ---------------- CTA partials; the last CTA to finish folds them ----------------
+    const int n_vals = kLossScalars + (gaussian ? a.act_dim : 0);
     double* part = reinterpret_cast<double*>(a.partials);
-    if (tid < n_vals) {
-        double t = 0.0;
-#pragma unroll
-        for (int w = 0; w < kLossThreads / 32; ++w) t += s_red[w][tid];
-        part[size_t(blockIdx.x) * kPartialStride + tid] = t;
-    }
+    loss_cta_partials(sc, dsd, n_vals, s_red, part, CtaBarrier{});
     LOSS_STAMP(6);
     __threadfence();
     __syncthreads();
@@ -294,56 +180,9 @@ __global__ void __launch_bounds__(kLossThreads) ppo_loss_kernel(const LossArgs a
     LOSS_STAMP(8);
 
     // ---------------- last CTA: totals -> d(log_std), epoch statistics, value-clip weights -----------
-    // thread (slot = tid % 32, subset = tid / 32) sums CTAs subset, subset + 8, ... for values slot, slot + 32, slot + 64
-    // (all loads independent and in flight at once); the 8 subsets are then added in a fixed order
-    {
-        constexpr int kSub = kLossThreads / 32, kSlots = (kPartialStride + 31) / 32;
-        double acc3[kSlots];
-#pragma unroll
-        for (int q = 0; q < kSlots; ++q) acc3[q] = 0.0;
-        for (unsigned b = warp; b < gridDim.x; b += kSub) {
-#pragma unroll
-            for (int q = 0; q < kSlots; ++q) {
-                const int vi = lane + 32 * q;
-                if (vi < n_vals) acc3[q] += __ldcg(&part[size_t(b) * kPartialStride + vi]);
-            }
-        }
-#pragma unroll
-        for (int q = 0; q < kSlots; ++q) {
-            const int vi = lane + 32 * q;
-            if (vi < kPartialStride) s_red[warp][vi] = acc3[q];
-        }
-    }
-    __syncthreads();
-    __shared__ double s_sq[kLossThreads / 32];
-    double my_sq = 0.0;
-    if (tid < n_vals) {
-        double t = 0.0;
-#pragma unroll
-        for (int w = 0; w < kLossThreads / 32; ++w) t += s_red[w][tid];
-        s_tot[tid] = t;
-        if (tid >= kLossScalars) {
-            const float gls = float(t) * s_dsd[tid - kLossScalars];
-            a.d_log_std[tid - kLossScalars] = gls;
-            for (int q = 0; q < a.n_mirror; ++q)
-                *reinterpret_cast<float*>(reinterpret_cast<char*>(a.d_log_std + (tid - kLossScalars)) + a.mirror_delta[q]) = gls;
-            my_sq = double(gls) * double(gls);
-        }
-    }
-    my_sq = warp_sum(my_sq);
-    LOSS_STAMP(9);
-    if (lane == 0) s_sq[warp] = my_sq;
-    __syncthreads();
-    if (tid == 0 && a.sq_log_std) {                        // sum of squares of d(log_std) for the gradient-norm clip
-        double t = 0.0;
-#pragma unroll
-        for (int k = 0; k < kLossThreads / 32; ++k) t += s_sq[k];
-        *a.sq_log_std = t;
-    }
-    __syncthreads();
+    loss_fold(a, n_vals, s_dsd, s_red, s_tot, s_sq, CtaBarrier{});
     if (tid == 0) {
         const double nb = double(a.batch);
-        const float actor_mean = float(s_tot[LS_ACTOR] / nb);
         float critic_mean = float(s_tot[LS_CRITIC] / nb);
         if (a.vf_clip_enabled) {
             // critic_loss = max(loss(v), loss(clamp(v)))  (ppo.py:2427-2436; intended semantics, SURVEY Q4);
@@ -355,17 +194,7 @@ __global__ void __launch_bounds__(kLossThreads) ppo_loss_kernel(const LossArgs a
             float* wsel = reinterpret_cast<float*>(part + size_t(gridDim.x) * kPartialStride);
             wsel[0] = w1; wsel[1] = w2;
         }
-        const double e0 = a.epoch_stats[PPOAF_ST_ACTOR_LOSS], e1 = a.epoch_stats[PPOAF_ST_CRITIC_LOSS];
-        const double e2 = a.epoch_stats[PPOAF_ST_ENTROPY], e3 = a.epoch_stats[PPOAF_ST_KL];
-        const double e4 = a.epoch_stats[PPOAF_ST_COUNTER], e5 = a.epoch_stats[PPOAF_ST_BAD_RATIO];
-        const double e6 = a.epoch_stats[PPOAF_ST_BAD_VALUE];            // seven independent loads, then the stores
-        a.epoch_stats[PPOAF_ST_ACTOR_LOSS] = e0 + double(actor_mean);
-        a.epoch_stats[PPOAF_ST_CRITIC_LOSS] = e1 + double(critic_mean);
-        if (w_ent != 0.f) a.epoch_stats[PPOAF_ST_ENTROPY] = e2 + double(float(s_tot[LS_ENTROPY] / nb));
-        a.epoch_stats[PPOAF_ST_KL] = e3 + double(float(s_tot[LS_KL] / nb));
-        a.epoch_stats[PPOAF_ST_COUNTER] = e4 + 1.0;
-        a.epoch_stats[PPOAF_ST_BAD_RATIO] = e5 + s_tot[LS_BAD_RATIO];
-        a.epoch_stats[PPOAF_ST_BAD_VALUE] = e6 + s_tot[LS_BAD_VALUE];
+        add_epoch_stats(a, s_tot, critic_mean, w_ent);
         *a.ticket = 0u;  // ready for the next launch
     }
     LOSS_STAMP(10);
@@ -413,160 +242,80 @@ extern "C" int ppoaf_debug_loss_stamps(long long* out_host) {
 }
 #endif
 
-// ---- stand-alone head evaluation (PPOPolicy.evaluate's distribution half, policies/ppo_policy.py:939-950) ----
+// ---- stand-alone heads (PPOPolicy.evaluate's distribution half, policies/ppo_policy.py:939-950, and rollout-time
+// sampling, :729-794): one thread per row.  The Categorical head runs the multi-categorical kernels with a table of one
+// section. ----
 namespace ppoaf {
 
-__global__ void head_evaluate_kernel(int head, const float* __restrict__ actor_out, int pred_dim,
-                                     const float* __restrict__ log_std, float min_std, const void* __restrict__ actions,
-                                     int act_dim, int n_rows, float* __restrict__ lp_out, float* __restrict__ ent_out) {
+__global__ void head_evaluate_kernel(const float* __restrict__ actor_out, int pred_dim, const float* __restrict__ log_std,
+                                     float min_std, const float* __restrict__ actions, int act_dim, int n_rows,
+                                     float* __restrict__ lp_out, float* __restrict__ ent_out) {
     __shared__ float s_sd[kMaxAct];
-    const bool gaussian = head == PPOAF_HEAD_GAUSSIAN_TANH;
-    if (gaussian && threadIdx.x < act_dim) s_sd[threadIdx.x] = fmaxf(softplus_torch(log_std[threadIdx.x]), min_std);
+    float dstd;
+    if (threadIdx.x < act_dim) s_sd[threadIdx.x] = std_of_log_std(log_std[threadIdx.x], min_std, dstd);
     __syncthreads();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_rows) return;
     const float* pred = actor_out + int64_t(i) * pred_dim;
-    float lp = 0.f, ent = 0.f;
-    if (gaussian) {
-        const float* x = reinterpret_cast<const float*>(actions) + int64_t(i) * act_dim;
-        float nsum = 0.f, slog = 0.f, ensum = 0.f, eslog = 0.f;
-        for (int d = 0; d < act_dim; ++d) {
-            const float mu = pred[d], sd = s_sd[d], z = x[d] - mu, lsd = logf(sd);
-            nsum += fminf(fmaxf(-(z * z) / (2.f * (sd * sd)) - lsd - kLogSqrt2Pi, -100.f), 100.f);
-            const float th = tanhf(x[d]);
-            slog += logf(fmaxf(1.f - th * th, 1e-6f));
-            ensum += fminf(fmaxf(-lsd - kLogSqrt2Pi, -100.f), 100.f);
-            const float thm = tanhf(mu);
-            eslog += logf(fmaxf(1.f - thm * thm, 1e-6f));
-        }
-        lp = nsum - slog;
-        ent = -(ensum - eslog);
-    } else {
-        const int action = int(reinterpret_cast<const int64_t*>(actions)[int64_t(i) * act_dim]);
-        float mx = pred[0];
-        for (int c = 1; c < pred_dim; ++c) mx = fmaxf(mx, pred[c]);
-        float se = 0.f;
-        for (int c = 0; c < pred_dim; ++c) se += expf(pred[c] - mx);
-        float S = 0.f;
-        for (int c = 0; c < pred_dim; ++c) S += expf(pred[c] - mx) / se;
-        const float ceps = 1.1920928955078125e-07f;
-        float h = 0.f;
-        for (int c = 0; c < pred_dim; ++c) {
-            const float pn = (expf(pred[c] - mx) / se) / S;
-            const float l = logf(fminf(fmaxf(pn, ceps), 1.f - ceps));
-            h += pn * l;
-            if (c == action) lp = l;
-        }
-        ent = -h;
+    const float* x = actions + int64_t(i) * act_dim;
+    float nsum = 0.f, slog = 0.f, ensum = 0.f, eslog = 0.f;
+    for (int d = 0; d < act_dim; ++d) {
+        const float mu = pred[d], sd = s_sd[d], z = x[d] - mu, lsd = logf(sd);
+        nsum += fminf(fmaxf(-(z * z) / (2.f * (sd * sd)) - lsd - kLogSqrt2Pi, -100.f), 100.f);
+        const float th = tanhf(x[d]);
+        slog += logf(fmaxf(1.f - th * th, 1e-6f));
+        ensum += fminf(fmaxf(-lsd - kLogSqrt2Pi, -100.f), 100.f);
+        const float thm = tanhf(mu);
+        eslog += logf(fmaxf(1.f - thm * thm, 1e-6f));
     }
-    lp_out[i] = lp;
-    if (ent_out) ent_out[i] = ent;
+    lp_out[i] = nsum - slog;
+    if (ent_out) ent_out[i] = -(ensum - eslog);
 }
 
-}  // namespace ppoaf
-
-namespace ppoaf {
-
-// Rollout-time sampling (PPOPolicy.get_rollout_actions, policies/ppo_policy.py:729-794).  The random draws come from the
-// HOST generator in the order the reference's CPU sampling consumes them (`noise`), so the actions are the reference's
-// actions; everything else -- scaling by std, tanh squashing, range mapping, log-prob -- happens here.
-//   Gaussian:    noise = N(0,1) [n, act_dim];  raw = noise * std + mean  (torch.normal: mul_ then add_)
-//                action = tanh(raw), mapped to [min, max] when given (distributions.py:560-610); log-prob :518-558
-//   Categorical: noise = Exp(1) [n, pred];  sample = argmax(p / noise)  (aten multinomial, one draw); log-prob :223-249
-__global__ void head_sample_kernel(int head, const float* __restrict__ actor_out, int pred_dim,
-                                   const float* __restrict__ log_std, float min_std, const float* __restrict__ noise,
-                                   const float* __restrict__ dist_min, const float* __restrict__ dist_max, int act_dim,
-                                   int n_rows, void* __restrict__ raw_out, void* __restrict__ act_out,
-                                   float* __restrict__ lp_out) {
+// The random draws come from the HOST generator in the order the reference's CPU sampling consumes them (`noise`), so
+// the actions are the reference's actions; everything else -- scaling by std, tanh squashing, range mapping, log-prob --
+// happens here.  noise = N(0,1) [n, act_dim];  raw = noise * std + mean  (torch.normal: mul_ then add_);
+// action = tanh(raw), mapped to [min, max] when given (distributions.py:560-610); log-prob :518-558
+__global__ void head_sample_kernel(const float* __restrict__ actor_out, int pred_dim, const float* __restrict__ log_std,
+                                   float min_std, const float* __restrict__ noise, const float* __restrict__ dist_min,
+                                   const float* __restrict__ dist_max, int act_dim, int n_rows, float* __restrict__ raw_out,
+                                   float* __restrict__ act_out, float* __restrict__ lp_out) {
     __shared__ float s_sd[kMaxAct];
-    const bool gaussian = head == PPOAF_HEAD_GAUSSIAN_TANH;
-    if (gaussian && threadIdx.x < act_dim) s_sd[threadIdx.x] = fmaxf(softplus_torch(log_std[threadIdx.x]), min_std);
+    float dstd;
+    if (threadIdx.x < act_dim) s_sd[threadIdx.x] = std_of_log_std(log_std[threadIdx.x], min_std, dstd);
     __syncthreads();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_rows) return;
     const float* pred = actor_out + int64_t(i) * pred_dim;
-    if (gaussian) {
-        const float* z = noise + int64_t(i) * act_dim;
-        float* raw = reinterpret_cast<float*>(raw_out) + int64_t(i) * act_dim;
-        float* act = reinterpret_cast<float*>(act_out) + int64_t(i) * act_dim;
-        float nsum = 0.f, slog = 0.f;
-        for (int d = 0; d < act_dim; ++d) {
-            const float mu = pred[d], sd = s_sd[d];
-            const float x = __fadd_rn(__fmul_rn(z[d], sd), mu);
-            const float th = tanhf(x);
-            float a = th;
-            if (dist_min && dist_max)
-                a = __fadd_rn(__fmul_rn(__fdiv_rn(__fadd_rn(th, 1.f), 2.f), __fsub_rn(dist_max[d], dist_min[d])), dist_min[d]);
-            raw[d] = x;
-            act[d] = a;
-            const float dz = x - mu;
-            nsum += fminf(fmaxf(-(dz * dz) / (2.f * (sd * sd)) - logf(sd) - kLogSqrt2Pi, -100.f), 100.f);
-            slog += logf(fmaxf(1.f - th * th, 1e-6f));
-        }
-        lp_out[i] = nsum - slog;
-    } else {
-        const float* q = noise + int64_t(i) * pred_dim;
-        float S = 0.f;
-        for (int c = 0; c < pred_dim; ++c) S += pred[c];
-        int best = 0;
-        float best_v = -INFINITY, best_p = 0.f;
-        for (int c = 0; c < pred_dim; ++c) {
-            const float pn = pred[c] / S;
-            const float v = pn / q[c];
-            if (v > best_v) { best_v = v; best = c; best_p = pn; }          // first maximum, like argmax
-        }
-        reinterpret_cast<int64_t*>(raw_out)[i] = best;
-        reinterpret_cast<int64_t*>(act_out)[i] = best;
-        lp_out[i] = logf(fminf(fmaxf(best_p, kCatEps), 1.f - kCatEps));
+    const float* z = noise + int64_t(i) * act_dim;
+    float* raw = raw_out + int64_t(i) * act_dim;
+    float* act = act_out + int64_t(i) * act_dim;
+    float nsum = 0.f, slog = 0.f;
+    for (int d = 0; d < act_dim; ++d) {
+        const float mu = pred[d], sd = s_sd[d];
+        const float x = __fadd_rn(__fmul_rn(z[d], sd), mu);
+        const float th = tanhf(x);
+        float a = th;
+        if (dist_min && dist_max)
+            a = __fadd_rn(__fmul_rn(__fdiv_rn(__fadd_rn(th, 1.f), 2.f), __fsub_rn(dist_max[d], dist_min[d])), dist_min[d]);
+        raw[d] = x;
+        act[d] = a;
+        const float dz = x - mu;
+        nsum += fminf(fmaxf(-(dz * dz) / (2.f * (sd * sd)) - logf(sd) - kLogSqrt2Pi, -100.f), 100.f);
+        slog += logf(fmaxf(1.f - th * th, 1e-6f));
     }
+    lp_out[i] = nsum - slog;
 }
 
-}  // namespace ppoaf
-
-extern "C" int ppoaf_head_sample(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std,
-                                 float min_std, const float* noise, const float* dist_min, const float* dist_max,
-                                 int32_t act_dim, int32_t n_rows, void* raw_action_out, void* action_out,
-                                 float* log_prob_out, void* stream) {
-    using namespace ppoaf;
-    PPOAF_CHECK_ARG(head == PPOAF_HEAD_GAUSSIAN_TANH || head == PPOAF_HEAD_CATEGORICAL, "ppoaf_head_sample: unknown head");
-    PPOAF_CHECK_ARG(act_dim >= 1 && act_dim <= kMaxAct && pred_dim >= 1 && pred_dim <= kMaxAct,
-                    "ppoaf_head_sample: widths must be in [1, %d]", kMaxAct);
-    PPOAF_CHECK_ARG(n_rows >= 0 && noise != nullptr, "ppoaf_head_sample: bad arguments");
-    PPOAF_CHECK_ARG((dist_min == nullptr) == (dist_max == nullptr), "ppoaf_head_sample: give both range bounds or neither");
-    if (n_rows == 0) return 0;
-    head_sample_kernel<<<(n_rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        head, actor_out, pred_dim, log_std, min_std, noise, dist_min, dist_max, act_dim, n_rows, raw_action_out, action_out,
-        log_prob_out);
-    PPOAF_CHECK_LAUNCH("ppoaf_head_sample");
-    return 0;
-}
-
-extern "C" int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std,
-                                   float min_std, const void* actions, int32_t act_dim, int32_t n_rows,
-                                   float* log_prob_out, float* entropy_out, void* stream) {
-    using namespace ppoaf;
-    PPOAF_CHECK_ARG(head == PPOAF_HEAD_GAUSSIAN_TANH || head == PPOAF_HEAD_CATEGORICAL, "ppoaf_head_evaluate: unknown head");
-    PPOAF_CHECK_ARG(act_dim >= 1 && act_dim <= kMaxAct && pred_dim >= 1 && pred_dim <= kMaxAct,
-                    "ppoaf_head_evaluate: widths must be in [1, %d]", kMaxAct);
-    PPOAF_CHECK_ARG(n_rows >= 0, "ppoaf_head_evaluate: n_rows < 0");
-    if (n_rows == 0) return 0;
-    head_evaluate_kernel<<<(n_rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        head, actor_out, pred_dim, log_std, min_std, actions, act_dim, n_rows, log_prob_out, entropy_out);
-    PPOAF_CHECK_LAUNCH("ppoaf_head_evaluate");
-    return 0;
-}
-
-// ---- the multi-categorical head on its own (PPOAF_HEAD_MULTI_CATEGORICAL): one thread per row, sections in order ----
-namespace ppoaf {
-
+// Multi-categorical evaluation; actions: int64 rows of act_ld (the number of sections; act_dim for the Categorical ABI)
 __global__ void multi_categorical_evaluate_kernel(const float* __restrict__ actor_out, int pred_dim,
                                                   unsigned long long ends, const int64_t* __restrict__ actions,
-                                                  int n_sections, int n_rows, float* __restrict__ lp_out,
+                                                  int act_ld, int n_rows, float* __restrict__ lp_out,
                                                   float* __restrict__ ent_out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_rows) return;
     const float* pred = actor_out + int64_t(i) * pred_dim;
-    const int64_t* act = actions + int64_t(i) * n_sections;
+    const int64_t* act = actions + int64_t(i) * act_ld;
     float mx = pred[0];
     for (int c = 1; c < pred_dim; ++c) mx = fmaxf(mx, pred[c]);
     float se = 0.f;
@@ -590,13 +339,19 @@ __global__ void multi_categorical_evaluate_kernel(const float* __restrict__ acto
     if (ent_out) ent_out[i] = -h;
 }
 
-// probs: the softmax of the whole row; noise: section k's Exp(1) block [n_rows, n_k] starts at n_rows * o_k
-__global__ void multi_categorical_sample_kernel(const float* __restrict__ probs, int pred_dim, unsigned long long ends,
-                                                const float* __restrict__ noise, int n_sections, int n_rows,
-                                                int64_t* __restrict__ act_out, float* __restrict__ lp_out) {
+// Multi-categorical sampling.  probs: the softmax of the whole row; noise: section k's Exp(1) block [n_rows, n_k] starts
+// at n_rows * o_k; in each section a_k = first argmax(p~_k / q_k) (aten multinomial, one draw; distributions.py:223-249).
+// raw_out (nullable): a second copy of the actions, which the Categorical ABI writes.  16 blocks of 128 per SM keep it
+// at 32 registers, full occupancy.
+__global__ void __launch_bounds__(128, 16)
+multi_categorical_sample_kernel(const float* __restrict__ probs, int pred_dim, unsigned long long ends,
+                                const float* __restrict__ noise, int n_sections, int n_rows, int64_t* __restrict__ act_out,
+                                float* __restrict__ lp_out, int64_t* __restrict__ raw_out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_rows) return;
     const float* p = probs + int64_t(i) * pred_dim;
+    int64_t* act = act_out + int64_t(i) * n_sections;
+    int64_t* raw = raw_out ? raw_out + int64_t(i) * n_sections : nullptr;
     float lp = 0.f;
     for (int o = 0, k = 0, c = 0; c < pred_dim; ++c) {
         if (!((ends >> c) & 1ull)) continue;
@@ -611,7 +366,8 @@ __global__ void multi_categorical_sample_kernel(const float* __restrict__ probs,
             const float v = pn / q[d];
             if (v > best_v) { best_v = v; best = d; best_p = pn; }        // first maximum, like argmax
         }
-        act_out[int64_t(i) * n_sections + k] = best;
+        act[k] = best;
+        if (raw) raw[k] = best;
         lp += logf(fminf(fmaxf(best_p, kCatEps), 1.f - kCatEps));
         o = c + 1;
         ++k;
@@ -620,6 +376,51 @@ __global__ void multi_categorical_sample_kernel(const float* __restrict__ probs,
 }
 
 }  // namespace ppoaf
+
+extern "C" int ppoaf_head_sample(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std,
+                                 float min_std, const float* noise, const float* dist_min, const float* dist_max,
+                                 int32_t act_dim, int32_t n_rows, void* raw_action_out, void* action_out,
+                                 float* log_prob_out, void* stream) {
+    using namespace ppoaf;
+    PPOAF_CHECK_ARG(head == PPOAF_HEAD_GAUSSIAN_TANH || head == PPOAF_HEAD_CATEGORICAL, "ppoaf_head_sample: unknown head");
+    PPOAF_CHECK_ARG(act_dim >= 1 && act_dim <= kMaxAct && pred_dim >= 1 && pred_dim <= kMaxAct,
+                    "ppoaf_head_sample: widths must be in [1, %d]", kMaxAct);
+    PPOAF_CHECK_ARG(n_rows >= 0 && noise != nullptr, "ppoaf_head_sample: bad arguments");
+    PPOAF_CHECK_ARG((dist_min == nullptr) == (dist_max == nullptr), "ppoaf_head_sample: give both range bounds or neither");
+    if (n_rows == 0) return 0;
+    const dim3 grid((n_rows + 127) / 128), block(128);
+    if (head == PPOAF_HEAD_GAUSSIAN_TANH)
+        head_sample_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(
+            actor_out, pred_dim, log_std, min_std, noise, dist_min, dist_max, act_dim, n_rows, static_cast<float*>(raw_action_out),
+            static_cast<float*>(action_out), log_prob_out);
+    else
+        multi_categorical_sample_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(
+            actor_out, pred_dim, 1ull << (pred_dim - 1), noise, 1, n_rows, static_cast<int64_t*>(action_out), log_prob_out,
+            static_cast<int64_t*>(raw_action_out));
+    PPOAF_CHECK_LAUNCH("ppoaf_head_sample");
+    return 0;
+}
+
+extern "C" int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std,
+                                   float min_std, const void* actions, int32_t act_dim, int32_t n_rows,
+                                   float* log_prob_out, float* entropy_out, void* stream) {
+    using namespace ppoaf;
+    PPOAF_CHECK_ARG(head == PPOAF_HEAD_GAUSSIAN_TANH || head == PPOAF_HEAD_CATEGORICAL, "ppoaf_head_evaluate: unknown head");
+    PPOAF_CHECK_ARG(act_dim >= 1 && act_dim <= kMaxAct && pred_dim >= 1 && pred_dim <= kMaxAct,
+                    "ppoaf_head_evaluate: widths must be in [1, %d]", kMaxAct);
+    PPOAF_CHECK_ARG(n_rows >= 0, "ppoaf_head_evaluate: n_rows < 0");
+    if (n_rows == 0) return 0;
+    const dim3 grid((n_rows + 127) / 128), block(128);
+    if (head == PPOAF_HEAD_GAUSSIAN_TANH)
+        head_evaluate_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(
+            actor_out, pred_dim, log_std, min_std, static_cast<const float*>(actions), act_dim, n_rows, log_prob_out, entropy_out);
+    else
+        multi_categorical_evaluate_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(
+            actor_out, pred_dim, 1ull << (pred_dim - 1), static_cast<const int64_t*>(actions), act_dim, n_rows,
+            log_prob_out, entropy_out);
+    PPOAF_CHECK_LAUNCH("ppoaf_head_evaluate");
+    return 0;
+}
 
 extern "C" int ppoaf_multi_categorical_evaluate(const float* actor_out, int32_t pred_dim, uint32_t section_ends_lo,
                                                 uint32_t section_ends_hi, const int64_t* actions_i64, int32_t n_sections,
@@ -650,7 +451,7 @@ extern "C" int ppoaf_multi_categorical_sample(const float* probs, int32_t pred_d
     if (n_rows == 0) return 0;
     PPOAF_CHECK_ARG(noise != nullptr, "ppoaf_multi_categorical_sample: noise is required");
     multi_categorical_sample_kernel<<<(n_rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        probs, pred_dim, ends, noise, n_sections, n_rows, actions_out_i64, log_prob_out);
+        probs, pred_dim, ends, noise, n_sections, n_rows, actions_out_i64, log_prob_out, nullptr);
     PPOAF_CHECK_LAUNCH("ppoaf_multi_categorical_sample");
     return 0;
 }

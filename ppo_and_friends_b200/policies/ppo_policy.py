@@ -126,9 +126,9 @@ class PPOPolicy:
         else:
             self.bootstrap_clip = None
 
+        # a Discrete space is the multi-categorical head's table of one section
         if self.action_dtype == "discrete":
-            self.action_dim = 1
-            self.action_pred_size = int(action_space.n)
+            self.nvec = [int(action_space.n)]
         elif self.action_dtype == "multi-discrete":
             nvec = np.asarray(action_space.nvec)
             start = getattr(action_space, "start", None)
@@ -142,12 +142,13 @@ class PPOPolicy:
                 abort(f"ERROR: MultiDiscrete sum(nvec) = {int(nvec.sum())} exceeds the 64 actor outputs the "
                       "multi-categorical head supports.")
             self.nvec = [int(n) for n in nvec]
+        if self.action_dtype == "continuous":
+            self.action_dim = _flat_dim(action_space)
+            self.action_pred_size = self.action_dim
+        else:
             self.action_dim = len(self.nvec)
             self.action_pred_size = sum(self.nvec)
             self.section_ends = _lib.section_ends(self.nvec)
-        else:
-            self.action_dim = _flat_dim(action_space)
-            self.action_pred_size = self.action_dim
         self.actor_kw_args = dict(actor_kw_args)
         self.critic_kw_args = dict(critic_kw_args)
         self._ring = None
@@ -342,17 +343,13 @@ class PPOPolicy:
         values = self.critic(batch_critic_obs).reshape(-1)
         pred = self.actor(batch_obs)
         acts = batch_actions if torch.is_tensor(batch_actions) else torch.as_tensor(np.asarray(batch_actions))
-        if self.action_dtype == "multi-discrete":
-            acts = acts.to(self.device, torch.int64).reshape(pred.shape[0], -1).contiguous()
-            lp, ent = ops.multi_categorical_evaluate(pred, self.section_ends, acts)
-            return values, lp, ent
         if self.action_dtype == "continuous":
             acts = acts.to(self.device, torch.float32).reshape(pred.shape[0], -1).contiguous()
-            log_std = self.actor.state_dict()["distribution.log_std"]
+            lp, ent = ops.head_evaluate(self.head, pred, self.actor.state_dict()["distribution.log_std"], acts,
+                                        self.min_std)
         else:
             acts = acts.to(self.device, torch.int64).reshape(pred.shape[0], -1).contiguous()
-            log_std = None
-        lp, ent = ops.head_evaluate(self.head, pred, log_std, acts, self.min_std)
+            lp, ent = ops.multi_categorical_evaluate(pred, self.section_ends, acts)
         return values, lp, ent
 
     def get_rollout_actions(self, obs):
@@ -373,23 +370,18 @@ class PPOPolicy:
         n = t_obs.shape[0]
         discrete = self.action_dtype != "continuous"
         action_pred = self.actor(t_obs, softmax_out=discrete)
-        if self.action_dtype == "multi-discrete":
+        if discrete:
             noise = torch.cat([torch.empty(n, k, dtype=torch.float32).exponential_(1).reshape(-1) for k in self.nvec])
             act, lp = ops.multi_categorical_sample(action_pred, self.section_ends,
                                                    noise.to(self.device, non_blocking=True), len(self.nvec))
             raw = act
-        elif discrete:
-            noise = torch.empty(n, self.action_pred_size, dtype=torch.float32).exponential_(1)
-            log_std = dist_min = dist_max = None
         else:
             noise = torch.empty(n, self.action_dim, dtype=torch.float32).normal_(0, 1)
-            log_std = self.actor.state_dict()["distribution.log_std"]
             rescale = bool((self.dist_min != -1.0).any() or (self.dist_max != 1.0).any())
-            dist_min = self._dist_dev("min") if rescale else None
-            dist_max = self._dist_dev("max") if rescale else None
-        if self.action_dtype != "multi-discrete":
-            raw, act, lp = ops.head_sample(self.head, action_pred, log_std, noise.to(self.device, non_blocking=True),
-                                           self.min_std, dist_min, dist_max, act_dim=1 if discrete else self.action_dim)
+            raw, act, lp = ops.head_sample(self.head, action_pred, self.actor.state_dict()["distribution.log_std"],
+                                           noise.to(self.device, non_blocking=True), self.min_std,
+                                           self._dist_dev("min") if rescale else None,
+                                           self._dist_dev("max") if rescale else None, act_dim=self.action_dim)
         # the reference aborts on NaN observations / predictions (:758-775); one check of the results covers both
         bad = torch.isnan(t_obs).any() | torch.isnan(action_pred).any()
         # ONE device->host transfer and one sync per call: the three results and the NaN flag travel as one byte buffer

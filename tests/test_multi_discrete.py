@@ -237,7 +237,8 @@ def test_rollout_and_inference_actions_vs_restatement():
 @pytest.mark.gpu
 def test_one_section_reproduces_discrete_exactly(gemm_backend):
     """MultiDiscrete([n]) and Discrete(n) on the same rollout, seeds and initial weights: identical sampled actions,
-    log-probs, status scalars, parameters, Adam moments and dataset.values."""
+    log-probs, status scalars, parameters, Adam moments, dataset.values and PPOPolicy.evaluate's log-probs and
+    entropies."""
     from ppo_and_friends_b200.ppo import PPOUpdateState, _Loader, ppo_batch_train
     from ppo_and_friends_b200.synthetic import make_rollout
     out = {}
@@ -256,13 +257,14 @@ def test_one_section_reproduces_discrete_exactly(gemm_backend):
         loader = _Loader(ds, 128)
         for _ in range(2):
             ppo_batch_train(state, loader, "pol")
+        _, eval_lp, eval_ent = pol.evaluate(ds.critic_observations, ds.observations, ds.raw_actions)
         out[kind] = dict(act=act, lp=lp.numpy(), params=pol.nets.flat_params.cpu(), m=pol.nets.adam_m.cpu(),
                          v=pol.nets.adam_v.cpu(), values=ds.values.cpu(), status=dict(state.status_dict["pol"]),
-                         fused=pol._engine.fused)
+                         fused=pol._engine.fused, eval_lp=eval_lp.cpu(), eval_ent=eval_ent.cpu())
     a, b = out["discrete"], out["multi"]
     assert a["fused"] == b["fused"] == (gemm_backend == "fused")
     assert np.array_equal(a["act"], b["act"]) and np.array_equal(a["lp"], b["lp"])
-    for k in ("params", "m", "v", "values"):
+    for k in ("params", "m", "v", "values", "eval_lp", "eval_ent"):
         assert torch.equal(a[k], b[k]), k
     assert a["status"] == b["status"]
 
