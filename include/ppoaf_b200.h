@@ -37,8 +37,10 @@ enum { PPOAF_ACT_IDENTITY = 0, PPOAF_ACT_RELU = 1, PPOAF_ACT_LEAKY_RELU = 2, PPO
  * actor output row, then one torch Categorical(probs) per section of the row (renormalised, clamped to [eps, 1-eps]);
  * log-prob and entropy are the sums over the sections.  The sections are described by a 64-bit table of section
  * ends (bit c set: actor output c is the last of its section), so the row holds at most 64 outputs; nvec must be
- * 1-D with start = 0 and every entry >= 1. */
-enum { PPOAF_HEAD_GAUSSIAN_TANH = 0, PPOAF_HEAD_CATEGORICAL = 1, PPOAF_HEAD_MULTI_CATEGORICAL = 2 };
+ * 1-D with start = 0 and every entry >= 1.  PPOAF_HEAD_BERNOULLI (MultiBinary action spaces, BernoulliDistribution
+ * :134-196) is a restatement too: one torch Bernoulli(probs = sigmoid(actor output)) per output column, log-prob and
+ * entropy summed over the columns; act_dim = actor output width = number of columns (at most 64), fp32 0/1 actions. */
+enum { PPOAF_HEAD_GAUSSIAN_TANH = 0, PPOAF_HEAD_CATEGORICAL = 1, PPOAF_HEAD_MULTI_CATEGORICAL = 2, PPOAF_HEAD_BERNOULLI = 3 };
 
 int         ppoaf_abi_version(void);
 const char* ppoaf_last_error(void);
@@ -151,8 +153,9 @@ enum {
 typedef struct {
     ppoaf_mlp_desc actor, critic;
     int32_t head;                 /* PPOAF_HEAD_*                                                    */
-    int32_t act_dim;              /* stored action width: Da (Gaussian), 1 (Categorical index) or the
-                                     number of sections (Multi-categorical, one int64 index each)   */
+    int32_t act_dim;              /* stored action width: Da (Gaussian), 1 (Categorical index), the
+                                     number of sections (Multi-categorical, one int64 index each) or
+                                     the number of columns (Bernoulli, = actor output width)        */
     int32_t use_huber;            /* nn.HuberLoss(delta=10) instead of MSE (ppo.py:2416-2419)       */
     int32_t normalize_adv;        /* ppo.py:2325-2333                                               */
     int32_t normalize_values;     /* ppo.py:2299-2303                                               */
@@ -178,7 +181,7 @@ typedef struct {
     /* dataset in flat order (PPODataset attributes, utils/episode_info.py:823-912) */
     const float*   critic_obs;    /* [N, Dc] */
     const float*   obs;           /* [N, Do] */
-    const void*    raw_actions;   /* [N, act_dim] fp32 (Gaussian) or int64 (Categorical) */
+    const void*    raw_actions;   /* [N, act_dim] fp32 (Gaussian, Bernoulli 0/1) or int64 (Categorical) */
     const float*   advantages;    /* [N] */
     const float*   log_probs;     /* [N] */
     const float*   rewards_to_go; /* [N] */
@@ -253,7 +256,9 @@ int ppoaf_mlp_forward(const ppoaf_mlp_desc* net, const float* params, const floa
 
 /* P1  Action-head evaluation on its own (policies/ppo_policy.py:939-950): log-prob of `actions`
  * and entropy under the head parameterised by actor_out [n_rows, pred] (+ log_std for the
- * Gaussian head).  actions: fp32 [n_rows, act_dim] raw (pre-tanh) or int64 [n_rows, 1]. */
+ * Gaussian head).  actions: fp32 [n_rows, act_dim] raw (pre-tanh), int64 [n_rows, 1] (Categorical) or
+ * fp32 0/1 [n_rows, act_dim] (Bernoulli: actor_out holds the logits, pred = act_dim, log_std must be NULL;
+ * log-prob and entropy are summed over the columns). */
 int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std,
                         float min_std, const void* actions, int32_t act_dim, int32_t n_rows,
                         float* log_prob_out, float* entropy_out, void* stream);
@@ -261,9 +266,12 @@ int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t pred_dim, 
 /* "Next" row 1 (SURVEY §8f): rollout-time sampling, PPOPolicy.get_rollout_actions (policies/ppo_policy.py:729-794,
  * networks/distributions.py:518-655, 199-249).  `noise` holds the draws of the HOST generator in the order the reference's
  * CPU sampling consumes them -- N(0,1) [n_rows, act_dim] for the Gaussian head, Exp(1) [n_rows, pred_dim] for the
- * Categorical head (aten multinomial's one-sample path) -- so the sampled actions are the reference's.  Outputs:
- * raw_action / action fp32 [n_rows, act_dim] (Gaussian; action = tanh(raw) mapped to [dist_min, dist_max] when given) or
- * int64 [n_rows, 1] (Categorical), log_prob fp32 [n_rows]. */
+ * Categorical head (aten multinomial's one-sample path), U[0,1) [n_rows, act_dim] for the Bernoulli head (torch.rand,
+ * as Bernoulli(probs).sample() draws it) -- so the sampled actions are the reference's.  Outputs:
+ * raw_action / action fp32 [n_rows, act_dim] (Gaussian; action = tanh(raw) mapped to [dist_min, dist_max] when given),
+ * int64 [n_rows, 1] (Categorical) or fp32 0/1 [n_rows, act_dim] (Bernoulli: action = [u < sigmoid(actor_out)], both
+ * outputs get the same actions, each may be NULL; pred = act_dim; log_std, dist_min and dist_max must be NULL; noise of
+ * 0.5 everywhere gives the deterministic action [p > 0.5]), log_prob fp32 [n_rows] (summed over the Bernoulli columns). */
 int ppoaf_head_sample(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std, float min_std,
                       const float* noise, const float* dist_min, const float* dist_max, int32_t act_dim,
                       int32_t n_rows, void* raw_action_out, void* action_out, float* log_prob_out, void* stream);

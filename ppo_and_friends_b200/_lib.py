@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(_HERE, "csrc", "libppoaf_b200.so")
 
 MAX_LAYERS = 8
 ACT_IDS = {"identity": 0, "relu": 1, "leaky_relu": 2, "tanh": 3}
-HEAD_GAUSSIAN_TANH, HEAD_CATEGORICAL, HEAD_MULTI_CATEGORICAL = 0, 1, 2
+HEAD_GAUSSIAN_TANH, HEAD_CATEGORICAL, HEAD_MULTI_CATEGORICAL, HEAD_BERNOULLI = 0, 1, 2, 3
 
 HP = dict(LR=0, ENTROPY_WEIGHT=1, SURR_CLIP=2, GRAD_CLIP=3, KL_WEIGHT=4, VF_CLIP=5, BETA1=6, BETA2=7,
           ADAM_EPS=8, INV_WORLD=9, COUNT=16)

@@ -681,7 +681,7 @@ __device__ __forceinline__ void loss_phase(const LossArgs& a, int cur, float* s_
         const float* pred = hs.pred + warp * kFusedPredLd;
         float* dpred = a.d_actor_out + int64_t(i) * (a.d_actor_ld ? a.d_actor_ld : a.pred_dim);
         float* sdp = hs.dpred + warp * kFusedPredLd;
-        actor_head_loss<true>(a, gaussian, true, gl, j, pred, dpred, sdp, s_sd, adv, lp_old, inv_b, w_ent, clip_lo, clip_hi, sc,
+        actor_head_loss<true>(a, a.head, true, gl, j, pred, dpred, sdp, s_sd, adv, lp_old, inv_b, w_ent, clip_lo, clip_hi, sc,
                               dsd, bad_value);
 
         if (dbg) dbg[4] = clock64();

@@ -1,5 +1,5 @@
 // Fused PPO loss, forward + backward, for one minibatch (reference ppo.py:2299-2438 with the
-// distribution arithmetic of networks/distributions.py:491-558,694 and torch's Normal/Categorical).
+// distribution arithmetic of networks/distributions.py:491-558,694 and torch's Normal/Categorical/Bernoulli).
 // One WARP per sample (each lane owns action dims l, l + 32 and 8 hidden columns); nothing but the gradients w.r.t. the two network outputs, d(log_std) and
 // six scalars ever reaches HBM.  Reductions are deterministic: per-CTA partials in fp64, summed in
 // CTA order by the last CTA to finish (self-resetting ticket).
@@ -139,7 +139,7 @@ __global__ void __launch_bounds__(kLossThreads) ppo_loss_kernel(const LossArgs a
     const float* pred = FUSED ? hs.pred + smp * kFusedPredLd : a.actor_out + int64_t(live ? i : 0) * a.pred_dim;
     float* dpred = a.d_actor_out + int64_t(live ? i : 0) * a.pred_dim;
     float* sdp = hs.dpred + smp * kFusedPredLd;                      // FUSED: dL/d(actor out) kept for the head's dX
-    actor_head_loss<FUSED>(a, gaussian, live, gl, j, pred, dpred, sdp, s_sd, adv, lp_old, inv_b, w_ent, clip_lo, clip_hi,
+    actor_head_loss<FUSED>(a, a.head, live, gl, j, pred, dpred, sdp, s_sd, adv, lp_old, inv_b, w_ent, clip_lo, clip_hi,
                            sc, dsd, bad_value);
 
     LOSS_STAMP(4);
@@ -375,6 +375,45 @@ multi_categorical_sample_kernel(const float* __restrict__ probs, int pred_dim, u
     lp_out[i] = lp;
 }
 
+// Bernoulli (MultiBinary) evaluation: log-prob of fp32 0/1 actions [n_rows, k] and entropy, summed over the k columns,
+// from the actor's logits [n_rows, k]
+__global__ void bernoulli_evaluate_kernel(const float* __restrict__ actor_out, int k, const float* __restrict__ actions,
+                                          int n_rows, float* __restrict__ lp_out, float* __restrict__ ent_out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_rows) return;
+    const float* z = actor_out + int64_t(i) * k;
+    const float* x = actions + int64_t(i) * k;
+    float lp = 0.f, h = 0.f;
+    for (int c = 0; c < k; ++c) {
+        const float p = sigmoid_f(z[c]), l = bernoulli_logit(p), ls = log_sigmoid(l);
+        lp += ls - (1.f - x[c]) * l;
+        h += (1.f - p) * l - ls;
+    }
+    lp_out[i] = lp;
+    if (ent_out) ent_out[i] = h;
+}
+
+// Bernoulli sampling from the actor's logits [n_rows, k]: noise holds the host generator's U[0,1) draws [n_rows, k]
+// (torch.rand, which Bernoulli(probs).sample() consumes the same way) and a = (u < sigmoid(z)) as fp32 0/1; all 0.5
+// gives the deterministic action [p > 0.5].  Writes whichever of raw_out / act_out is given, and the summed log-prob.
+__global__ void bernoulli_sample_kernel(const float* __restrict__ actor_out, int k, const float* __restrict__ noise,
+                                        int n_rows, float* __restrict__ raw_out, float* __restrict__ act_out,
+                                        float* __restrict__ lp_out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_rows) return;
+    const float* z = actor_out + int64_t(i) * k;
+    const float* u = noise + int64_t(i) * k;
+    float lp = 0.f;
+    for (int c = 0; c < k; ++c) {
+        const float p = sigmoid_f(z[c]), l = bernoulli_logit(p);
+        const float x = u[c] < p ? 1.f : 0.f;
+        if (raw_out) raw_out[int64_t(i) * k + c] = x;
+        if (act_out) act_out[int64_t(i) * k + c] = x;
+        lp += log_sigmoid(l) - (1.f - x) * l;
+    }
+    lp_out[i] = lp;
+}
+
 }  // namespace ppoaf
 
 extern "C" int ppoaf_head_sample(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std,
@@ -382,17 +421,27 @@ extern "C" int ppoaf_head_sample(int32_t head, const float* actor_out, int32_t p
                                  int32_t act_dim, int32_t n_rows, void* raw_action_out, void* action_out,
                                  float* log_prob_out, void* stream) {
     using namespace ppoaf;
-    PPOAF_CHECK_ARG(head == PPOAF_HEAD_GAUSSIAN_TANH || head == PPOAF_HEAD_CATEGORICAL, "ppoaf_head_sample: unknown head");
+    PPOAF_CHECK_ARG(head == PPOAF_HEAD_GAUSSIAN_TANH || head == PPOAF_HEAD_CATEGORICAL || head == PPOAF_HEAD_BERNOULLI,
+                    "ppoaf_head_sample: unknown head");
     PPOAF_CHECK_ARG(act_dim >= 1 && act_dim <= kMaxAct && pred_dim >= 1 && pred_dim <= kMaxAct,
                     "ppoaf_head_sample: widths must be in [1, %d]", kMaxAct);
     PPOAF_CHECK_ARG(n_rows >= 0 && noise != nullptr, "ppoaf_head_sample: bad arguments");
     PPOAF_CHECK_ARG((dist_min == nullptr) == (dist_max == nullptr), "ppoaf_head_sample: give both range bounds or neither");
+    if (head == PPOAF_HEAD_BERNOULLI) {
+        PPOAF_CHECK_ARG(pred_dim == act_dim, "ppoaf_head_sample: Bernoulli actor output width must equal act_dim");
+        PPOAF_CHECK_ARG(log_std == nullptr && dist_min == nullptr,
+                        "ppoaf_head_sample: the Bernoulli head takes no log_std and no range bounds");
+    }
     if (n_rows == 0) return 0;
     const dim3 grid((n_rows + 127) / 128), block(128);
     if (head == PPOAF_HEAD_GAUSSIAN_TANH)
         head_sample_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(
             actor_out, pred_dim, log_std, min_std, noise, dist_min, dist_max, act_dim, n_rows, static_cast<float*>(raw_action_out),
             static_cast<float*>(action_out), log_prob_out);
+    else if (head == PPOAF_HEAD_BERNOULLI)
+        bernoulli_sample_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(
+            actor_out, act_dim, noise, n_rows, static_cast<float*>(raw_action_out), static_cast<float*>(action_out),
+            log_prob_out);
     else
         multi_categorical_sample_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(
             actor_out, pred_dim, 1ull << (pred_dim - 1), noise, 1, n_rows, static_cast<int64_t*>(action_out), log_prob_out,
@@ -405,15 +454,23 @@ extern "C" int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t
                                    float min_std, const void* actions, int32_t act_dim, int32_t n_rows,
                                    float* log_prob_out, float* entropy_out, void* stream) {
     using namespace ppoaf;
-    PPOAF_CHECK_ARG(head == PPOAF_HEAD_GAUSSIAN_TANH || head == PPOAF_HEAD_CATEGORICAL, "ppoaf_head_evaluate: unknown head");
+    PPOAF_CHECK_ARG(head == PPOAF_HEAD_GAUSSIAN_TANH || head == PPOAF_HEAD_CATEGORICAL || head == PPOAF_HEAD_BERNOULLI,
+                    "ppoaf_head_evaluate: unknown head");
     PPOAF_CHECK_ARG(act_dim >= 1 && act_dim <= kMaxAct && pred_dim >= 1 && pred_dim <= kMaxAct,
                     "ppoaf_head_evaluate: widths must be in [1, %d]", kMaxAct);
     PPOAF_CHECK_ARG(n_rows >= 0, "ppoaf_head_evaluate: n_rows < 0");
+    if (head == PPOAF_HEAD_BERNOULLI) {
+        PPOAF_CHECK_ARG(pred_dim == act_dim, "ppoaf_head_evaluate: Bernoulli actor output width must equal act_dim");
+        PPOAF_CHECK_ARG(log_std == nullptr, "ppoaf_head_evaluate: the Bernoulli head takes no log_std");
+    }
     if (n_rows == 0) return 0;
     const dim3 grid((n_rows + 127) / 128), block(128);
     if (head == PPOAF_HEAD_GAUSSIAN_TANH)
         head_evaluate_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(
             actor_out, pred_dim, log_std, min_std, static_cast<const float*>(actions), act_dim, n_rows, log_prob_out, entropy_out);
+    else if (head == PPOAF_HEAD_BERNOULLI)
+        bernoulli_evaluate_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(
+            actor_out, act_dim, static_cast<const float*>(actions), n_rows, log_prob_out, entropy_out);
     else
         multi_categorical_evaluate_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(
             actor_out, pred_dim, 1ull << (pred_dim - 1), static_cast<const int64_t*>(actions), act_dim, n_rows,

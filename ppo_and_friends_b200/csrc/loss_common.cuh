@@ -1,6 +1,6 @@
 // The per-sample PPO loss, shared by the stand-alone loss kernel (loss.cu) and the LOSS phase of the persistent
 // whole-step kernel (fused_step.cu): widths, the partial-sum layout, the action-head arithmetic (reference
-// ppo.py:2342-2410 with networks/distributions.py:491-558, 694 and torch's Normal / Categorical), the fused head layers
+// ppo.py:2342-2410 with networks/distributions.py:491-558, 694 and torch's Normal / Categorical / Bernoulli), the fused head layers
 // and the reductions.  The two kernels differ only in how they load their inputs and how their CTAs meet.
 #pragma once
 #include "internal.h"
@@ -100,6 +100,15 @@ __device__ __forceinline__ void section_sum(const float (&v)[kPerLane], const in
     }
 }
 
+// Bernoulli (MultiBinary) columns, torch's Bernoulli(probs = sigmoid(z)) restated (DESIGN §4): q = clamp(p, eps,
+// 1 - eps), l = log q - log1p(-q); log_prob(x) = logsigmoid(l) - (1 - x) l, entropy = (1 - p) l - logsigmoid(l)
+__device__ __forceinline__ float sigmoid_f(float z) { return 1.f / (1.f + expf(-z)); }
+__device__ __forceinline__ float bernoulli_logit(float p) {
+    const float q = fminf(fmaxf(p, kCatEps), 1.f - kCatEps);
+    return logf(q) - log1pf(-q);
+}
+__device__ __forceinline__ float log_sigmoid(float l) { return fminf(l, 0.f) - log1pf(expf(-fabsf(l))); }
+
 // std = max(softplus(log_std), min_std) (distributions.py:514-515) and dstd = d std / d log_std (torch's max splits the
 // gradient evenly on a tie)
 __device__ __forceinline__ float std_of_log_std(float ls, float min_std, float& dstd) {
@@ -127,15 +136,16 @@ __device__ __forceinline__ float ppo_surrogate(float lp, float ent, float lp_old
 
 // Action-head part of the loss for one sample shared by the 32 lanes of a warp (lane gl owns dims gl, gl + 32):
 // log-prob, entropy, ratio, clipped surrogate and their gradients w.r.t. the head outputs (written to dpred, and
-// to sdp when the head layer itself is fused) and w.r.t. std (dsd).  Lane 0 receives the sample's scalars in sc.
+// to sdp when the head layer itself is fused) and w.r.t. std (dsd, Gaussian head only).  Lane 0 receives the sample's
+// scalars in sc.  head: PPOAF_HEAD_*.
 template <bool FUSED>
-__device__ __forceinline__ void actor_head_loss(const LossArgs& a, bool gaussian, bool live, int gl, int64_t j,
+__device__ __forceinline__ void actor_head_loss(const LossArgs& a, int head, bool live, int gl, int64_t j,
                                                 const float* pred, float* dpred, float* sdp, const float* s_sd,
                                                 float adv, float lp_old, float inv_b, float w_ent, float clip_lo,
                                                 float clip_hi, float (&sc)[kLossScalars], float (&dsd)[kPerLane],
                                                 float& bad_value) {
     const float g_ent = -w_ent * inv_b;                               // dL/dH_i
-    if (gaussian) {
+    if (head == PPOAF_HEAD_GAUSSIAN_TANH) {
         const float* x = reinterpret_cast<const float*>(a.raw_actions) + j * a.act_dim;
         float mu[kPerLane], z[kPerLane], on[kPerLane], one[kPerLane], thm[kPerLane];
         float nsum = 0.f, slog = 0.f, ensum = 0.f, eslog = 0.f;
@@ -176,6 +186,45 @@ __device__ __forceinline__ void actor_head_loss(const LossArgs& a, bool gaussian
                 if constexpr (FUSED) sdp[d] = gd;
                 // dlp/dsd = z^2/sd^3 - 1/sd ; dH/dsd = 1/sd
                 dsd[k] = g_lp * on[k] * ((z[k] * z[k]) / (var * sd) - 1.f / sd) + g_ent * one[k] * (1.f / sd);
+            }
+        }
+    } else if (head == PPOAF_HEAD_BERNOULLI) {
+        // independent columns p = sigmoid(z) (bernoulli_logit / log_sigmoid above); log-prob and entropy are the sums
+        // over the act_dim columns.  Backward with s = sigmoid(l) and m = [eps <= p <= 1 - eps] (the clamp passes the
+        // gradient on its bounds): dL/dp = g_lp (x - s) m / (q (1 - q)) + g_ent ((s - p) m / (q (1 - q)) - l), then
+        // dL/dz = dL/dp p (1 - p).
+        const float* x = reinterpret_cast<const float*>(a.raw_actions) + j * a.act_dim;
+        float p[kPerLane], l[kPerLane], xv[kPerLane];
+        float lpa = 0.f, h = 0.f;
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) {
+            const int c = gl + k * kG;
+            p[k] = l[k] = xv[k] = 0.f;
+            if (c < a.act_dim && live) {
+                const float zc = pred[c];
+                bad_value = fmaxf(bad_value, isnan(zc) ? 1.f : 0.f);
+                xv[k] = x[c];
+                p[k] = sigmoid_f(zc);
+                l[k] = bernoulli_logit(p[k]);
+                const float ls = log_sigmoid(l[k]);
+                lpa += ls - (1.f - xv[k]) * l[k];
+                h += (1.f - p[k]) * l[k] - ls;
+            }
+        }
+        const float lp = group_sum(lpa);
+        const float ent = group_sum(h);
+        const float g_lp = ppo_surrogate(lp, ent, lp_old, adv, inv_b, clip_lo, clip_hi, gl == 0 && live, sc);
+#pragma unroll
+        for (int k = 0; k < kPerLane; ++k) {
+            const int c = gl + k * kG;
+            if (c < a.act_dim && live) {
+                const float q = fminf(fmaxf(p[k], kCatEps), 1.f - kCatEps);
+                const float r = (p[k] >= kCatEps && p[k] <= 1.f - kCatEps) ? 1.f / (q * (1.f - q)) : 0.f;
+                const float s = sigmoid_f(l[k]);
+                const float gp = g_lp * (xv[k] - s) * r + g_ent * ((s - p[k]) * r - l[k]);
+                const float gd = gp * (p[k] * (1.f - p[k]));
+                dpred[c] = gd;
+                if constexpr (FUSED) sdp[c] = gd;
             }
         }
     } else {

@@ -101,10 +101,13 @@ int check_cfg(const ppoaf_update_cfg* cfg, const char* who) {
     if (check_mlp_desc(&cfg->actor, who) || check_mlp_desc(&cfg->critic, who)) return 1;
     PPOAF_CHECK_ARG(cfg->critic.dims[cfg->critic.n_layers] == 1, "%s: critic output width must be 1", who);
     PPOAF_CHECK_ARG(cfg->head == PPOAF_HEAD_GAUSSIAN_TANH || cfg->head == PPOAF_HEAD_CATEGORICAL ||
-                    cfg->head == PPOAF_HEAD_MULTI_CATEGORICAL, "%s: unknown head", who);
+                    cfg->head == PPOAF_HEAD_MULTI_CATEGORICAL || cfg->head == PPOAF_HEAD_BERNOULLI, "%s: unknown head", who);
     if (cfg->head == PPOAF_HEAD_GAUSSIAN_TANH)
         PPOAF_CHECK_ARG(cfg->actor.dims[cfg->actor.n_layers] == cfg->act_dim,
                         "%s: Gaussian actor output width must equal act_dim", who);
+    else if (cfg->head == PPOAF_HEAD_BERNOULLI)
+        PPOAF_CHECK_ARG(cfg->actor.dims[cfg->actor.n_layers] == cfg->act_dim,
+                        "%s: Bernoulli actor output width must equal act_dim (one column per binary action)", who);
     else if (cfg->head == PPOAF_HEAD_MULTI_CATEGORICAL)
         PPOAF_CHECK_ARG(section_table_ok(cfg_section_ends(cfg), cfg->actor.dims[cfg->actor.n_layers], cfg->act_dim),
                         "%s: bad multi-categorical section table (must be nonzero, its highest set bit must be the last "

@@ -149,8 +149,7 @@ def head_sample(head, actor_out, log_std, noise, min_std=0.01, dist_min=None, di
     """(raw_action, action, log_prob) from the actor output and host-drawn noise (see ppoaf_head_sample)."""
     n, pred = actor_out.shape
     dev = actor_out.device
-    gaussian = head == _lib.HEAD_GAUSSIAN_TANH
-    if gaussian:
+    if head in (_lib.HEAD_GAUSSIAN_TANH, _lib.HEAD_BERNOULLI):
         raw = torch.empty((n, act_dim), dtype=torch.float32, device=dev)
         act = torch.empty((n, act_dim), dtype=torch.float32, device=dev)
     else:

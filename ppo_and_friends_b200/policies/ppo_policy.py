@@ -17,7 +17,10 @@ no counterpart because the losses never exist as tensors — the fused step in p
 MultiDiscrete action spaces take a multi-categorical head (reference MultiCategoricalDistribution,
 networks/distributions.py:272-438, restated: softmax over the whole actor output, one Categorical per section, log-prob
 and entropy summed over the sections); `nvec` must be 1-D with `start` = 0, every entry >= 1 and sum(nvec) <= 64.
-Out of scope (raise): LSTM networks, ICM, MAT, Bernoulli/Mixed action heads.
+MultiBinary action spaces take a Bernoulli head (reference BernoulliDistribution, networks/distributions.py:134-196,
+restated: one Bernoulli(probs=sigmoid(actor output)) per column, log-prob and entropy summed over the columns, fp32 0/1
+actions); the shape must be 1-D with 1 <= n <= 64.
+Out of scope (raise): LSTM networks, ICM, MAT, Mixed action heads.
 """
 import os
 
@@ -115,9 +118,9 @@ class PPOPolicy:
         self.action_dtype = space_dtype_str(action_space)
         if self.action_dtype == "unknown":
             abort(f"ERROR: unknown action type: {type(action_space)} with dtype {getattr(action_space, 'dtype', None)}.")
-        if self.action_dtype not in ("continuous", "discrete", "multi-discrete"):
+        if self.action_dtype not in ("continuous", "discrete", "multi-discrete", "multi-binary"):
             abort(f"ERROR: {self.action_dtype} action heads are outside the B200 update path "
-                  "(Gaussian, Categorical and MultiCategorical only, SURVEY.md §2 row 8).")
+                  "(Gaussian, Categorical, MultiCategorical and Bernoulli only, SURVEY.md §2 row 8).")
         rank_print("{} policy using {} actions.".format(self.name, self.action_dtype))
 
         self.have_bootstrap_clip = bootstrap_clip is not None
@@ -142,7 +145,14 @@ class PPOPolicy:
                 abort(f"ERROR: MultiDiscrete sum(nvec) = {int(nvec.sum())} exceeds the 64 actor outputs the "
                       "multi-categorical head supports.")
             self.nvec = [int(n) for n in nvec]
-        if self.action_dtype == "continuous":
+        elif self.action_dtype == "multi-binary":
+            shape = tuple(getattr(action_space, "shape", ()) or ())
+            if len(shape) != 1:
+                abort(f"ERROR: MultiBinary spaces must be 1-D on the B200 path, got shape {shape}.")
+            if not 1 <= int(shape[0]) <= 64:
+                abort(f"ERROR: MultiBinary n = {int(shape[0])} is outside the 1 .. 64 actor outputs the Bernoulli "
+                      "head supports.")
+        if self.action_dtype in ("continuous", "multi-binary"):
             self.action_dim = _flat_dim(action_space)
             self.action_pred_size = self.action_dim
         else:
@@ -228,7 +238,7 @@ class PPOPolicy:
     @property
     def head(self):
         return {"continuous": _lib.HEAD_GAUSSIAN_TANH, "discrete": _lib.HEAD_CATEGORICAL,
-                "multi-discrete": _lib.HEAD_MULTI_CATEGORICAL}[self.action_dtype]
+                "multi-discrete": _lib.HEAD_MULTI_CATEGORICAL, "multi-binary": _lib.HEAD_BERNOULLI}[self.action_dtype]
 
     def to(self, device):
         self.device = torch.device(device)
@@ -245,7 +255,7 @@ class PPOPolicy:
         if self._ring is None or self._ring.E != E or self._ring.A != len(self.agent_ids):
             self._ring = RolloutRing(self.device, E, len(self.agent_ids), _flat_dim(self.actor_obs_space),
                                      _flat_dim(self.critic_obs_space), self.action_dim,
-                                     self.action_dtype != "continuous",
+                                     self.action_dtype in ("discrete", "multi-discrete"),
                                      capacity_steps=max(64, getattr(self, "rollout_steps_hint", 64)))
         self._ring.reset()
         if self.dataset is not None:
@@ -347,6 +357,9 @@ class PPOPolicy:
             acts = acts.to(self.device, torch.float32).reshape(pred.shape[0], -1).contiguous()
             lp, ent = ops.head_evaluate(self.head, pred, self.actor.state_dict()["distribution.log_std"], acts,
                                         self.min_std)
+        elif self.action_dtype == "multi-binary":
+            acts = acts.to(self.device, torch.float32).reshape(pred.shape[0], -1).contiguous()
+            lp, ent = ops.head_evaluate(self.head, pred, None, acts)
         else:
             acts = acts.to(self.device, torch.int64).reshape(pred.shape[0], -1).contiguous()
             lp, ent = ops.multi_categorical_evaluate(pred, self.section_ends, acts)
@@ -359,8 +372,8 @@ class PPOPolicy:
         mapping and the log-prob run on the device; the random draws come from torch's global CPU generator in exactly
         the order the reference's CPU sampling consumes them (Normal.sample -> normal_(0, 1) of shape [n, act_dim];
         Categorical.sample -> exponential_(1) of shape [n, n_actions]; MultiDiscrete: one Categorical.sample per section,
-        in section order), so a seeded run reproduces the reference's actions.  Returns numpy raw_action / action and a
-        CPU log_prob tensor, like the reference.
+        in section order; MultiBinary: Bernoulli.sample -> rand of shape [n, n_binary]), so a seeded run reproduces the
+        reference's actions.  Returns numpy raw_action / action and a CPU log_prob tensor, like the reference.
         """
         obs = np.asarray(obs) if not torch.is_tensor(obs) else obs
         if len(obs.shape) < 2:
@@ -368,13 +381,17 @@ class PPOPolicy:
                   "instead received shape {}.".format(tuple(obs.shape)))
         t_obs = torch.as_tensor(obs, dtype=torch.float32).to(self.device).reshape(obs.shape[0], -1).contiguous()
         n = t_obs.shape[0]
-        discrete = self.action_dtype != "continuous"
+        discrete = self.action_dtype in ("discrete", "multi-discrete")
         action_pred = self.actor(t_obs, softmax_out=discrete)
         if discrete:
             noise = torch.cat([torch.empty(n, k, dtype=torch.float32).exponential_(1).reshape(-1) for k in self.nvec])
             act, lp = ops.multi_categorical_sample(action_pred, self.section_ends,
                                                    noise.to(self.device, non_blocking=True), len(self.nvec))
             raw = act
+        elif self.action_dtype == "multi-binary":
+            noise = torch.rand(n, self.action_dim, dtype=torch.float32)
+            raw, act, lp = ops.head_sample(self.head, action_pred, None, noise.to(self.device, non_blocking=True),
+                                           act_dim=self.action_dim)
         else:
             noise = torch.empty(n, self.action_dim, dtype=torch.float32).normal_(0, 1)
             rescale = bool((self.dist_min != -1.0).any() or (self.dist_max != 1.0).any())
@@ -407,8 +424,8 @@ class PPOPolicy:
         """
         Environment actions only, for `ppoaf test` (reference policies/ppo_policy.py:796-888; ppo.py:972, 1023).
         deterministic: tanh(mean) mapped to the action range (Gaussian, networks/distributions.py:596-631), the arg-max
-        class (Categorical, :251-269) or the arg-max class of every section ([n, n_sections], MultiDiscrete); otherwise a
-        sample drawn with the rollout protocol.
+        class (Categorical, :251-269), the arg-max class of every section ([n, n_sections], MultiDiscrete) or
+        [sigmoid(z) > 0.5] as fp32 0/1 ([n, n_binary], MultiBinary); otherwise a sample drawn with the rollout protocol.
         """
         obs = np.asarray(obs) if not torch.is_tensor(obs) else obs
         if len(obs.shape) < 2:
@@ -417,13 +434,17 @@ class PPOPolicy:
         if not deterministic:
             return torch.as_tensor(self.get_rollout_actions(obs)[1])
         t_obs = torch.as_tensor(obs, dtype=torch.float32).to(self.device).reshape(obs.shape[0], -1).contiguous()
-        discrete = self.action_dtype != "continuous"
+        discrete = self.action_dtype in ("discrete", "multi-discrete")
         action_pred = self.actor(t_obs, softmax_out=discrete)
         if self.action_dtype == "multi-discrete":
             return torch.stack([s.argmax(dim=-1) for s in action_pred.split(self.nvec, dim=1)], dim=1).cpu()
         if discrete:
             return torch.argmax(action_pred, dim=-1).cpu()
         n = t_obs.shape[0]
+        if self.action_dtype == "multi-binary":
+            half = torch.full((n, self.action_dim), 0.5, dtype=torch.float32, device=self.device)   # u = 0.5: p > 0.5
+            _, act, _ = ops.head_sample(self.head, action_pred, None, half, act_dim=self.action_dim)
+            return act.cpu()
         rescale = bool((self.dist_min != -1.0).any() or (self.dist_max != 1.0).any())
         zeros = torch.zeros(n, self.action_dim, dtype=torch.float32, device=self.device)   # no noise: raw = mean
         _, act, _ = ops.head_sample(self.head, action_pred, self.actor.state_dict()["distribution.log_std"], zeros,

@@ -1,6 +1,6 @@
 """
-Minimal Box / Discrete / MultiDiscrete stand-ins with the attributes the update path reads from gymnasium spaces
-(`shape`, `dtype`, `low`, `high`, `n`, `nvec`, `start`).  gymnasium is not part of this image; real gymnasium
+Minimal Box / Discrete / MultiDiscrete / MultiBinary stand-ins with the attributes the update path reads from gymnasium
+spaces (`shape`, `dtype`, `low`, `high`, `n`, `nvec`, `start`).  gymnasium is not part of this image; real gymnasium
 spaces work unchanged because the policy only duck-types these attributes.
 """
 import numpy as np
@@ -29,3 +29,12 @@ class MultiDiscrete:
         self.start = None if start is None else np.asarray(start, dtype=np.int64)
         self.shape = self.nvec.shape
         self.dtype = np.dtype(np.int64)
+
+
+class MultiBinary:
+    """`n` binary actions; like gymnasium, `n` may also be a shape (which the policy refuses unless it is 1-D)."""
+
+    def __init__(self, n):
+        self.n = n
+        self.shape = tuple(int(d) for d in np.atleast_1d(n))
+        self.dtype = np.dtype(np.int8)
