@@ -38,6 +38,9 @@ void configure_gemm_kernels();
 int64_t param_layout(const ppoaf_mlp_desc* net, int32_t log_std_dim, int64_t* offsets);
 int check_mlp_desc(const ppoaf_mlp_desc* net, const char* who);
 
+// stats.cu — opts the column-moments kernel into the shared memory of its widest plan
+void configure_stats_kernels();
+
 // loss.cu
 struct LossArgs {
     const float* actor_out;      // [batch, pred]  mean (Gaussian) or logits (Categorical)

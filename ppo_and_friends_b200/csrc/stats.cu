@@ -5,7 +5,7 @@
 // rows (coalesced 128-bit loads, 4 rows in flight), keeping fp32 Welford state; partials are merged
 // with Chan's formula in fp64: across threadIdx.y in shared memory, across CTAs by a second kernel
 // in which one warp per column tree-merges the CTA partials with shuffles.
-#include "common.cuh"
+#include "internal.h"
 
 namespace ppoaf {
 
@@ -71,8 +71,10 @@ __device__ __forceinline__ void welford4(float4 x, float rn, float4& mean, float
 // partial[(block * width + col) * 3 + {0,1,2}] = n, mean, M2
 // fold > 1 (narrow rows folded `fold` at a time into super-rows of `width` floats): the CTA also merges the fold copies of
 // every true column, so it publishes `dim` triples instead of `width` and the finalize kernel has fold x fewer to fold.
-__global__ void moments_partial_kernel(const float4* __restrict__ x, int64_t rows, int vec, int dim, int fold,
-                                       double* __restrict__ partial) {
+// Rows of 388..512 floats run it with 1024 threads, which leaves at most 64 registers a thread.
+__global__ void __launch_bounds__(1024)
+moments_partial_kernel(const float4* __restrict__ x, int64_t rows, int vec, int dim, int fold,
+                       double* __restrict__ partial) {
     extern __shared__ double s_part[];  // [blockDim.y][vec*4][2] mean, m2 ; counts in s_cnt
     __shared__ float s_cnt[kStatRowsPerBlock];
     const int g = threadIdx.x, y = threadIdx.y;
@@ -373,7 +375,8 @@ __global__ void reward_norm_triples_kernel(const float* __restrict__ rewards, co
     for (int e = 0; e < E; ++e) { const double d = running_reward[e] - mean; m2 += d * d; }
     for (int e = 0; e < E; ++e) {
         const double old = running_reward[e];
-        const double nw = old * gamma + double(rewards[e]);
+        // rounded product then rounded sum, as the reference's numpy does: a contracted fma would drift from it
+        const double nw = __dadd_rn(__dmul_rn(old, gamma), double(rewards[e]));
         running_reward[e] = nw;
         const double new_mean = mean + (nw - old) / double(E);
         m2 += (nw - old) * ((nw - new_mean) + (old - mean));
@@ -394,6 +397,22 @@ __global__ void reward_scale_clip_kernel(const float* __restrict__ r, const doub
     float v = float(double(r[i]) / sd);
     if (lo < hi) v = fminf(fmaxf(v, lo), hi);
     y[i] = v;
+}
+
+// The widest vectorised moments plan is fold = 1 with blockDim.x * kStatRowsPerBlock = 1024 threads, i.e. rows of 512
+// floats, whose per-row-lane (mean, M2) partials take 64 KB of dynamic shared memory: more than the 48 KB a kernel may
+// use without opting in.
+constexpr int kMaxVecWidth = 4 * 1024 / kStatRowsPerBlock;
+constexpr size_t kMomentsSmemMax = size_t(kStatRowsPerBlock) * kMaxVecWidth * 2 * sizeof(double);
+static_assert(size_t(kStatRowsPerBlock) * kMaxFoldWidth * 2 * sizeof(double) + kMaxFoldWidth * sizeof(Moments) <=
+              kMomentsSmemMax, "folded plans need more shared memory than the widest unfolded one");
+
+// Called from ppoaf_runtime_init (so that the attribute call normally happens before any stream capture) and, for callers
+// of the C ABI that never initialise the runtime, lazily by the first ppoaf_batch_moments.
+static bool g_stats_configured = false;
+void configure_stats_kernels() {
+    g_stats_configured = true;
+    cudaFuncSetAttribute(moments_partial_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kMomentsSmemMax));
 }
 
 }  // namespace ppoaf
@@ -440,6 +459,7 @@ extern "C" int ppoaf_batch_moments(const float* x, int64_t n_rows, int32_t dim, 
                     "ppoaf_batch_moments: workspace too small");
     PPOAF_CHECK_ARG(reinterpret_cast<uintptr_t>(workspace) % 8 == 0, "ppoaf_batch_moments: workspace alignment");
     double* partial = reinterpret_cast<double*>(workspace);
+    if (!g_stats_configured) configure_stats_kernels();
     const dim3 block(f.bx, kStatRowsPerBlock);
     const size_t smem = size_t(kStatRowsPerBlock) * f.width * 2 * sizeof(double) + (f.fold > 1 ? size_t(f.width) * sizeof(Moments) : 0);
     moments_partial_kernel<<<f.grid, block, smem, s>>>(reinterpret_cast<const float4*>(x), f.rows, f.vec, dim, f.fold, partial);

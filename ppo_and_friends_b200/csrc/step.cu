@@ -146,6 +146,7 @@ extern "C" int ppoaf_runtime_init(void) {
     cudaError_t e0 = cudaGetDevice(&dev);
     PPOAF_CHECK_ARG(e0 == cudaSuccess, "ppoaf_runtime_init: no CUDA device: %s", cudaGetErrorString(e0));
     configure_gemm_kernels();
+    configure_stats_kernels();
     cudaError_t e = cudaGetLastError();
     PPOAF_CHECK_ARG(e == cudaSuccess, "ppoaf_runtime_init: %s", cudaGetErrorString(e));
     return 0;
