@@ -7,6 +7,10 @@
 //   RTG_t = f32(r_t) + gamma RTG_{t+1},  RTG_L = f32(clip(r_boot))                             (f64)
 // Each element is the affine map x -> a + b x (b = 0 at a segment's last element, where the
 // seeds enter through a); maps compose associatively, so the reverse scan parallelises.
+// A map that contains a segment end carries the bit `e` and is the constant a: the value from the right is DROPPED
+// there, not multiplied by zero, so a NaN or Inf stays inside its own segment (IEEE 0 * NaN = 0 * Inf = NaN) as it
+// does in the per-episode reference.  b == 0 is not such a test: it also holds inside a segment when gamma*lambda is 0
+// or gamma*lambda^k underflows, where the reference does propagate a NaN.
 #include "common.cuh"
 
 namespace ppoaf {
@@ -31,24 +35,30 @@ __global__ void build_flat_map_kernel(const int32_t* __restrict__ seg_col, const
 }
 
 // ------------------------------------------------------------------------------------------------
-struct Affine2 {  // advantage map (aA, bA) and reward-to-go map (aR, bR)
+struct Affine2 {  // advantage map (aA, bA) and reward-to-go map (aR, bR); e: the range contains a segment end
     double aA, bA, aR, bR;
+    int e;
 };
 // result(x) = l(r(x)): l is the element/range on the LEFT (lower index), applied after r.
 __device__ __forceinline__ Affine2 compose(const Affine2& l, const Affine2& r) {
     Affine2 o;
-    o.aA = fma(l.bA, r.aA, l.aA);
+    o.aA = l.e ? l.aA : fma(l.bA, r.aA, l.aA);
     o.bA = l.bA * r.bA;
-    o.aR = fma(l.bR, r.aR, l.aR);
+    o.aR = l.e ? l.aR : fma(l.bR, r.aR, l.aR);
     o.bR = l.bR * r.bR;
+    o.e = l.e | r.e;
     return o;
 }
+// m(x) for a value x entering from the right of the range m
+__device__ __forceinline__ double apply_adv(const Affine2& m, double x) { return m.e ? m.aA : fma(m.bA, x, m.aA); }
+__device__ __forceinline__ double apply_rtg(const Affine2& m, double x) { return m.e ? m.aR : fma(m.bR, x, m.aR); }
 __device__ __forceinline__ Affine2 shfl_down_affine(const Affine2& v, int d) {
     Affine2 o;
     o.aA = __shfl_down_sync(kFull, v.aA, d);
     o.bA = __shfl_down_sync(kFull, v.bA, d);
     o.aR = __shfl_down_sync(kFull, v.aR, d);
     o.bR = __shfl_down_sync(kFull, v.bR, d);
+    o.e = __shfl_down_sync(kFull, v.e, d);
     return o;
 }
 
@@ -56,7 +66,7 @@ struct alignas(64) TileDesc {
     double aA, bA, aR, bR;  // tile aggregate map
     double vA, vR;          // A and RTG at the tile's first (lowest) element
     int status;             // 0 = empty, 1 = aggregate ready, 2 = value ready
-    int pad;
+    int e;                  // the tile contains a segment end
 };
 
 __device__ __forceinline__ int ld_acquire(const int* p) {
@@ -234,13 +244,14 @@ segscan_kernel(const float* __restrict__ rewards, const float* __restrict__ valu
             a_rtg[k] = aR;
         }
         Affine2 agg;  // identity
-        agg.aA = 0.0; agg.bA = 1.0; agg.aR = 0.0; agg.bR = 1.0;
+        agg.aA = 0.0; agg.bA = 1.0; agg.aR = 0.0; agg.bR = 1.0; agg.e = 0;
 #pragma unroll
         for (int k = kScanItems - 1; k >= 0; --k) {
             Affine2 e;
             const bool end = (endmask >> k) & 1u;
             e.aA = a_adv[k]; e.bA = end ? 0.0 : gamma_lambda;
             e.aR = a_rtg[k]; e.bR = end ? 0.0 : gamma;
+            e.e = end;
             agg = compose(e, agg);
         }
 
@@ -254,7 +265,7 @@ segscan_kernel(const float* __restrict__ rewards, const float* __restrict__ valu
         if (lane == 0) s_warp_agg[warp] = suffix;
         __syncthreads();
         Affine2 right_in_tile;
-        right_in_tile.aA = 0.0; right_in_tile.bA = 1.0; right_in_tile.aR = 0.0; right_in_tile.bR = 1.0;
+        right_in_tile.aA = 0.0; right_in_tile.bA = 1.0; right_in_tile.aR = 0.0; right_in_tile.bR = 1.0; right_in_tile.e = 0;
         {
             const Affine2 lane_right = shfl_down_affine(suffix, 1);
             if (lane < 31) right_in_tile = lane_right;
@@ -271,9 +282,9 @@ segscan_kernel(const float* __restrict__ rewards, const float* __restrict__ valu
             Affine2 tile_agg = s_warp_agg[0];
             for (int w = 1; w < kScanThreads / 32; ++w) tile_agg = compose(tile_agg, s_warp_agg[w]);
             TileDesc* d = desc + tile;
-            const bool closed = (tile_agg.bA == 0.0 && tile_agg.bR == 0.0) || tile == n_tiles - 1;
-            d->aA = tile_agg.aA; d->bA = tile_agg.bA; d->aR = tile_agg.aR; d->bR = tile_agg.bR;
-            if (closed) {  // carry-in cannot matter (or is zero past the end): value known at once
+            const bool closed = tile_agg.e || tile == n_tiles - 1;
+            d->aA = tile_agg.aA; d->bA = tile_agg.bA; d->aR = tile_agg.aR; d->bR = tile_agg.bR; d->e = tile_agg.e;
+            if (closed) {  // carry-in is dropped at a segment end (or is zero past the end): value known at once
                 d->vA = tile_agg.aA; d->vR = tile_agg.aR;
                 __threadfence();
                 st_release(&d->status, 2);
@@ -284,25 +295,26 @@ segscan_kernel(const float* __restrict__ rewards, const float* __restrict__ valu
             double cA = 0.0, cR = 0.0;  // carry entering the tile from the right
             if (tile != n_tiles - 1) {
                 Affine2 acc;  // composition of the tiles inspected so far
-                acc.aA = 0.0; acc.bA = 1.0; acc.aR = 0.0; acc.bR = 1.0;
+                acc.aA = 0.0; acc.bA = 1.0; acc.aR = 0.0; acc.bR = 1.0; acc.e = 0;
                 int k = tile + 1;
                 while (true) {
                     if (k == n_tiles) { cA = acc.aA; cR = acc.aR; break; }
                     const TileDesc* p = desc + k;
                     int stt;
                     do { stt = ld_acquire(&p->status); } while (stt == 0);
-                    if (stt == 2) {
+                    if (stt == 2) {  // acc has no segment end here: the loop leaves as soon as it gains one
                         cA = fma(acc.bA, __ldcg(&p->vA), acc.aA);
                         cR = fma(acc.bR, __ldcg(&p->vR), acc.aR);
                         break;
                     }
                     Affine2 t;
                     t.aA = __ldcg(&p->aA); t.bA = __ldcg(&p->bA); t.aR = __ldcg(&p->aR); t.bR = __ldcg(&p->bR);
+                    t.e = __ldcg(&p->e);
                     acc = compose(acc, t);
-                    if (acc.bA == 0.0 && acc.bR == 0.0) { cA = acc.aA; cR = acc.aR; break; }
+                    if (acc.e) { cA = acc.aA; cR = acc.aR; break; }
                     ++k;
                 }
-                if (!closed) {
+                if (!closed) {  // (no segment end in the tile)
                     d->vA = fma(tile_agg.bA, cA, tile_agg.aA);
                     d->vR = fma(tile_agg.bR, cR, tile_agg.aR);
                     __threadfence();
@@ -314,8 +326,8 @@ segscan_kernel(const float* __restrict__ rewards, const float* __restrict__ valu
         __syncthreads();
 
         // ---- apply: values right of this thread, then walk the thread's items right to left ----
-        double xA = fma(right_in_tile.bA, s_carry[0], right_in_tile.aA);
-        double xR = fma(right_in_tile.bR, s_carry[1], right_in_tile.aR);
+        double xA = apply_adv(right_in_tile, s_carry[0]);
+        double xR = apply_rtg(right_in_tile, s_carry[1]);
         float oa[kScanItems], og[kScanItems];
 #pragma unroll
         for (int k = kScanItems - 1; k >= 0; --k) {
