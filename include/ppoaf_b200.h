@@ -49,8 +49,8 @@ int         ppoaf_device_info(int* sm_count, int* cc_major, int* cc_minor);
 /* One-time per-device setup (kernel attributes such as > 48 KB dynamic shared memory); call once
  * before the first stream capture. */
 int         ppoaf_runtime_init(void);
-/* Engine of the MLP GEMM phases: 0 = fp32 FFMA tiles (default), 1 = tcgen05 3xTF32 tensor-core tiles (fp32-accurate).
- * Takes effect for update engines / forwards created afterwards. */
+/* Engine of ppoaf_mlp_forward's GEMMs: 0 = fp32 FFMA tiles (default), 1 = tcgen05 3xTF32 tensor-core tiles.
+ * The update always runs the FFMA tiles (or the fused step's own tensor-core tiles, PPOAF_STEP=fused). */
 int         ppoaf_set_gemm_backend(int backend);
 int         ppoaf_get_gemm_backend(void);
 

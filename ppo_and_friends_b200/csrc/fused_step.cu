@@ -28,7 +28,6 @@ namespace fused {
 using umma::mbar_init;
 using umma::mbar_wait;
 using umma::smem_u32;
-using umma::tf32_rna;
 
 constexpr int kFM = 128, kFK = 32, kFStages = 4;
 constexpr int kStageThreads = 256, kFThreads = kStageThreads + 128;   // 8 staging warps + the MMA warpgroup (warp 8 issues)

@@ -6,7 +6,7 @@ namespace ppoaf {
 
 // mlp.cu — grouped GEMM launches (all GEMMs of one phase of the minibatch step in ONE launch)
 enum { GEMM_BACKEND_FFMA = 0, GEMM_BACKEND_TCGEN05 = 1 };
-int gemm_backend();             // PPOAF_GEMM=ffma|tcgen05 (default tcgen05: 3xTF32 tensor-core tiles)
+int gemm_backend();             // PPOAF_GEMM=ffma|tcgen05 (default ffma); selects forward-only launches, see umma.cuh
 struct GroupedGemmArgs;
 constexpr int kMaxGroupHost = 6;    // problems one grouped launch carries (== kMaxGroup of mlp.cuh)
 struct GemmGroup {
@@ -17,7 +17,6 @@ struct GemmGroup {
     ~GemmGroup();
     GemmGroup(const GemmGroup&) = delete;
     GemmGroup& operator=(const GemmGroup&) = delete;
-    void reset();               // empty the group for reuse after launch()
     // Y[rows, out] = act(X[idx][rows, in] W^T + b)
     // w_static / x_static: the operand is not written by the launch that precedes this one in the stream, so the
     // FFMA kernel may stage it before its programmatic-dependency wait (see common.cuh, PDL)
@@ -27,13 +26,14 @@ struct GemmGroup {
     void add_backward_x(const float* dZ, const float* W, const float* Xact, float* dX, int rows, int in, int out, int act);
     // dW[out, in] = dZ[rows, out]^T X[idx][rows, in]; db[out] = column sums of dZ; sq_out[tile] = tile sum of squares
     // returns the number of sum-of-squares slots (tiles) this problem writes
+    // (backward problems run on the FFMA tiles only: launch() refuses them in a GEMM_BACKEND_TCGEN05 group)
     int add_backward_w(const float* dZ, const float* X, int ldx, const int64_t* idx, float* dW, float* db, int rows,
                        int in, int out, double* sq_out, bool x_static = false);
     // n_mirror / mirror_delta: peer copies of the gradient buffer (ppoaf_update_bufs), applied to backward-w outputs
     int launch(const int32_t* cursor, int cursor_stride, cudaStream_t s, int n_mirror = 0,
                const int64_t* mirror_delta = nullptr);
 };
-int backward_w_tiles(int in, int out, int backend);
+int backward_w_tiles(int in, int out);
 void configure_gemm_kernels();
 int64_t param_layout(const ppoaf_mlp_desc* net, int32_t log_std_dim, int64_t* offsets);
 int check_mlp_desc(const ppoaf_mlp_desc* net, const char* who);

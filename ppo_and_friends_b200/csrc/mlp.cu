@@ -25,7 +25,6 @@ static inline int tile_n(int backend) { return backend == GEMM_BACKEND_TCGEN05 ?
 
 GemmGroup::GemmGroup(int backend_) : args(new GroupedGemmArgs()), n_tiles(0), backend(backend_) { args->n_problems = 0; }
 GemmGroup::~GemmGroup() { delete args; }
-void GemmGroup::reset() { args->n_problems = 0; n_tiles = 0; }
 static_assert(kMaxGroupHost == kMaxGroup, "internal.h and mlp.cuh disagree on the group size");
 
 static GemmProblem* next_problem(GemmGroup* grp, int M, int N) {
@@ -57,8 +56,8 @@ void GemmGroup::add_backward_x(const float* dZ, const float* W, const float* Xac
     g->flavour = EPI_BWD_X * 4 + (vec4_ok(dZ, out, out) ? 2 : 0) + (vec4_ok(W, in, in) ? 1 : 0);
 }
 
-int backward_w_tiles(int in, int out, int backend) {
-    return ((in + tile_n(backend) - 1) / tile_n(backend)) * ((out + tile_m(backend) - 1) / tile_m(backend));
+int backward_w_tiles(int in, int out) {
+    return ((in + kBN - 1) / kBN) * ((out + kBM - 1) / kBM);
 }
 
 int GemmGroup::add_backward_w(const float* dZ, const float* X, int ldx, const int64_t* idx, float* dW, float* db,
@@ -69,7 +68,7 @@ int GemmGroup::add_backward_w(const float* dZ, const float* X, int ldx, const in
     g->M = out; g->N = in; g->K = rows;
     g->idxB = idx; g->dbias = db; g->sq_out = sq_out;
     g->flavour = EPI_BWD_W * 4 + (vec4_ok(dZ, out, out) ? 2 : 0) + (vec4_ok(X, ldx, in) ? 1 : 0);
-    return backward_w_tiles(in, out, backend);
+    return backward_w_tiles(in, out);
 }
 
 int GemmGroup::launch(const int32_t* cursor, int cursor_stride, cudaStream_t s, int n_mirror, const int64_t* mirror_delta) {
@@ -80,6 +79,8 @@ int GemmGroup::launch(const int32_t* cursor, int cursor_stride, cudaStream_t s, 
     args->mirror.n = n_mirror;
     for (int q = 0; q < n_mirror && q < PPOAF_MAX_MIRROR; ++q) args->mirror.delta[q] = mirror_delta[q];
     if (backend == GEMM_BACKEND_TCGEN05) {
+        for (int i = 0; i < args->n_problems; ++i)
+            PPOAF_CHECK_ARG(args->p[i].flavour >> 2 == EPI_FWD, "GemmGroup::launch: the tcgen05 tiles run forward problems only");
         launch_chain(umma::umma_grouped_gemm_kernel, dim3(n_tiles), dim3(umma::kUThreads + 32), umma::kUmmaSmemBytes, s, *args);
         PPOAF_CHECK_LAUNCH("umma_grouped_gemm_kernel");
     } else {
@@ -100,8 +101,8 @@ __global__ void softmax_rows_kernel(float* __restrict__ y, int rows, int n) {
     for (int j = 0; j < n; ++j) p[j] = p[j] / s;
 }
 
-// Backend of the grouped GEMM launches: FFMA tiles (default: faster at B = 128..512, see DESIGN.md §5) or the
-// tcgen05 3xTF32 tiles (PPOAF_GEMM=tcgen05 or ppoaf_set_gemm_backend(1)).
+// Backend of the forward-only launches (ppoaf_mlp_forward; the update always runs the FFMA tiles): FFMA tiles (default:
+// faster up to 512 rows, DESIGN.md §3.3) or the tcgen05 3xTF32 tiles (PPOAF_GEMM=tcgen05 or ppoaf_set_gemm_backend(1)).
 static int g_backend = -1;
 int gemm_backend() {
     if (g_backend < 0) {

@@ -64,7 +64,7 @@ struct StepScratch {
 
 static int count_sq_slots(const ppoaf_mlp_desc* net) {
     int n = 0;
-    for (int l = 0; l < net->n_layers; ++l) n += backward_w_tiles(net->dims[l], net->dims[l + 1], GEMM_BACKEND_FFMA);
+    for (int l = 0; l < net->n_layers; ++l) n += backward_w_tiles(net->dims[l], net->dims[l + 1]);
     return n;
 }
 

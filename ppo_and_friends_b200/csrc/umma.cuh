@@ -1,6 +1,9 @@
-// tcgen05 (5th-gen tensor core) grouped GEMM for the actor/critic MLP phases, fp32-accurate.
+// tcgen05 (5th-gen tensor core) grouped GEMM for forward-only MLP launches (ppoaf_mlp_forward), fp32-accurate.
+// The update never runs these tiles (their single accumulator misses its parameter tolerance, DESIGN.md §3.3), so the
+// kernel carries only the forward epilogue (bias + activation) and K-major operands; the fused step kernel
+// (fused_step.cu) reuses the descriptor helpers below for both operand layouts.
 //
-// Why tensor cores at all at B = 512: the FFMA tile kernel (mlp.cuh) is bound by the per-thread
+// Why tensor cores at all: the FFMA tile kernel (mlp.cuh) is bound by the per-thread
 // instruction stream (~40 K warp-instructions per 32x64x256 tile); tcgen05.mma is issued by ONE
 // thread and reads its operands straight from shared memory, so the threads only stage data.
 // Why 3xTF32: parity with the reference needs fp32-grade products (post-epoch parameters within
@@ -11,7 +14,7 @@
 // Tile 128 (M) x 64 (N) per CTA, K in chunks of 32; 256 threads stage A and B (global -> registers ->
 // hi/lo shared tiles, 3 stages), thread 0 issues 12 MMAs (3 terms x 4 k-steps of 8) per chunk and
 // commits to an mbarrier that frees the stage; the accumulator (64 TMEM columns) is read back with
-// tcgen05.ld by all 8 warps for the fused epilogues.
+// tcgen05.ld by all 8 warps for the bias + activation epilogue.
 //
 // Shared-memory operand layouts (verified on hardware by scratch/umma_test.cu, scratch/umma_probe.cu):
 //   K-major  operand (reduction contiguous in global; X, dZ as A;  W as B in forward):
@@ -79,64 +82,39 @@ __device__ __forceinline__ float4 load4(const float* __restrict__ p, int n_valid
     return v;
 }
 
-// One operand's per-thread staging plan: N_CH 16-byte chunks per K chunk, pointers computed once.
-//   K-major  (RC): chunk (row = tid/8 + 32 i, kq = tid%8)            global P[row(out0+row)*ld + k0 + 4 kq]
-//   MN-major (OC): chunk (k = tid/(R/4) + (1024/R) i, rq = tid%(R/4))  global P[row(k0+k)*ld + out0 + 4 rq]
-template <int R, bool RC>
+// One K-major operand's per-thread staging plan: N_CH 16-byte chunks per K chunk, pointers computed once.
+//   chunk (row = tid/8 + 32 i, kq = tid%8): global P[row(out0+row)*ld + k0 + 4 kq]
+template <int R>
 struct Stager {
     static constexpr int N_CH = R * kUK / 4 / kUThreads;   // 4 for R = 128, 2 for R = 64
     int dst[N_CH];                                         // float offset inside the tile (swizzled)
-    const float* src[N_CH];                                // RC: row base + 4 kq ; OC (no gather): P + k*ld + o
-    int lim[N_CH];                                         // RC: row valid ? K : 0 ; OC: valid outputs from o (<= 0: none)
-    int k_of[N_CH];                                        // OC: k offset of the chunk inside a K chunk
-    const int64_t* idx;
-    const float* P;
-    int ld, o_off, kq4;
+    const float* src[N_CH];                                // row base + 4 kq
+    int lim[N_CH];                                         // row valid ? K : 0
+    int kq4;
     bool vec;
 
-    __device__ __forceinline__ void plan(int tid, const float* P_, int ld_, const int64_t* idx_, int out0, int out_ext,
+    __device__ __forceinline__ void plan(int tid, const float* P, int ld, const int64_t* idx, int out0, int out_ext,
                                          int k_ext, bool vec_) {
-        P = P_; ld = ld_; idx = idx_; vec = vec_;
+        vec = vec_;
 #pragma unroll
         for (int i = 0; i < N_CH; ++i) {
-            if constexpr (RC) {
-                const int row = tid / 8 + 32 * i, kq = tid % 8;
-                dst[i] = row * 32 + ((kq ^ (row & 7)) * 4);
-                const int grow = out0 + row;
-                kq4 = kq * 4;
-                if (grow < out_ext) {
-                    const int64_t r = idx ? idx[grow] : int64_t(grow);
-                    src[i] = P + r * ld + kq4;
-                    lim[i] = k_ext;
-                } else {
-                    src[i] = P;
-                    lim[i] = 0;
-                }
+            const int row = tid / 8 + 32 * i, kq = tid % 8;
+            dst[i] = row * 32 + ((kq ^ (row & 7)) * 4);
+            const int grow = out0 + row;
+            kq4 = kq * 4;
+            if (grow < out_ext) {
+                const int64_t r = idx ? idx[grow] : int64_t(grow);
+                src[i] = P + r * ld + kq4;
+                lim[i] = k_ext;
             } else {
-                const int k = tid / (R / 4) + (kUThreads / (R / 4)) * i, rq = tid % (R / 4);
-                dst[i] = (rq / 8) * 1024 + (k / 4) * 128 + (k % 4) * 32 + ((((rq / 2) % 4) ^ (k % 4)) * 8) + (rq % 2) * 4;
-                k_of[i] = k;
-                o_off = out0 + rq * 4;
-                lim[i] = out_ext - o_off;
-                src[i] = P + int64_t(k) * ld + o_off;
+                src[i] = P;
+                lim[i] = 0;
             }
         }
     }
-    __device__ __forceinline__ void load(float4 (&v)[N_CH], int k0, int k_ext) const {
+    __device__ __forceinline__ void load(float4 (&v)[N_CH], int k0) const {
 #pragma unroll
-        for (int i = 0; i < N_CH; ++i) {
-            if constexpr (RC) {
-                v[i] = load4(src[i] + k0, lim[i] - (k0 + kq4), vec);
-            } else {
-                const int k = k0 + k_of[i];
-                if (k < k_ext) {
-                    const float* p = idx ? P + idx[k] * ld + o_off : src[i] + int64_t(k0) * ld;
-                    v[i] = load4(p, lim[i], vec);
-                } else {
-                    v[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-                }
-            }
-        }
+        for (int i = 0; i < N_CH; ++i) v[i] = load4(src[i] + k0, lim[i] - (k0 + kq4), vec);
     }
     // split into hi / lo tf32 parts and store both tiles
     __device__ __forceinline__ void store(const float4 (&v)[N_CH], float* hi_tile, float* lo_tile) const {
@@ -167,8 +145,8 @@ __device__ __forceinline__ uint32_t kstep_units() { return RC ? 2u : 64u; }   //
 //   full[s]  : 8 arrivals (one per staging warp, after its stores + proxy fence)  -> MMA warp may read stage s
 //   free[s]  : tcgen05.commit                                                     -> stage s may be overwritten
 //   acc      : tcgen05.commit after the last chunk                                 -> accumulator complete
-template <bool A_RC, bool B_RC, int EPI>
-__device__ __forceinline__ void umma_tile(const GemmProblem& g, int tile, int64_t idx_off, const MirrorSet& mir, float* smem, uint64_t* bars,
+// Y = act(X[idx] W^T + b): both operands K-major (A = X, B = W).
+__device__ __forceinline__ void umma_tile(const GemmProblem& g, int tile, int64_t idx_off, float* smem, uint64_t* bars,
                                           uint32_t tmem) {
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int m0 = (tile / g.tiles_n) * kUM, n0 = (tile % g.tiles_n) * kUN;
@@ -181,24 +159,23 @@ __device__ __forceinline__ void umma_tile(const GemmProblem& g, int tile, int64_
     if (warp == kUThreads / 32) {
         // ------------------------------ MMA issuer ------------------------------
         if (lane == 0) {
-            constexpr uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((A_RC ? 0u : 1u) << 15) |
-                                       ((B_RC ? 0u : 1u) << 16) | (uint32_t(kUN >> 3) << 17) | (uint32_t(kUM >> 4) << 24);
-            const uint64_t da0 = desc_base<A_RC>(), db0 = desc_base<B_RC>();
+            constexpr uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | (uint32_t(kUN >> 3) << 17) | (uint32_t(kUM >> 4) << 24);
+            const uint64_t d0 = desc_base<true>();
             for (int c = 0; c < n_chunks; ++c) {
                 const int s = c % kUStages;
                 mbar_wait(&bar_full[s], uint32_t((c / kUStages) & 1));
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 const uint32_t st = smem_u32(smem + s * kStageFloats);
-                const uint64_t a_hi = da0 | uint64_t((st >> 4) & 0x3FFF);
-                const uint64_t a_lo = da0 | uint64_t(((st + kATileFloats * 4) >> 4) & 0x3FFF);
-                const uint64_t b_hi = db0 | uint64_t(((st + 2 * kATileFloats * 4) >> 4) & 0x3FFF);
-                const uint64_t b_lo = db0 | uint64_t(((st + (2 * kATileFloats + kBTileFloats) * 4) >> 4) & 0x3FFF);
+                const uint64_t a_hi = d0 | uint64_t((st >> 4) & 0x3FFF);
+                const uint64_t a_lo = d0 | uint64_t(((st + kATileFloats * 4) >> 4) & 0x3FFF);
+                const uint64_t b_hi = d0 | uint64_t(((st + 2 * kATileFloats * 4) >> 4) & 0x3FFF);
+                const uint64_t b_lo = d0 | uint64_t(((st + (2 * kATileFloats + kBTileFloats) * 4) >> 4) & 0x3FFF);
 #pragma unroll
                 for (uint32_t ks = 0; ks < kUK / 8; ++ks) {
-                    const uint64_t oa = ks * kstep_units<A_RC>(), ob = ks * kstep_units<B_RC>();
-                    mma_tf32(tmem, a_hi + oa, b_hi + ob, idesc, (c > 0 || ks > 0) ? 1u : 0u);
-                    mma_tf32(tmem, a_hi + oa, b_lo + ob, idesc, 1u);
-                    mma_tf32(tmem, a_lo + oa, b_hi + ob, idesc, 1u);
+                    const uint64_t o = ks * kstep_units<true>();
+                    mma_tf32(tmem, a_hi + o, b_hi + o, idesc, (c > 0 || ks > 0) ? 1u : 0u);
+                    mma_tf32(tmem, a_hi + o, b_lo + o, idesc, 1u);
+                    mma_tf32(tmem, a_lo + o, b_hi + o, idesc, 1u);
                 }
                 umma_commit(&bar_free[s]);
             }
@@ -208,40 +185,31 @@ __device__ __forceinline__ void umma_tile(const GemmProblem& g, int tile, int64_
     }
 
     // ------------------------------ staging warps ------------------------------
-    const int64_t* idxA = g.idxA ? g.idxA + idx_off : nullptr;
-    const int64_t* idxB = g.idxB ? g.idxB + idx_off : nullptr;
-    Stager<kUM, A_RC> sa;
-    Stager<kUN, B_RC> sb;
-    sa.plan(tid, g.A, g.lda, idxA, m0, g.M, g.K, (g.flavour & 2) != 0);
-    sb.plan(tid, g.B, g.ldb, idxB, n0, g.N, g.K, (g.flavour & 1) != 0);
-    constexpr int NA = Stager<kUM, A_RC>::N_CH, NB = Stager<kUN, B_RC>::N_CH;
+    Stager<kUM> sa;
+    Stager<kUN> sb;
+    sa.plan(tid, g.A, g.lda, g.idxA ? g.idxA + idx_off : nullptr, m0, g.M, g.K, (g.flavour & 2) != 0);
+    sb.plan(tid, g.B, g.ldb, nullptr, n0, g.N, g.K, (g.flavour & 1) != 0);
+    constexpr int NA = Stager<kUM>::N_CH, NB = Stager<kUN>::N_CH;
     float4 va[2][NA], vb[2][NB];                    // two register sets: chunk c+2 is in flight while chunk c+1 waits
-    float colsum[4] = {0.f, 0.f, 0.f, 0.f};       // EPI_BWD_W: bias gradient = column sums of the A operand (dZ)
 
-    sa.load(va[0], 0, g.K);
-    sb.load(vb[0], 0, g.K);
+    sa.load(va[0], 0);
+    sb.load(vb[0], 0);
     if (n_chunks > 1) {
-        sa.load(va[1], kUK, g.K);
-        sb.load(vb[1], kUK, g.K);
+        sa.load(va[1], kUK);
+        sb.load(vb[1], kUK);
     }
     PPOAF_STAMP(2);
 
-    // epilogue operands are fetched now, so their latency hides behind the main loop
+    // the bias is fetched now, so its latency hides behind the main loop
     const int q = warp & 3, h = warp >> 2;
     const int m = m0 + q * 32 + lane;
     const int nb = n0 + h * 32;
     const bool vec_out = (g.ldc % 4 == 0) && (reinterpret_cast<uintptr_t>(g.C) % 16 == 0);
-    float4 epi[8];
+    float4 bias[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
-        epi[j] = make_float4(0.f, 0.f, 0.f, 0.f);
         const int n = nb + 4 * j;
-        if constexpr (EPI == EPI_FWD) {
-            if (n < g.N) epi[j] = load4(g.bias + n, g.N - n, vec_out);
-        }
-        if constexpr (EPI == EPI_BWD_X) {
-            if (n < g.N && m < g.M) epi[j] = load4(g.aux + int64_t(m) * g.ldaux + n, g.N - n, vec_out && g.ldaux % 4 == 0);
-        }
+        bias[j] = n < g.N ? load4(g.bias + n, g.N - n, vec_out) : make_float4(0.f, 0.f, 0.f, 0.f);
     }
 
     auto stage_chunk = [&](int c, float4 (&a_regs)[NA], float4 (&b_regs)[NB]) {
@@ -250,18 +218,12 @@ __device__ __forceinline__ void umma_tile(const GemmProblem& g, int tile, int64_
         if (c >= kUStages) mbar_wait(&bar_free[s], uint32_t((c / kUStages - 1) & 1));   // MMAs of chunk c-3 have read it
         sa.store(a_regs, st, st + kATileFloats);
         sb.store(b_regs, st + 2 * kATileFloats, st + 2 * kATileFloats + kBTileFloats);
-        if constexpr (EPI == EPI_BWD_W) {
-#pragma unroll
-            for (int i = 0; i < NA; ++i) {
-                colsum[0] += a_regs[i].x; colsum[1] += a_regs[i].y; colsum[2] += a_regs[i].z; colsum[3] += a_regs[i].w;
-            }
-        }
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy stores -> visible to the tensor core
         __syncwarp();
         if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&bar_full[s])) : "memory");
         if (c + 2 < n_chunks) {
-            sa.load(a_regs, (c + 2) * kUK, g.K);
-            sb.load(b_regs, (c + 2) * kUK, g.K);
+            sa.load(a_regs, (c + 2) * kUK);
+            sb.load(b_regs, (c + 2) * kUK);
         }
     };
     for (int c = 0; c < n_chunks; c += 2) {
@@ -286,67 +248,26 @@ __device__ __forceinline__ void umma_tile(const GemmProblem& g, int tile, int64_
         : "r"(taddr));
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 
-    float sq = 0.f;
     if (m < g.M) {
         float* crow = g.C + int64_t(m) * g.ldc;
         const int act = g.act;
 #pragma unroll
         for (int j4 = 0; j4 < 8; ++j4) {
             const int n = nb + 4 * j4;
-            const float ev[4] = {epi[j4].x, epi[j4].y, epi[j4].z, epi[j4].w};
+            const float bv[4] = {bias[j4].x, bias[j4].y, bias[j4].z, bias[j4].w};
             float o[4];
 #pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                float v = __uint_as_float(r[4 * j4 + j]);
-                if constexpr (EPI == EPI_FWD) v = act_fwd_fast(v + ev[j], act);
-                if constexpr (EPI == EPI_BWD_X) v *= act_bwd_from_out(ev[j], act);
-                if constexpr (EPI == EPI_BWD_W) { if (n + j < g.N) sq = fmaf(v, v, sq); }
-                o[j] = v;
-            }
+            for (int j = 0; j < 4; ++j) o[j] = act_fwd_fast(__uint_as_float(r[4 * j4 + j]) + bv[j], act);
             if (vec_out && n + 3 < g.N) {
-                const float4 o4 = make_float4(o[0], o[1], o[2], o[3]);
-                *reinterpret_cast<float4*>(crow + n) = o4;
-                if constexpr (EPI == EPI_BWD_W) mirror_store(mir, reinterpret_cast<float4*>(crow + n), o4);
+                *reinterpret_cast<float4*>(crow + n) = make_float4(o[0], o[1], o[2], o[3]);
             } else {
 #pragma unroll
                 for (int j = 0; j < 4; ++j)
-                    if (n + j < g.N) {
-                        crow[n + j] = o[j];
-                        if constexpr (EPI == EPI_BWD_W) mirror_store(mir, crow + n + j, o[j]);
-                    }
+                    if (n + j < g.N) crow[n + j] = o[j];
             }
         }
     }
     PPOAF_STAMP(14);
-
-    if constexpr (EPI == EPI_BWD_W) {
-        // bias gradient: thread (warp w, lane l) summed rows k = w + 8 i of A columns 4 l .. 4 l + 3 (MN-major A: rq = tid % 32)
-        float* red = smem;                                     // pipeline memory is idle now: [8 warps][128]
-        __shared__ double s_sq[kUThreads / 32];
-        asm volatile("bar.sync 1, %0;" ::"n"(kUThreads) : "memory");
-#pragma unroll
-        for (int j = 0; j < 4; ++j) red[warp * kUM + lane * 4 + j] = colsum[j];
-        const double w = warp_sum(double(sq));
-        asm volatile("bar.sync 1, %0;" ::"n"(kUThreads) : "memory");
-        float db = 0.f;
-        if (tid < kUM) {
-#pragma unroll
-            for (int k = 0; k < kUThreads / 32; ++k) db += red[k * kUM + tid];
-            if (n0 == 0 && g.dbias && m0 + tid < g.M) {
-                g.dbias[m0 + tid] = db;
-                mirror_store(mir, g.dbias + m0 + tid, db);
-            }
-        }
-        const double wdb = warp_sum((n0 == 0 && tid < kUM && m0 + tid < g.M) ? double(db) * double(db) : 0.0);
-        if (lane == 0) s_sq[warp] = w + wdb;
-        asm volatile("bar.sync 1, %0;" ::"n"(kUThreads) : "memory");
-        if (tid == 0 && g.sq_out) {
-            double t = 0.0;
-#pragma unroll
-            for (int k = 0; k < kUThreads / 32; ++k) t += s_sq[k];
-            g.sq_out[tile] = t;
-        }
-    }
 }
 
 __global__ void __launch_bounds__(kUThreads + 32) umma_grouped_gemm_kernel(const GroupedGemmArgs args) {
@@ -384,11 +305,7 @@ __global__ void __launch_bounds__(kUThreads + 32) umma_grouped_gemm_kernel(const
     pdl_wait();
     pdl_trigger();
     const int64_t idx_off = args.cursor ? int64_t(*args.cursor) * args.cursor_stride : 0;
-    switch (g.flavour >> 2) {
-        case EPI_FWD:   umma_tile<true, true, EPI_FWD>(g, tile, idx_off, args.mirror, smem, s_bars, tmem); break;
-        case EPI_BWD_X: umma_tile<true, false, EPI_BWD_X>(g, tile, idx_off, args.mirror, smem, s_bars, tmem); break;
-        default:        umma_tile<false, false, EPI_BWD_W>(g, tile, idx_off, args.mirror, smem, s_bars, tmem); break;
-    }
+    umma_tile(g, tile, idx_off, smem, s_bars, tmem);
 
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();

@@ -31,7 +31,7 @@ def runtime_init():
 
 
 def set_gemm_backend(name):
-    """'ffma' (default) or 'tcgen05' (3xTF32 tensor-core tiles); applies to engines created afterwards."""
+    """GEMM tiles of mlp_forward: 'ffma' (default) or 'tcgen05' (3xTF32 tensor-core tiles); the update always runs FFMA."""
     check(load().ppoaf_set_gemm_backend({'ffma': 0, 'tcgen05': 1}[name]), 'ppoaf_set_gemm_backend')
 
 
