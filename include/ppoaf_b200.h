@@ -39,7 +39,10 @@ enum { PPOAF_ACT_IDENTITY = 0, PPOAF_ACT_RELU = 1, PPOAF_ACT_LEAKY_RELU = 2, PPO
  * ends (bit c set: actor output c is the last of its section), so the row holds at most 64 outputs; nvec must be
  * 1-D with start = 0 and every entry >= 1.  PPOAF_HEAD_BERNOULLI (MultiBinary action spaces, BernoulliDistribution
  * :134-196) is a restatement too: one torch Bernoulli(probs = sigmoid(actor output)) per output column, log-prob and
- * entropy summed over the columns; act_dim = actor output width = number of columns (at most 64), fp32 0/1 actions. */
+ * entropy summed over the columns; act_dim = actor output width = number of columns (at most 64), fp32 0/1 actions.
+ * Widths: PPOAF_HEAD_CATEGORICAL takes 1 .. 65536 classes and PPOAF_HEAD_GAUSSIAN_TANH 1 .. 4096 dimensions; rows of
+ * more than 64 outputs run one CTA (update) or one warp (evaluation, sampling) per row instead of one warp / thread.
+ * The multi-categorical and Bernoulli heads take at most 64 outputs.  Wider rows are refused, naming the width. */
 enum { PPOAF_HEAD_GAUSSIAN_TANH = 0, PPOAF_HEAD_CATEGORICAL = 1, PPOAF_HEAD_MULTI_CATEGORICAL = 2, PPOAF_HEAD_BERNOULLI = 3 };
 
 int         ppoaf_abi_version(void);
@@ -153,9 +156,10 @@ enum {
 typedef struct {
     ppoaf_mlp_desc actor, critic;
     int32_t head;                 /* PPOAF_HEAD_*                                                    */
-    int32_t act_dim;              /* stored action width: Da (Gaussian), 1 (Categorical index), the
-                                     number of sections (Multi-categorical, one int64 index each) or
-                                     the number of columns (Bernoulli, = actor output width)        */
+    int32_t act_dim;              /* stored action width: Da (Gaussian, 1 .. 4096), 1 (Categorical
+                                     index, 1 .. 65536 classes), the number of sections
+                                     (Multi-categorical, one int64 index each) or the number of
+                                     columns (Bernoulli, = actor output width); the last two <= 64   */
     int32_t use_huber;            /* nn.HuberLoss(delta=10) instead of MSE (ppo.py:2416-2419)       */
     int32_t normalize_adv;        /* ppo.py:2325-2333                                               */
     int32_t normalize_values;     /* ppo.py:2299-2303                                               */
@@ -248,7 +252,8 @@ int    ppoaf_ppo_fused_steps(const ppoaf_update_cfg* cfg, const ppoaf_update_buf
 
 /* Forward only (P1/P2; also rollout-time inference, SURVEY §8f row 1): y = MLP(x[idx]) for
  * n_rows rows; idx may be NULL (identity).  softmax applied when `softmax_out` (Discrete actor,
- * networks/distributions.py:1045). */
+ * networks/distributions.py:1045); rows of more than 64 columns take a warp per row, whose sums run in a
+ * different order than the one-thread-per-row kernel of narrower rows. */
 size_t ppoaf_mlp_forward_workspace_bytes(const ppoaf_mlp_desc* net, int32_t n_rows);
 int ppoaf_mlp_forward(const ppoaf_mlp_desc* net, const float* params, const float* x, const int64_t* idx,
                       int32_t n_rows, int softmax_out, float* y, void* workspace, size_t workspace_bytes,
@@ -256,7 +261,7 @@ int ppoaf_mlp_forward(const ppoaf_mlp_desc* net, const float* params, const floa
 
 /* P1  Action-head evaluation on its own (policies/ppo_policy.py:939-950): log-prob of `actions`
  * and entropy under the head parameterised by actor_out [n_rows, pred] (+ log_std for the
- * Gaussian head).  actions: fp32 [n_rows, act_dim] raw (pre-tanh), int64 [n_rows, 1] (Categorical) or
+ * Gaussian head).  Widths (pred_dim and act_dim): Gaussian <= 4096, Categorical <= 65536, Bernoulli <= 64.  actions: fp32 [n_rows, act_dim] raw (pre-tanh), int64 [n_rows, 1] (Categorical) or
  * fp32 0/1 [n_rows, act_dim] (Bernoulli: actor_out holds the logits, pred = act_dim, log_std must be NULL;
  * log-prob and entropy are summed over the columns). */
 int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std,
@@ -271,7 +276,8 @@ int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t pred_dim, 
  * raw_action / action fp32 [n_rows, act_dim] (Gaussian; action = tanh(raw) mapped to [dist_min, dist_max] when given),
  * int64 [n_rows, 1] (Categorical) or fp32 0/1 [n_rows, act_dim] (Bernoulli: action = [u < sigmoid(actor_out)], both
  * outputs get the same actions, each may be NULL; pred = act_dim; log_std, dist_min and dist_max must be NULL; noise of
- * 0.5 everywhere gives the deterministic action [p > 0.5]), log_prob fp32 [n_rows] (summed over the Bernoulli columns). */
+ * 0.5 everywhere gives the deterministic action [p > 0.5]), log_prob fp32 [n_rows] (summed over the Bernoulli columns).
+ * The Categorical head samples from softmax probs in actor_out.  Widths as for ppoaf_head_evaluate. */
 int ppoaf_head_sample(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std, float min_std,
                       const float* noise, const float* dist_min, const float* dist_max, int32_t act_dim,
                       int32_t n_rows, void* raw_action_out, void* action_out, float* log_prob_out, void* stream);

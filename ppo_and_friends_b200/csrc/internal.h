@@ -92,10 +92,16 @@ struct LossArgs {
     int d_actor_ld, d_critic_ld;
 };
 bool loss_head_fusable(int pred_dim, int Ha, int Hc, int vf_clip_enabled);
+// Head widths.  Every head runs rows of up to kMaxNarrowHead actor outputs on the warp-per-sample kernels
+// (loss_common.cuh); the Categorical and Gaussian heads also take wider rows, up to the bounds below, on the wide
+// kernels of loss.cu.
+constexpr int kMaxNarrowHead = 64;
+constexpr int kMaxCategoricalClasses = 65536;
+constexpr int kMaxGaussianDims = 4096;
 // a multi-categorical section table that fits the row: nonzero, last section ends at pred_dim - 1, n_sections ends
 bool section_table_ok(unsigned long long section_ends, int pred_dim, int n_sections);
-// The Categorical head is the table of one section (its callers leave cfg->section_ends zero); rows wider than 64 are
-// refused by the loss launch.
+// The Categorical head up to 64 classes is the table of one section (its callers leave cfg->section_ends zero); wider
+// rows have no table: they run the wide loss kernel.
 inline unsigned long long cfg_section_ends(const ppoaf_update_cfg* cfg) {
     if (cfg->head == PPOAF_HEAD_CATEGORICAL) {
         const int pred_dim = cfg->actor.dims[cfg->actor.n_layers];

@@ -7,8 +7,8 @@
 
 namespace ppoaf {
 
-constexpr int kMaxAct = 64;
-constexpr int kG = 32;                      // lanes that share one sample: one warp (each lane owns dims l, l+32)
+constexpr int kMaxAct = kMaxNarrowHead;      // wider Categorical / Gaussian rows: the wide kernels of loss.cu
+constexpr int kG = 32;                     // lanes that share one sample: one warp (each lane owns dims l, l+32)
 constexpr int kPerLane = kMaxAct / kG;      // 2
 constexpr int kLossThreads = 256;           // 8 samples per CTA
 constexpr int kSamplesPerBlock = kLossThreads / kG;
@@ -446,6 +446,13 @@ __device__ __forceinline__ void loss_cta_partials(const T (&sc)[kLossScalars], c
     }
 }
 
+// d(log_std) of dim d (the batch total of dL/d std times d std / d log_std), stored with its peer mirrors
+__device__ __forceinline__ void store_d_log_std(const LossArgs& a, int d, float gls) {
+    a.d_log_std[d] = gls;
+    for (int q = 0; q < a.n_mirror; ++q)
+        *reinterpret_cast<float*>(reinterpret_cast<char*>(a.d_log_std + d) + a.mirror_delta[q]) = gls;
+}
+
 // One CTA, after every CTA's partials are visible: totals -> s_tot, d(log_std) (and its peer mirrors) and the sum of
 // squares of d(log_std) for the gradient-norm clip.  Thread (slot = tid % 32, subset = tid / 32) sums CTAs subset,
 // subset + 8, ... for values slot, slot + 32, slot + 64 (all loads independent and in flight at once, from L2); the 8
@@ -482,9 +489,7 @@ __device__ __forceinline__ void loss_fold(const LossArgs& a, int n_vals, const f
         s_tot[tid] = t;
         if (tid >= kLossScalars) {
             const float gls = float(t) * s_dsd[tid - kLossScalars];
-            a.d_log_std[tid - kLossScalars] = gls;
-            for (int q = 0; q < a.n_mirror; ++q)
-                *reinterpret_cast<float*>(reinterpret_cast<char*>(a.d_log_std + (tid - kLossScalars)) + a.mirror_delta[q]) = gls;
+            store_d_log_std(a, tid - kLossScalars, gls);
             my_sq = double(gls) * double(gls);
         }
     }

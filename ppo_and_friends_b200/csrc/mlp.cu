@@ -101,6 +101,22 @@ __global__ void softmax_rows_kernel(float* __restrict__ y, int rows, int n) {
     for (int j = 0; j < n; ++j) p[j] = p[j] / s;
 }
 
+// Rows wider than 64 columns: one warp per row, the lanes striding over it (sums in a different order from
+// softmax_rows_kernel, so results can differ from it in the last bits)
+__global__ void __launch_bounds__(256) softmax_rows_wide_kernel(float* __restrict__ y, int rows, int n) {
+    const int lane = threadIdx.x & 31, r = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (r >= rows) return;
+    float* p = y + int64_t(r) * n;
+    float mx = -INFINITY;
+    for (int j = lane; j < n; j += 32) mx = fmaxf(mx, p[j]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(kFull, mx, o));
+    float s = 0.f;
+    for (int j = lane; j < n; j += 32) { const float e = expf(p[j] - mx); p[j] = e; s += e; }
+    s = warp_sum(s);
+    for (int j = lane; j < n; j += 32) p[j] = p[j] / s;
+}
+
 // Backend of the forward-only launches (ppoaf_mlp_forward; the update always runs the FFMA tiles): FFMA tiles (default:
 // faster up to 512 rows, DESIGN.md §3.3) or the tcgen05 3xTF32 tiles (PPOAF_GEMM=tcgen05 or ppoaf_set_gemm_backend(1)).
 static int g_backend = -1;
@@ -181,7 +197,11 @@ extern "C" int ppoaf_mlp_forward(const ppoaf_mlp_desc* net, const float* params,
         in_idx = nullptr;
     }
     if (softmax_out) {
-        softmax_rows_kernel<<<(n_rows + 127) / 128, 128, 0, s>>>(y, n_rows, net->dims[net->n_layers]);
+        const int n = net->dims[net->n_layers];
+        if (n > 64)
+            softmax_rows_wide_kernel<<<(n_rows + 7) / 8, 256, 0, s>>>(y, n_rows, n);
+        else
+            softmax_rows_kernel<<<(n_rows + 127) / 128, 128, 0, s>>>(y, n_rows, n);
         PPOAF_CHECK_LAUNCH("ppoaf_mlp_forward(softmax)");
     }
     return 0;

@@ -102,18 +102,29 @@ int check_cfg(const ppoaf_update_cfg* cfg, const char* who) {
     PPOAF_CHECK_ARG(cfg->critic.dims[cfg->critic.n_layers] == 1, "%s: critic output width must be 1", who);
     PPOAF_CHECK_ARG(cfg->head == PPOAF_HEAD_GAUSSIAN_TANH || cfg->head == PPOAF_HEAD_CATEGORICAL ||
                     cfg->head == PPOAF_HEAD_MULTI_CATEGORICAL || cfg->head == PPOAF_HEAD_BERNOULLI, "%s: unknown head", who);
-    if (cfg->head == PPOAF_HEAD_GAUSSIAN_TANH)
-        PPOAF_CHECK_ARG(cfg->actor.dims[cfg->actor.n_layers] == cfg->act_dim,
-                        "%s: Gaussian actor output width must equal act_dim", who);
-    else if (cfg->head == PPOAF_HEAD_BERNOULLI)
-        PPOAF_CHECK_ARG(cfg->actor.dims[cfg->actor.n_layers] == cfg->act_dim,
+    const int pred = cfg->actor.dims[cfg->actor.n_layers];
+    if (cfg->head == PPOAF_HEAD_GAUSSIAN_TANH) {
+        PPOAF_CHECK_ARG(pred == cfg->act_dim, "%s: Gaussian actor output width must equal act_dim", who);
+        PPOAF_CHECK_ARG(pred <= kMaxGaussianDims, "%s: head width %d is outside the 1 .. %d dims of the Gaussian head",
+                        who, pred, kMaxGaussianDims);
+    } else if (cfg->head == PPOAF_HEAD_BERNOULLI) {
+        PPOAF_CHECK_ARG(pred == cfg->act_dim,
                         "%s: Bernoulli actor output width must equal act_dim (one column per binary action)", who);
-    else if (cfg->head == PPOAF_HEAD_MULTI_CATEGORICAL)
-        PPOAF_CHECK_ARG(section_table_ok(cfg_section_ends(cfg), cfg->actor.dims[cfg->actor.n_layers], cfg->act_dim),
+        PPOAF_CHECK_ARG(pred <= kMaxNarrowHead, "%s: head width %d is outside the 1 .. %d columns of the Bernoulli head",
+                        who, pred, kMaxNarrowHead);
+    } else if (cfg->head == PPOAF_HEAD_MULTI_CATEGORICAL) {
+        PPOAF_CHECK_ARG(pred <= kMaxNarrowHead,
+                        "%s: head width %d is outside the 1 .. %d outputs of the multi-categorical head", who, pred,
+                        kMaxNarrowHead);
+        PPOAF_CHECK_ARG(section_table_ok(cfg_section_ends(cfg), pred, cfg->act_dim),
                         "%s: bad multi-categorical section table (must be nonzero, its highest set bit must be the last "
                         "actor output, at most 64 outputs, and it must have act_dim = %d bits)", who, cfg->act_dim);
-    else
+    } else {
         PPOAF_CHECK_ARG(cfg->act_dim == 1, "%s: Categorical actions are stored as one int64 index", who);
+        PPOAF_CHECK_ARG(pred <= kMaxCategoricalClasses,
+                        "%s: head width %d is outside the 1 .. %d classes of the Categorical head", who, pred,
+                        kMaxCategoricalClasses);
+    }
     return 0;
 }
 

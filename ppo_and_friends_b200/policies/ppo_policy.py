@@ -20,6 +20,8 @@ and entropy summed over the sections); `nvec` must be 1-D with `start` = 0, ever
 MultiBinary action spaces take a Bernoulli head (reference BernoulliDistribution, networks/distributions.py:134-196,
 restated: one Bernoulli(probs=sigmoid(actor output)) per column, log-prob and entropy summed over the columns, fp32 0/1
 actions); the shape must be 1-D with 1 <= n <= 64.
+Discrete spaces take 1 <= n <= 65536 actions (n <= 64: the multi-categorical head with one section; wider: the
+Categorical head's wide kernels) and Box spaces 1 .. 4096 flattened dimensions.
 Out of scope (raise): LSTM networks, ICM, MAT, Mixed action heads.
 """
 import os
@@ -32,6 +34,10 @@ from ..networks.feed_forward import PolicyNetworks, _AdamView, hidden_sizes
 from ..utils.episode_info import PPODataset, RolloutRing
 from ..utils.misc import update_optimizer_lr
 from ..utils.mpi_utils import abort, barrier, broadcast_model_parameters, get_rank, rank_print
+
+
+MAX_DISCRETE_ACTIONS = 65536      # include/ppoaf_b200.h: the Categorical and Gaussian heads' widest rows
+MAX_BOX_DIMS = 4096
 
 
 class CallableValue:
@@ -129,8 +135,12 @@ class PPOPolicy:
         else:
             self.bootstrap_clip = None
 
-        # a Discrete space is the multi-categorical head's table of one section
+        # a Discrete space of up to 64 actions is the multi-categorical head's table of one section; a wider one runs
+        # the Categorical head's wide kernels and has no section table
         if self.action_dtype == "discrete":
+            if not 1 <= int(action_space.n) <= MAX_DISCRETE_ACTIONS:
+                abort(f"ERROR: Discrete n = {int(action_space.n)} is outside the 1 .. {MAX_DISCRETE_ACTIONS} actions the "
+                      "Categorical head supports.")
             self.nvec = [int(action_space.n)]
         elif self.action_dtype == "multi-discrete":
             nvec = np.asarray(action_space.nvec)
@@ -152,13 +162,17 @@ class PPOPolicy:
             if not 1 <= int(shape[0]) <= 64:
                 abort(f"ERROR: MultiBinary n = {int(shape[0])} is outside the 1 .. 64 actor outputs the Bernoulli "
                       "head supports.")
+        elif self.action_dtype == "continuous" and not 1 <= _flat_dim(action_space) <= MAX_BOX_DIMS:
+            abort(f"ERROR: Box spaces of {_flat_dim(action_space)} dimensions are outside the 1 .. {MAX_BOX_DIMS} the "
+                  "Gaussian head supports.")
         if self.action_dtype in ("continuous", "multi-binary"):
             self.action_dim = _flat_dim(action_space)
             self.action_pred_size = self.action_dim
         else:
             self.action_dim = len(self.nvec)
             self.action_pred_size = sum(self.nvec)
-            self.section_ends = _lib.section_ends(self.nvec)
+            if not self.wide_categorical:
+                self.section_ends = _lib.section_ends(self.nvec)
         self.actor_kw_args = dict(actor_kw_args)
         self.critic_kw_args = dict(critic_kw_args)
         self._ring = None
@@ -234,6 +248,11 @@ class PPOPolicy:
     def shuffle_agent_ids(self):
         """policies/ppo_policy.py:364-371 (only called for agent-grouping policies, ppo.py:1643-1644)."""
         np.random.shuffle(self.agent_ids)
+
+    @property
+    def wide_categorical(self):
+        """A Discrete space of more than 64 actions: the Categorical head's own entry points, no section table."""
+        return self.action_dtype == "discrete" and self.nvec[0] > 64
 
     @property
     def head(self):
@@ -360,6 +379,9 @@ class PPOPolicy:
         elif self.action_dtype == "multi-binary":
             acts = acts.to(self.device, torch.float32).reshape(pred.shape[0], -1).contiguous()
             lp, ent = ops.head_evaluate(self.head, pred, None, acts)
+        elif self.wide_categorical:
+            acts = acts.to(self.device, torch.int64).reshape(pred.shape[0], -1).contiguous()
+            lp, ent = ops.head_evaluate(self.head, pred, None, acts)
         else:
             acts = acts.to(self.device, torch.int64).reshape(pred.shape[0], -1).contiguous()
             lp, ent = ops.multi_categorical_evaluate(pred, self.section_ends, acts)
@@ -383,7 +405,10 @@ class PPOPolicy:
         n = t_obs.shape[0]
         discrete = self.action_dtype in ("discrete", "multi-discrete")
         action_pred = self.actor(t_obs, softmax_out=discrete)
-        if discrete:
+        if self.wide_categorical:
+            noise = torch.empty(n, self.nvec[0], dtype=torch.float32).exponential_(1)
+            raw, act, lp = ops.head_sample(self.head, action_pred, None, noise.to(self.device, non_blocking=True))
+        elif discrete:
             noise = torch.cat([torch.empty(n, k, dtype=torch.float32).exponential_(1).reshape(-1) for k in self.nvec])
             act, lp = ops.multi_categorical_sample(action_pred, self.section_ends,
                                                    noise.to(self.device, non_blocking=True), len(self.nvec))
