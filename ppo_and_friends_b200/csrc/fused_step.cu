@@ -776,11 +776,7 @@ __device__ __forceinline__ void adam_phase(const FusedPlan& P, double p1, double
         const float inv_world = float(hp[PPOAF_HP_INV_WORLD]);
         const float max_norm = float(hp[PPOAF_HP_GRAD_CLIP]);
         const double scale = double(inv_world);
-        float ca = 1.f, cc = 1.f;
-        if (max_norm >= 0.f) {
-            ca = fminf(max_norm / (float(sqrt(sa) * scale) + 1e-6f), 1.f);
-            cc = fminf(max_norm / (float(sqrt(sc) * scale) + 1e-6f), 1.f);
-        }
+        const float ca = clip_coef(max_norm, sa, scale), cc = clip_coef(max_norm, sc, scale);
         const double b1d = hp[PPOAF_HP_BETA1], b2d = hp[PPOAF_HP_BETA2];
         const double bc1 = 1.0 - p1, bc2 = 1.0 - p2;
         s_f[0] = float(-(hp[PPOAF_HP_LR] / bc1));

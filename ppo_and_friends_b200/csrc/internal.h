@@ -115,11 +115,24 @@ size_t loss_workspace_bytes(int max_batch, int act_dim);
 int launch_ppo_loss(const LossArgs& a, cudaStream_t s);
 
 // optim.cu
-// beta^t for the Adam bias corrections without a double pow() on the critical path: cache = (t, b1^t, b2^t) of the
-// previous step; one multiply when t advanced by one, pow() otherwise (first step, restored checkpoints).
+// beta^t for the Adam bias corrections without a double pow() on the critical path: cache = (t, b1, b2, b1^t, b2^t) of
+// the previous step; one multiply when t advanced by one under the same betas, pow() otherwise (first step, restored
+// checkpoints, betas changed between steps, or a workspace shared by parameter sets with different betas).
+constexpr int kBetaCacheDoubles = 5;
 __device__ __forceinline__ void beta_powers(const double* cache, int64_t t, double b1, double b2, double& p1, double& p2) {
-    if (cache[0] == double(t - 1) && t > 1) { p1 = cache[1] * b1; p2 = cache[2] * b2; }
+    if (cache[0] == double(t - 1) && t > 1 && cache[1] == b1 && cache[2] == b2) { p1 = cache[3] * b1; p2 = cache[4] * b2; }
     else { p1 = pow(b1, double(t)); p2 = pow(b2, double(t)); }
+}
+__device__ __forceinline__ void store_beta_powers(double* cache, int64_t t, double b1, double b2, double p1, double p2) {
+    cache[0] = double(t); cache[1] = b1; cache[2] = b2; cache[3] = p1; cache[4] = p2;
+}
+// torch clip_grad_norm_'s coefficient for one network: max_norm / (norm + 1e-6) clamped to at most 1, with
+// norm = sqrt(sumsq) * scale.  A NaN norm gives a NaN coefficient (torch.clamp keeps NaN), so a NaN gradient element
+// makes every gradient of that network NaN, as in torch.  max_norm < 0: clipping off.
+__device__ __forceinline__ float clip_coef(float max_norm, double sumsq, double scale) {
+    if (!(max_norm >= 0.f)) return 1.f;
+    const float c = max_norm / (float(sqrt(sumsq) * scale) + 1e-6f);
+    return isnan(c) ? c : fminf(c, 1.f);
 }
 size_t optim_workspace_bytes();
 // sq_a / sq_c: per-network sum-of-squares slots already produced by the backward-w epilogues (n_sq_* > 0), or

@@ -64,7 +64,7 @@ adam_update_kernel(float* __restrict__ params, const float* __restrict__ grads, 
     __shared__ double s_scr[32];
     __shared__ double s_pw[2];
     __shared__ float s_coef[2];
-    double* pw = reinterpret_cast<double*>(ticket + 2);   // cached (t, beta1^t, beta2^t)
+    double* pw = reinterpret_cast<double*>(ticket + 2);   // cached (t, beta1, beta2, beta1^t, beta2^t)
     const int64_t nv = n_total / 4, na = n_actor / 4;
     const int64_t stride = int64_t(gridDim.x) * blockDim.x;
     const int64_t i0 = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -99,13 +99,8 @@ adam_update_kernel(float* __restrict__ params, const float* __restrict__ grads, 
     if (threadIdx.x == 0) {
         const float max_norm = float(hp[PPOAF_HP_GRAD_CLIP]);
         // the slots hold sums over the SUMMED gradients; the averaged gradient is inv_world times that
-        const double scale = double(inv_world);
-        if (max_norm >= 0.f) {  // clip_coef = max_norm / (total_norm + 1e-6), clamped to 1 (torch clip_grad_norm_)
-            s_coef[0] = fminf(max_norm / (float(sqrt(ta) * scale) + 1e-6f), 1.f);
-            s_coef[1] = fminf(max_norm / (float(sqrt(tc) * scale) + 1e-6f), 1.f);
-        } else {
-            s_coef[0] = s_coef[1] = 1.f;
-        }
+        s_coef[0] = clip_coef(max_norm, ta, double(inv_world));
+        s_coef[1] = clip_coef(max_norm, tc, double(inv_world));
     }
     const int64_t t = *adam_step + 1;
     __shared__ float s_f[6];
@@ -148,7 +143,7 @@ adam_update_kernel(float* __restrict__ params, const float* __restrict__ grads, 
         if (atomicAdd(ticket, 1u) == gridDim.x - 1) {
             *adam_step = t;
             if (mb_cursor) *mb_cursor += 1;
-            pw[0] = double(t); pw[1] = s_pw[0]; pw[2] = s_pw[1];
+            store_beta_powers(pw, t, hp[PPOAF_HP_BETA1], hp[PPOAF_HP_BETA2], s_pw[0], s_pw[1]);
             *ticket = 0u;
         }
     }
@@ -162,8 +157,11 @@ static int opt_grid(int64_t n_total) {
     return int(b < 1 ? 1 : (b > cap ? cap : b));
 }
 
+constexpr size_t kTicketBytes = 256;    // ticket word, one spare word, the beta-power cache
+static_assert(2 * sizeof(unsigned int) + kBetaCacheDoubles * sizeof(double) <= kTicketBytes,
+              "the beta-power cache must fit the ticket region");
 size_t optim_workspace_bytes() {
-    return align_up(size_t(sm_count()) * 2 * sizeof(double), 256) + 256;  // norm-pass partials | ticket
+    return align_up(size_t(sm_count()) * 2 * sizeof(double), 256) + kTicketBytes;  // norm-pass partials | ticket region
 }
 
 int launch_clip_adam(float* params, const float* grads, float* m, float* v, int64_t* adam_step, int32_t* mb_cursor,

@@ -71,7 +71,7 @@ __device__ __forceinline__ uint32_t ld_acquire_gpu(const uint32_t* p) {
 }
 
 // ctrl (local, zero-initialised): [0] epoch (barrier value of the last call), [2] grid-barrier "go" word, [3] ticket,
-// [4] error flag;
+// [4] error flag, [8..] beta-power cache (store_beta_powers);
 // arrive (local, zero-initialised): one word per CTA (grid barriers of the NVLS variant; the peer kernel counts on ctrl[2])
 __global__ void __launch_bounds__(kPeerThreads)
 peer_allreduce_adam_kernel(const PeerArgs pa, float* __restrict__ params, float* __restrict__ m, float* __restrict__ v,
@@ -84,7 +84,7 @@ peer_allreduce_adam_kernel(const PeerArgs pa, float* __restrict__ params, float*
     __shared__ int s_err;
     const int tid = threadIdx.x;
     const int R = pa.n_ranks;
-    double* pw = reinterpret_cast<double*>(ctrl + 8);   // cached (t, beta1^t, beta2^t)
+    double* pw = reinterpret_cast<double*>(ctrl + 8);   // cached (t, beta1, beta2, beta1^t, beta2^t)
     PEER_STAMP(0);
     // ---- 0. before the dependency wait: parameters and moments (only ever written by this kernel) ----
     const int64_t nv = n_total / 4, na = n_actor / 4;
@@ -179,11 +179,8 @@ peer_allreduce_adam_kernel(const PeerArgs pa, float* __restrict__ params, float*
     if (tid == 0) {
         const float inv_world = float(hp[PPOAF_HP_INV_WORLD]);
         const float max_norm = float(hp[PPOAF_HP_GRAD_CLIP]);
-        float ca = 1.f, cc = 1.f;
-        if (max_norm >= 0.f) {                 // clip_grad_norm_ on the AVERAGED gradient
-            ca = fminf(max_norm / (float(sqrt(ta) * double(inv_world)) + 1e-6f), 1.f);
-            cc = fminf(max_norm / (float(sqrt(tc) * double(inv_world)) + 1e-6f), 1.f);
-        }
+        const float ca = clip_coef(max_norm, ta, double(inv_world));   // clip_grad_norm_ on the AVERAGED gradient
+        const float cc = clip_coef(max_norm, tc, double(inv_world));
         const double b1d = hp[PPOAF_HP_BETA1], b2d = hp[PPOAF_HP_BETA2];
         double p1, p2;
         beta_powers(pw, t, b1d, b2d, p1, p2);
@@ -231,7 +228,7 @@ peer_allreduce_adam_kernel(const PeerArgs pa, float* __restrict__ params, float*
         if (atomicAdd(ctrl + 3, 1u) == gridDim.x - 1) {
             *adam_step = t;
             if (mb_cursor) *mb_cursor += 1;
-            pw[0] = double(t); pw[1] = s_pw[0]; pw[2] = s_pw[1];
+            store_beta_powers(pw, t, hp[PPOAF_HP_BETA1], hp[PPOAF_HP_BETA2], s_pw[0], s_pw[1]);
             ctrl[0] = epoch;
             ctrl[3] = 0u;
         }
@@ -302,7 +299,7 @@ __device__ __forceinline__ void gather_to_cta0(uint32_t* arrive, uint32_t epoch,
     }
 }
 
-// ctrl (local, zero-initialised): [0] epoch, [3] ticket, [4] error flag, [8..] cached beta powers
+// ctrl (local, zero-initialised): [0] epoch, [3] ticket, [4] error flag, [8..] beta-power cache (store_beta_powers)
 // arrive: 2 x gridDim.x local words; partials: 2 doubles per CTA
 __global__ void __launch_bounds__(kPeerThreads)
 nvls_allreduce_adam_kernel(const NvlsArgs pa, float* __restrict__ params, float* __restrict__ m, float* __restrict__ v,
@@ -401,11 +398,8 @@ nvls_allreduce_adam_kernel(const NvlsArgs pa, float* __restrict__ params, float*
     const float inv_world = float(hp[PPOAF_HP_INV_WORLD]);
     if (tid == 0) {
         const float max_norm = float(hp[PPOAF_HP_GRAD_CLIP]);
-        float ca = 1.f, cc = 1.f;
-        if (max_norm >= 0.f) {
-            ca = fminf(max_norm / (float(sqrt(s_tot[0]) * double(inv_world)) + 1e-6f), 1.f);
-            cc = fminf(max_norm / (float(sqrt(s_tot[1]) * double(inv_world)) + 1e-6f), 1.f);
-        }
+        const float ca = clip_coef(max_norm, s_tot[0], double(inv_world));
+        const float cc = clip_coef(max_norm, s_tot[1], double(inv_world));
         const double b1d = hp[PPOAF_HP_BETA1], b2d = hp[PPOAF_HP_BETA2];
         double p1, p2;
         beta_powers(pw, t, b1d, b2d, p1, p2);
@@ -471,7 +465,7 @@ nvls_allreduce_adam_kernel(const NvlsArgs pa, float* __restrict__ params, float*
         if (atomicAdd(ctrl + 3, 1u) == gridDim.x - 1) {
             *adam_step = t;
             if (mb_cursor) *mb_cursor += 1;
-            pw[0] = double(t); pw[1] = s_pw[0]; pw[2] = s_pw[1];
+            store_beta_powers(pw, t, hp[PPOAF_HP_BETA1], hp[PPOAF_HP_BETA2], s_pw[0], s_pw[1]);
             ctrl[0] = epoch;
             ctrl[3] = 0u;
         }
@@ -519,7 +513,12 @@ extern "C" int ppoaf_peer_close(void* p) {
 }
 
 static size_t peer_arrive_bytes() { return align_up(size_t(sm_count()) * sizeof(uint32_t), 256); }
-extern "C" size_t ppoaf_peer_ctrl_bytes(void) { return size_t(sm_count()) * 2 * sizeof(double) + peer_arrive_bytes() + 256; }
+constexpr size_t kCtrlWordsBytes = 256;    // the control words of both kernels: 8 u32 words, then the beta-power cache
+static_assert(8 * sizeof(uint32_t) + kBetaCacheDoubles * sizeof(double) <= kCtrlWordsBytes,
+              "the beta-power cache must fit the control words");
+extern "C" size_t ppoaf_peer_ctrl_bytes(void) {
+    return size_t(sm_count()) * 2 * sizeof(double) + peer_arrive_bytes() + kCtrlWordsBytes;
+}
 
 // peer_grads[r] / peer_flags[r]: pointers valid on THIS device for rank r's buffers (own rank: the local pointers).
 // ctrl: local zero-initialised scratch of ppoaf_peer_ctrl_bytes() bytes (CTA partials | arrival words | control words).
@@ -563,7 +562,7 @@ extern "C" int ppoaf_debug_peer_stamps(long long* out_host) {
 
 // ---- NVLS variant ------------------------------------------------------------------------------------------------
 extern "C" size_t ppoaf_nvls_ctrl_bytes(void) { configure_spin_limit();
-    return size_t(sm_count()) * 2 * sizeof(double) + 2 * peer_arrive_bytes() + 256;
+    return size_t(sm_count()) * 2 * sizeof(double) + 2 * peer_arrive_bytes() + kCtrlWordsBytes;
 }
 extern "C" size_t ppoaf_nvls_flag_block_bytes(void) { return 256; }
 

@@ -205,11 +205,13 @@ __device__ __forceinline__ void umma_tile(const GemmProblem& g, int tile, int64_
     const int m = m0 + q * 32 + lane;
     const int nb = n0 + h * 32;
     const bool vec_out = (g.ldc % 4 == 0) && (reinterpret_cast<uintptr_t>(g.C) % 16 == 0);
+    // the bias keeps the alignment of the parameter buffer, which need not be 16 bytes (as in mlp.cuh's epilogue)
+    const bool vec_bias = reinterpret_cast<uintptr_t>(g.bias) % 16 == 0;
     float4 bias[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
         const int n = nb + 4 * j;
-        bias[j] = n < g.N ? load4(g.bias + n, g.N - n, vec_out) : make_float4(0.f, 0.f, 0.f, 0.f);
+        bias[j] = n < g.N ? load4(g.bias + n, g.N - n, vec_bias) : make_float4(0.f, 0.f, 0.f, 0.f);
     }
 
     auto stage_chunk = [&](int c, float4 (&a_regs)[NA], float4 (&b_regs)[NB]) {
