@@ -263,7 +263,14 @@ int ppoaf_mlp_forward(const ppoaf_mlp_desc* net, const float* params, const floa
  * and entropy under the head parameterised by actor_out [n_rows, pred] (+ log_std for the
  * Gaussian head).  Widths (pred_dim and act_dim): Gaussian <= 4096, Categorical <= 65536, Bernoulli <= 64.  actions: fp32 [n_rows, act_dim] raw (pre-tanh), int64 [n_rows, 1] (Categorical) or
  * fp32 0/1 [n_rows, act_dim] (Bernoulli: actor_out holds the logits, pred = act_dim, log_std must be NULL;
- * log-prob and entropy are summed over the columns). */
+ * log-prob and entropy are summed over the columns).  log_prob_out is required, entropy_out may be NULL.
+ *
+ * Non-finite inputs (all head entry points, evaluation and sampling): every clamp of the head arithmetic is torch.clamp,
+ * which keeps a NaN, so a NaN in a row's mean, action, logits or probabilities, or in log_std, gives that row a NaN
+ * log-prob wherever torch's float64 evaluation of the same formulas gives one (a NaN log_std: every row); the entropy
+ * likewise.  A sampled row whose probabilities (of one section) hold a NaN takes action 0 in that section and a NaN
+ * log-prob; a Gaussian row samples the NaN its arithmetic gives.  A multi-categorical section whose probabilities all
+ * underflow to 0 has no distribution either (torch's 0 / 0): NaN. */
 int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std,
                         float min_std, const void* actions, int32_t act_dim, int32_t n_rows,
                         float* log_prob_out, float* entropy_out, void* stream);
@@ -277,7 +284,9 @@ int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t pred_dim, 
  * int64 [n_rows, 1] (Categorical) or fp32 0/1 [n_rows, act_dim] (Bernoulli: action = [u < sigmoid(actor_out)], both
  * outputs get the same actions, each may be NULL; pred = act_dim; log_std, dist_min and dist_max must be NULL; noise of
  * 0.5 everywhere gives the deterministic action [p > 0.5]), log_prob fp32 [n_rows] (summed over the Bernoulli columns).
- * The Categorical head samples from softmax probs in actor_out.  Widths as for ppoaf_head_evaluate. */
+ * The Categorical head samples from softmax probs in actor_out; its raw_action_out may be NULL.  log_prob_out is
+ * required, as are log_std, raw_action_out and action_out for the Gaussian head.  Widths and non-finite inputs as for
+ * ppoaf_head_evaluate. */
 int ppoaf_head_sample(int32_t head, const float* actor_out, int32_t pred_dim, const float* log_std, float min_std,
                       const float* noise, const float* dist_min, const float* dist_max, int32_t act_dim,
                       int32_t n_rows, void* raw_action_out, void* action_out, float* log_prob_out, void* stream);

@@ -256,7 +256,7 @@ __device__ __forceinline__ CatColumn cat_column(float z, float mx, float se, flo
     CatColumn r;
     r.p = expf(z - mx) / se;
     r.pn = r.p / S;
-    r.lg = logf(fminf(fmaxf(r.pn, kCatEps), 1.f - kCatEps));
+    r.lg = logf(torch_clamp(r.pn, kCatEps, 1.f - kCatEps));
     return r;
 }
 
@@ -329,10 +329,10 @@ __device__ __forceinline__ float wide_gaussian_loss(const LossArgs& a, const flo
         const float sd = std_of_log_std(a.log_std[d], a.min_std, dstd), mu = pred[d], xd = x[d], z = xd - mu;
         s5[4] += isnan(mu) ? 1.f : 0.f;
         const float lsd = logf(sd);
-        s5[0] += fminf(fmaxf(-(z * z) / (2.f * (sd * sd)) - lsd - kLogSqrt2Pi, -100.f), 100.f);   // Normal.log_prob
+        s5[0] += torch_clamp(-(z * z) / (2.f * (sd * sd)) - lsd - kLogSqrt2Pi, -100.f, 100.f);   // Normal.log_prob
         const float th = tanhf(xd);
         s5[1] += logf(fmaxf(1.f - th * th, 1e-6f));
-        s5[2] += fminf(fmaxf(-lsd - kLogSqrt2Pi, -100.f), 100.f);                               // log N(mu; mu, sd)
+        s5[2] += torch_clamp(-lsd - kLogSqrt2Pi, -100.f, 100.f);                               // log N(mu; mu, sd)
         const float thm = tanhf(mu);
         s5[3] += logf(fmaxf(1.f - thm * thm, 1e-6f));
     }
@@ -547,12 +547,12 @@ __global__ void head_evaluate_kernel(const float* __restrict__ actor_out, int pr
     float nsum = 0.f, slog = 0.f, ensum = 0.f, eslog = 0.f;
     for (int d = 0; d < act_dim; ++d) {
         const float mu = pred[d], sd = s_sd[d], z = x[d] - mu, lsd = logf(sd);
-        nsum += fminf(fmaxf(-(z * z) / (2.f * (sd * sd)) - lsd - kLogSqrt2Pi, -100.f), 100.f);
+        nsum += torch_clamp(-(z * z) / (2.f * (sd * sd)) - lsd - kLogSqrt2Pi, -100.f, 100.f);
         const float th = tanhf(x[d]);
-        slog += logf(fmaxf(1.f - th * th, 1e-6f));
-        ensum += fminf(fmaxf(-lsd - kLogSqrt2Pi, -100.f), 100.f);
+        slog += logf(torch_clamp(1.f - th * th, 1e-6f, INFINITY));
+        ensum += torch_clamp(-lsd - kLogSqrt2Pi, -100.f, 100.f);
         const float thm = tanhf(mu);
-        eslog += logf(fmaxf(1.f - thm * thm, 1e-6f));
+        eslog += logf(torch_clamp(1.f - thm * thm, 1e-6f, INFINITY));
     }
     lp_out[i] = nsum - slog;
     if (ent_out) ent_out[i] = -(ensum - eslog);
@@ -587,8 +587,8 @@ __global__ void head_sample_kernel(const float* __restrict__ actor_out, int pred
         raw[d] = x;
         act[d] = a;
         const float dz = x - mu;
-        nsum += fminf(fmaxf(-(dz * dz) / (2.f * (sd * sd)) - logf(sd) - kLogSqrt2Pi, -100.f), 100.f);
-        slog += logf(fmaxf(1.f - th * th, 1e-6f));
+        nsum += torch_clamp(-(dz * dz) / (2.f * (sd * sd)) - logf(sd) - kLogSqrt2Pi, -100.f, 100.f);
+        slog += logf(torch_clamp(1.f - th * th, 1e-6f, INFINITY));
     }
     lp_out[i] = nsum - slog;
 }
@@ -614,7 +614,7 @@ __global__ void multi_categorical_evaluate_kernel(const float* __restrict__ acto
         const int a = int(act[k]);
         for (int d = o; d <= c; ++d) {
             const float pn = (expf(pred[d] - mx) / se) / S;
-            const float l = logf(fminf(fmaxf(pn, kCatEps), 1.f - kCatEps));
+            const float l = logf(torch_clamp(pn, kCatEps, 1.f - kCatEps));
             h += pn * l;
             if (d - o == a) lp += l;
         }
@@ -646,7 +646,7 @@ multi_categorical_sample_kernel(const float* __restrict__ probs, int pred_dim, u
         float S = 0.f;
         for (int d = 0; d < nk; ++d) S += p[o + d];
         int best = 0;
-        float best_v = -INFINITY, best_p = 0.f;
+        float best_v = -INFINITY, best_p = NAN;                    // no comparison holds (a NaN in the section): 0, NaN
         for (int d = 0; d < nk; ++d) {
             const float pn = p[o + d] / S;
             const float v = pn / q[d];
@@ -654,7 +654,7 @@ multi_categorical_sample_kernel(const float* __restrict__ probs, int pred_dim, u
         }
         act[k] = best;
         if (raw) raw[k] = best;
-        lp += logf(fminf(fmaxf(best_p, kCatEps), 1.f - kCatEps));
+        lp += logf(torch_clamp(best_p, kCatEps, 1.f - kCatEps));
         o = c + 1;
         ++k;
     }
@@ -731,12 +731,12 @@ gaussian_evaluate_wide_kernel(const float* __restrict__ actor_out, int pred_dim,
     float nsum = 0.f, slog = 0.f, ensum = 0.f, eslog = 0.f;
     for (int d = lane; d < act_dim; d += 32) {
         const float mu = pred[d], sd = s_sd[d], z = x[d] - mu, lsd = logf(sd);
-        nsum += fminf(fmaxf(-(z * z) / (2.f * (sd * sd)) - lsd - kLogSqrt2Pi, -100.f), 100.f);
+        nsum += torch_clamp(-(z * z) / (2.f * (sd * sd)) - lsd - kLogSqrt2Pi, -100.f, 100.f);
         const float th = tanhf(x[d]);
-        slog += logf(fmaxf(1.f - th * th, 1e-6f));
-        ensum += fminf(fmaxf(-lsd - kLogSqrt2Pi, -100.f), 100.f);
+        slog += logf(torch_clamp(1.f - th * th, 1e-6f, INFINITY));
+        ensum += torch_clamp(-lsd - kLogSqrt2Pi, -100.f, 100.f);
         const float thm = tanhf(mu);
-        eslog += logf(fmaxf(1.f - thm * thm, 1e-6f));
+        eslog += logf(torch_clamp(1.f - thm * thm, 1e-6f, INFINITY));
     }
     nsum = warp_sum(nsum); slog = warp_sum(slog); ensum = warp_sum(ensum); eslog = warp_sum(eslog);
     if (lane == 0) {
@@ -769,8 +769,8 @@ gaussian_sample_wide_kernel(const float* __restrict__ actor_out, int pred_dim, c
         raw[d] = x;
         act[d] = a;
         const float dz = x - mu;
-        nsum += fminf(fmaxf(-(dz * dz) / (2.f * (sd * sd)) - logf(sd) - kLogSqrt2Pi, -100.f), 100.f);
-        slog += logf(fmaxf(1.f - th * th, 1e-6f));
+        nsum += torch_clamp(-(dz * dz) / (2.f * (sd * sd)) - logf(sd) - kLogSqrt2Pi, -100.f, 100.f);
+        slog += logf(torch_clamp(1.f - th * th, 1e-6f, INFINITY));
     }
     nsum = warp_sum(nsum); slog = warp_sum(slog);
     if (lane == 0) lp_out[i] = nsum - slog;
@@ -819,7 +819,7 @@ categorical_sample_wide_kernel(const float* __restrict__ probs, int pred_dim, co
     for (int c = lane; c < pred_dim; c += 32) S += p[c];
     S = warp_sum(S);
     int best = pred_dim;                                              // past the row: loses every comparison
-    float best_v = -INFINITY, best_p = 0.f;
+    float best_v = -INFINITY, best_p = NAN;
     for (int c = lane; c < pred_dim; c += 32) {
         const float pn = p[c] / S;
         const float v = pn / q[c];
@@ -832,10 +832,10 @@ categorical_sample_wide_kernel(const float* __restrict__ probs, int pred_dim, co
         if (ov > best_v || (ov == best_v && oc < best)) { best_v = ov; best = oc; best_p = op; }
     }
     if (lane == 0) {
-        if (best == pred_dim) best = 0;                               // no comparison held (NaN row): column 0
+        if (best == pred_dim) best = 0;                               // no comparison held (NaN row): column 0, NaN
         act_out[i] = best;
         if (raw_out) raw_out[i] = best;
-        lp_out[i] = logf(fminf(fmaxf(best_p, kCatEps), 1.f - kCatEps));
+        lp_out[i] = logf(torch_clamp(best_p, kCatEps, 1.f - kCatEps));
     }
 }
 
@@ -866,6 +866,10 @@ extern "C" int ppoaf_head_sample(int32_t head, const float* actor_out, int32_t p
         PPOAF_CHECK_ARG(log_std == nullptr && dist_min == nullptr,
                         "ppoaf_head_sample: the Bernoulli head takes no log_std and no range bounds");
     }
+    PPOAF_CHECK_ARG(log_prob_out != nullptr, "ppoaf_head_sample: log_prob_out is required");
+    PPOAF_CHECK_ARG(head != PPOAF_HEAD_GAUSSIAN_TANH || (log_std != nullptr && raw_action_out != nullptr && action_out != nullptr),
+                    "ppoaf_head_sample: the Gaussian head needs log_std, raw_action_out and action_out");
+    PPOAF_CHECK_ARG(head != PPOAF_HEAD_CATEGORICAL || action_out != nullptr, "ppoaf_head_sample: the Categorical head needs action_out");
     if (n_rows == 0) return 0;
     if (head_is_wide(head, pred_dim, act_dim)) {
         const dim3 grid((n_rows + kWideRowsPerCta - 1) / kWideRowsPerCta), block(kWideRowThreads);
@@ -911,6 +915,8 @@ extern "C" int ppoaf_head_evaluate(int32_t head, const float* actor_out, int32_t
         PPOAF_CHECK_ARG(pred_dim == act_dim, "ppoaf_head_evaluate: Bernoulli actor output width must equal act_dim");
         PPOAF_CHECK_ARG(log_std == nullptr, "ppoaf_head_evaluate: the Bernoulli head takes no log_std");
     }
+    PPOAF_CHECK_ARG(log_prob_out != nullptr, "ppoaf_head_evaluate: log_prob_out is required");
+    PPOAF_CHECK_ARG(head != PPOAF_HEAD_GAUSSIAN_TANH || log_std != nullptr, "ppoaf_head_evaluate: the Gaussian head needs log_std");
     if (n_rows == 0) return 0;
     if (head_is_wide(head, pred_dim, act_dim)) {
         const dim3 grid((n_rows + kWideRowsPerCta - 1) / kWideRowsPerCta), block(kWideRowThreads);
@@ -948,6 +954,7 @@ extern "C" int ppoaf_multi_categorical_evaluate(const float* actor_out, int32_t 
                     "ppoaf_multi_categorical_evaluate: bad section table for %d outputs / %d sections (at most %d outputs)",
                     pred_dim, n_sections, kMaxAct);
     PPOAF_CHECK_ARG(n_rows >= 0, "ppoaf_multi_categorical_evaluate: n_rows < 0");
+    PPOAF_CHECK_ARG(log_prob_out != nullptr, "ppoaf_multi_categorical_evaluate: log_prob_out is required");
     if (n_rows == 0) return 0;
     multi_categorical_evaluate_kernel<<<(n_rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
         actor_out, pred_dim, ends, actions_i64, n_sections, n_rows, log_prob_out, entropy_out);
@@ -965,8 +972,9 @@ extern "C" int ppoaf_multi_categorical_sample(const float* probs, int32_t pred_d
                     "ppoaf_multi_categorical_sample: bad section table for %d outputs / %d sections (at most %d outputs)",
                     pred_dim, n_sections, kMaxAct);
     PPOAF_CHECK_ARG(n_rows >= 0, "ppoaf_multi_categorical_sample: n_rows < 0");
+    PPOAF_CHECK_ARG(noise != nullptr && actions_out_i64 != nullptr && log_prob_out != nullptr,
+                    "ppoaf_multi_categorical_sample: noise, actions_out_i64 and log_prob_out are required");
     if (n_rows == 0) return 0;
-    PPOAF_CHECK_ARG(noise != nullptr, "ppoaf_multi_categorical_sample: noise is required");
     multi_categorical_sample_kernel<<<(n_rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
         probs, pred_dim, ends, noise, n_sections, n_rows, actions_out_i64, log_prob_out, nullptr);
     PPOAF_CHECK_LAUNCH("ppoaf_multi_categorical_sample");

@@ -26,6 +26,10 @@ constexpr int kFusedStageSlots = kFusedMaxPred * (kG * kFusedMaxChunks) / 256;  
 constexpr float kLogSqrt2Pi = 0.91893853320467274178f;
 constexpr float kCatEps = 1.1920928955078125e-07f;   // torch.finfo(float32).eps
 
+// torch.clamp(x, lo, hi): a NaN x stays NaN (fminf / fmaxf alone would return a bound).  Finite and infinite x give
+// what fminf(fmaxf(x, lo), hi) gives.
+__device__ __forceinline__ float torch_clamp(float x, float lo, float hi) { return isnan(x) ? x : fminf(fmaxf(x, lo), hi); }
+
 __device__ __forceinline__ float softplus_torch(float x) { return x > 20.f ? x : log1pf(expf(x)); }
 
 __device__ __forceinline__ float critic_term(float v, float target, int use_huber, float& dv) {
@@ -104,18 +108,18 @@ __device__ __forceinline__ void section_sum(const float (&v)[kPerLane], const in
 // 1 - eps), l = log q - log1p(-q); log_prob(x) = logsigmoid(l) - (1 - x) l, entropy = (1 - p) l - logsigmoid(l)
 __device__ __forceinline__ float sigmoid_f(float z) { return 1.f / (1.f + expf(-z)); }
 __device__ __forceinline__ float bernoulli_logit(float p) {
-    const float q = fminf(fmaxf(p, kCatEps), 1.f - kCatEps);
+    const float q = torch_clamp(p, kCatEps, 1.f - kCatEps);
     return logf(q) - log1pf(-q);
 }
 __device__ __forceinline__ float log_sigmoid(float l) { return fminf(l, 0.f) - log1pf(expf(-fabsf(l))); }
 
 // std = max(softplus(log_std), min_std) (distributions.py:514-515) and dstd = d std / d log_std (torch's max splits the
-// gradient evenly on a tie)
+// gradient evenly on a tie); a NaN log_std gives a NaN std
 __device__ __forceinline__ float std_of_log_std(float ls, float min_std, float& dstd) {
     const float sp = softplus_torch(ls);
     const float sig = ls > 20.f ? 1.f : 1.f / (1.f + expf(-ls));
     dstd = sp > min_std ? sig : (sp == min_std ? 0.5f * sig : 0.f);
-    return fmaxf(sp, min_std);
+    return torch_clamp(sp, min_std, INFINITY);
 }
 
 // Clipped surrogate of one sample from its log-prob and entropy: returns dL/d lp; `first` (lane 0 of a live sample)
@@ -160,12 +164,12 @@ __device__ __forceinline__ void actor_head_loss(const LossArgs& a, int head, boo
                 bad_value = fmaxf(bad_value, isnan(mu[k]) ? 1.f : 0.f);
                 const float lsd = logf(sd);
                 const float nl = -(z[k] * z[k]) / (2.f * (sd * sd)) - lsd - kLogSqrt2Pi;   // Normal.log_prob
-                nsum += fminf(fmaxf(nl, -100.f), 100.f);
+                nsum += torch_clamp(nl, -100.f, 100.f);
                 on[k] = (nl >= -100.f && nl <= 100.f) ? 1.f : 0.f;
                 const float th = tanhf(xd);
                 slog += logf(fmaxf(1.f - th * th, 1e-6f));
                 const float nle = -lsd - kLogSqrt2Pi;                                     // log N(mu; mu, sd)
-                ensum += fminf(fmaxf(nle, -100.f), 100.f);
+                ensum += torch_clamp(nle, -100.f, 100.f);
                 one[k] = (nle >= -100.f && nle <= 100.f) ? 1.f : 0.f;
                 thm[k] = tanhf(mu[k]);
                 eslog += logf(fmaxf(1.f - thm[k] * thm[k], 1e-6f));

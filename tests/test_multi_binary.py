@@ -169,9 +169,10 @@ def _cfg(pred, act_dim):
     return cfg
 
 
-def test_bernoulli_width_mismatch_is_refused_through_the_c_abi():
+def test_bernoulli_width_mismatch_is_refused_ahead_of_the_output_checks():
     """The update entry points refuse act_dim != actor output width before they touch the device; so do the
-    stand-alone head entry points (which then return without launching for zero rows)."""
+    stand-alone head entry points, ahead of their check for a log_prob_out, and with one given they return without
+    launching for zero rows."""
     from ppo_and_friends_b200 import _lib
     from ppo_and_friends_b200.build import build
     build()
@@ -191,9 +192,9 @@ def test_bernoulli_width_mismatch_is_refused_through_the_c_abi():
     assert "Bernoulli actor output width" in msg()
     assert lib.ppoaf_head_evaluate(H, None, 7, fake, 0.01, None, 7, 0, None, None, None) != 0
     assert "log_std" in msg()
-    assert lib.ppoaf_head_evaluate(H, None, 7, None, 0.01, None, 7, 0, None, None, None) == 0
+    assert lib.ppoaf_head_evaluate(H, None, 7, None, 0.01, None, 7, 0, fake, None, None) == 0
     sample = lambda pred, act_dim, log_std=None, lo=None, hi=None: lib.ppoaf_head_sample(
-        H, None, pred, log_std, 0.01, fake, lo, hi, act_dim, 0, None, None, None, None)
+        H, None, pred, log_std, 0.01, fake, lo, hi, act_dim, 0, None, None, fake, None)
     assert sample(7, 6) != 0 and "Bernoulli actor output width" in msg()
     assert sample(7, 7, log_std=fake) != 0 and "log_std" in msg()
     assert sample(7, 7, lo=fake, hi=fake) != 0 and "range bounds" in msg()

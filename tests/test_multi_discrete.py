@@ -163,9 +163,10 @@ def _cfg(nvec, ends, act_dim):
     return cfg
 
 
-def test_malformed_section_table_is_refused_through_the_c_abi():
+def test_malformed_section_table_is_refused_ahead_of_the_output_checks():
     """The update entry points validate the configuration before they touch the device; so do the stand-alone head
-    entry points (which then return without launching for zero rows)."""
+    entry points, ahead of their checks for noise and outputs, and with those given they return without launching for
+    zero rows."""
     from ppo_and_friends_b200 import _lib
     from ppo_and_friends_b200.build import build
     build()
@@ -188,8 +189,9 @@ def test_malformed_section_table_is_refused_through_the_c_abi():
         assert "section table" in msg()
         assert lib.ppoaf_multi_categorical_sample(None, 7, ends & 0xFFFFFFFF, ends >> 32, None, act_dim, 0,
                                                   None, None, None) != 0
-    assert lib.ppoaf_multi_categorical_evaluate(None, 7, good, 0, None, 3, 0, None, None, None) == 0
-    assert lib.ppoaf_multi_categorical_sample(None, 7, good, 0, None, 3, 0, None, None, None) == 0
+    fake = C.c_void_p(16)                                                        # never dereferenced: zero rows
+    assert lib.ppoaf_multi_categorical_evaluate(None, 7, good, 0, None, 3, 0, fake, None, None) == 0
+    assert lib.ppoaf_multi_categorical_sample(None, 7, good, 0, fake, 3, 0, fake, fake, None) == 0
 
 
 # ----------------------------------------------------------------------------------------- GPU

@@ -52,9 +52,10 @@ def _cfg(head, pred, act_dim, ends=0):
     return cfg
 
 
-def test_wide_widths_through_the_c_abi():
+def test_wide_widths_through_the_c_abi_with_required_outputs():
     """In-bound wide Categorical / Gaussian widths pass the width checks of the update and head entry points (with
-    empty buffers the update calls are then refused for another reason; zero-row head calls return without launching).
+    empty buffers the update calls are then refused for another reason; zero-row head calls given log_std and their
+    required outputs return without launching).
     Wider rows, and Bernoulli / multi-categorical rows above 64, are refused with a message naming the width."""
     from ppo_and_friends_b200 import _lib
     from ppo_and_friends_b200.build import build
@@ -78,8 +79,9 @@ def test_wide_widths_through_the_c_abi():
         assert lib.ppoaf_ppo_fused_supported(C.byref(_cfg(head, pred, act_dim))) == 0
     fake = C.c_void_p(16)                                                        # never dereferenced: zero rows
     for head, pred, act_dim in ok:
-        assert lib.ppoaf_head_evaluate(head, None, pred, None, 0.01, None, act_dim, 0, None, None, None) == 0, msg()
-        assert lib.ppoaf_head_sample(head, None, pred, None, 0.01, fake, None, None, act_dim, 0, None, None, None,
+        log_std = fake if head == GAUSS else None
+        assert lib.ppoaf_head_evaluate(head, None, pred, log_std, 0.01, None, act_dim, 0, fake, None, None) == 0, msg()
+        assert lib.ppoaf_head_sample(head, None, pred, log_std, 0.01, fake, None, None, act_dim, 0, fake, fake, fake,
                                      None) == 0, msg()
     for head, pred, act_dim, _ in bad[:3]:
         assert lib.ppoaf_head_evaluate(head, None, pred, None, 0.01, None, act_dim, 0, None, None, None) != 0
