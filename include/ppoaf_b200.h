@@ -315,6 +315,14 @@ int ppoaf_multi_categorical_sample(const float* probs, int32_t pred_dim, uint32_
  * clip, Adam.  Buffers come from ppoaf_peer_alloc (cudaMalloc) and are shared with CUDA IPC
  * handles that the host exchanges through torch.distributed; gradients are double-buffered by step
  * parity so one barrier per step suffices.  `ctrl`: local zeroed scratch of ppoaf_peer_ctrl_bytes().
+ * n_ranks = 1 is accepted (peer_grads[0] / peer_flags[0] local buffers).
+ * Launch-order preconditions (both fused exchanges):
+ *  - the kernel is launched with programmatic stream serialization and reads params, m and v BEFORE
+ *    its dependency wait, so the launch right before it on the stream must not write them.  In a
+ *    training step that launch is the last backward GEMM.  Never enqueue two calls back to back:
+ *    put an ordinary stream operation (the gradient writes of the step) between them.
+ *  - one `ctrl` block serves one network size: its grid barrier counts calls x grid, so a call with
+ *    a different parameter count (a different grid) needs its own zeroed `ctrl`.
  * ---------------------------------------------------------------------------------------- */
 int    ppoaf_peer_alloc(size_t bytes, void** out);
 int    ppoaf_peer_free(void* p);
@@ -333,7 +341,9 @@ int    ppoaf_peer_allreduce_adam(const void* const* peer_grads, void* const* pee
  * sum of its slice, the slice norms are exchanged through the flag blocks, the owner applies clip + Adam (m, v are only
  * maintained for the owned slice) and stores the new parameters in its staging buffer; every rank then gathers all slices
  * from their owners' staging buffers (staging[r], peer mappings).  ~2 x 4 B/parameter of NVLink traffic per rank and
- * step, independent of R. */
+ * step, independent of R.  Outside the owned slice adam_m / adam_v go stale: gather every owner's slice before reading
+ * the full moments (a checkpoint).  The launch-order preconditions of ppoaf_peer_allreduce_adam apply (no two calls
+ * back to back; one zeroed `ctrl` per network size). */
 size_t ppoaf_nvls_ctrl_bytes(void);
 size_t ppoaf_nvls_flag_block_bytes(void);
 int    ppoaf_nvls_allreduce_adam(const float* g_mc, void* const* staging, void* const* flag_blocks,

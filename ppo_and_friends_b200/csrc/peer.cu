@@ -521,7 +521,10 @@ extern "C" size_t ppoaf_peer_ctrl_bytes(void) {
 }
 
 // peer_grads[r] / peer_flags[r]: pointers valid on THIS device for rank r's buffers (own rank: the local pointers).
-// ctrl: local zero-initialised scratch of ppoaf_peer_ctrl_bytes() bytes (CTA partials | arrival words | control words).
+// ctrl: local zero-initialised scratch of ppoaf_peer_ctrl_bytes() bytes (CTA partials | arrival words | control words),
+// one per network size (the grid barrier counts calls x grid on ctrl[2]).
+// The kernel fetches params / m / v before its dependency wait: the launch before it must not write them, so two calls
+// must never be enqueued back to back (the step's gradient writes come between them).
 extern "C" int ppoaf_peer_allreduce_adam(const void* const* peer_grads, void* const* peer_flags, int32_t n_ranks,
                                          int32_t my_rank, float* params, float* adam_m, float* adam_v,
                                          int64_t* adam_step, int32_t* mb_cursor, const double* hparams,
@@ -569,6 +572,8 @@ extern "C" size_t ppoaf_nvls_flag_block_bytes(void) { return 256; }
 // g_mc: multicast address of this parity's gradient buffer; staging[r]: rank r's parameter staging buffer mapped on
 // this device; flag_blocks[r]: rank r's zero-initialised flag block mapped on this device
 // (ppoaf_nvls_flag_block_bytes() bytes, symmetric memory); ctrl: local zeroed scratch of ppoaf_nvls_ctrl_bytes().
+// Same launch-order precondition as ppoaf_peer_allreduce_adam: never two calls back to back.  m and v are current only
+// on the owned slice (NvlsGroup.gather_moments assembles them for a checkpoint).
 extern "C" int ppoaf_nvls_allreduce_adam(const float* g_mc, void* const* staging, void* const* flag_blocks,
                                          int32_t n_ranks, int32_t my_rank, float* params, float* adam_m, float* adam_v,
                                          int64_t* adam_step, int32_t* mb_cursor, const double* hparams, int64_t n_actor,

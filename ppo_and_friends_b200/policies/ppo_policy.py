@@ -529,6 +529,10 @@ class PPOPolicy:
     def _save_optimizers(self, save_path):
         if self.test_mode:
             return
+        # the NVLS exchange keeps each rank's moments current only on the slice it owns: assemble them first
+        peer = getattr(self._engine, "peer", None)
+        if hasattr(peer, "gather_moments"):
+            peer.gather_moments(self.nets)
         torch.save(self.actor_optim.state_dict(), os.path.join(save_path, f"actor_optim_{get_rank()}"))
         torch.save(self.critic_optim.state_dict(), os.path.join(save_path, f"critic_optim_{get_rank()}"))
 

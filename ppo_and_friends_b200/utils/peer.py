@@ -151,6 +151,21 @@ class NvlsGroup:
         off = self._ctrl_bytes - 256 + 16
         return int(self.ctrl[off:off + 4].view(torch.int32).item())
 
+    def gather_moments(self, nets):
+        """The kernel keeps adam_m / adam_v current only on the float4 rows this rank owns, [r * slice, (r + 1) * slice)
+        with slice = ceil(nv / R).  Gather every owner's rows, so each rank holds the full moments a torch.optim.Adam
+        would (before a checkpoint).  Collective: every rank calls it."""
+        nv = (nets.n_actor + nets.n_critic) // 4
+        sl = -(-nv // self.world)
+        lo, hi = min(nv, self.rank * sl), min(nv, (self.rank + 1) * sl)
+        for buf in (nets.adam_m, nets.adam_v):
+            rows = buf[:4 * nv].view(nv, 4)
+            mine = torch.zeros(sl, 4, dtype=buf.dtype, device=buf.device)
+            mine[:hi - lo] = rows[lo:hi]
+            full = torch.empty(self.world * sl, 4, dtype=buf.dtype, device=buf.device)
+            dist.all_gather_into_tensor(full, mine)
+            rows.copy_(full[:nv])
+
     def close(self):
         torch.cuda.synchronize(self.device)
         if dist.is_initialized():
