@@ -30,8 +30,26 @@ extern "C" {
 #define PPOAF_ABI_VERSION 1
 #define PPOAF_MAX_LAYERS 8
 
-/* activation ids (hidden layers of FeedForwardNetwork, networks/utils.py:160-183) */
-enum { PPOAF_ACT_IDENTITY = 0, PPOAF_ACT_RELU = 1, PPOAF_ACT_LEAKY_RELU = 2, PPOAF_ACT_TANH = 3 };
+/* activation ids (hidden layers of FeedForwardNetwork, networks/utils.py:160-183): the torch module, its formula, and
+ * how the backward pass gets act'(z).  "output": recovered from the stored activation output y.  "stored": the function
+ * is not invertible, so the update's forward also writes act'(z) to a per-hidden-layer buffer of its workspace; the
+ * one-launch engine (ppoaf_ppo_fused_steps) does not take these ids. */
+enum {
+    PPOAF_ACT_IDENTITY = 0,
+    PPOAF_ACT_RELU = 1,        /* nn.ReLU: max(x, 0); output: y > 0 ? 1 : 0 */
+    PPOAF_ACT_LEAKY_RELU = 2,  /* nn.LeakyReLU(0.01): x > 0 ? x : 0.01 x; output: y > 0 ? 1 : 0.01 */
+    PPOAF_ACT_TANH = 3,        /* nn.Tanh; output: 1 - y^2 */
+    PPOAF_ACT_ELU = 4,         /* nn.ELU() / nn.CELU() (alpha = 1): x > 0 ? x : expm1(x); output: y > 0 ? 1 : y + 1 */
+    PPOAF_ACT_SELU = 5,        /* nn.SELU: lambda (x > 0 ? x : alpha expm1(x)); output: y > 0 ? lambda : y + lambda alpha */
+    PPOAF_ACT_SIGMOID = 6,     /* nn.Sigmoid: 1 / (1 + exp(-x)); output: y (1 - y) */
+    PPOAF_ACT_SOFTPLUS = 7,    /* nn.Softplus() (beta = 1, threshold = 20): x > 20 ? x : log1p(exp(x)); output: -expm1(-y) */
+    PPOAF_ACT_SILU = 8,        /* nn.SiLU: x / (1 + exp(-x)); stored: s (1 + x (1 - s)), s = sigmoid(x) */
+    PPOAF_ACT_GELU = 9,        /* nn.GELU(): 0.5 x (1 + erf(x / sqrt 2)); stored: Phi(x) + x phi(x) */
+    PPOAF_ACT_GELU_TANH = 10,  /* nn.GELU('tanh'): 0.5 x (1 + tanh(t)), t = sqrt(2/pi) (x + 0.044715 x^3);
+                                * stored: 0.5 (1 + tanh t) + 0.5 x (1 - tanh^2 t) sqrt(2/pi) (1 + 3 0.044715 x^2) */
+    PPOAF_ACT_MISH = 11,       /* nn.Mish: x tanh(sp), sp = log1p(exp(x)); stored: tanh(sp) + x sigmoid(x) (1 - tanh^2 sp) */
+    PPOAF_ACT_COUNT = 12
+};
 /* action heads (networks/distributions.py).  PPOAF_HEAD_MULTI_CATEGORICAL (MultiDiscrete action spaces,
  * MultiCategoricalDistribution :272-438) is a restatement, not pinned by a reference golden: softmax over the whole
  * actor output row, then one torch Categorical(probs) per section of the row (renormalised, clamped to [eps, 1-eps]);

@@ -14,7 +14,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "csrc", "libppoaf_b200.so")
 
 MAX_LAYERS = 8
-ACT_IDS = {"identity": 0, "relu": 1, "leaky_relu": 2, "tanh": 3}
+ACT_IDS = {"identity": 0, "relu": 1, "leaky_relu": 2, "tanh": 3, "elu": 4, "selu": 5, "sigmoid": 6, "softplus": 7,
+           "silu": 8, "gelu": 9, "gelu_tanh": 10, "mish": 11}
 HEAD_GAUSSIAN_TANH, HEAD_CATEGORICAL, HEAD_MULTI_CATEGORICAL, HEAD_BERNOULLI = 0, 1, 2, 3
 
 HP = dict(LR=0, ENTROPY_WEIGHT=1, SURR_CLIP=2, GRAD_CLIP=3, KL_WEIGHT=4, VF_CLIP=5, BETA1=6, BETA2=7,

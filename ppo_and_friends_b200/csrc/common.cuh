@@ -117,6 +117,70 @@ __device__ __forceinline__ float fast_tanh(float x) {
     const float t = __expf(2.f * x);
     return 1.f - __fdividef(2.f, t + 1.f);
 }
+// ---- hidden-layer activations beyond relu / leaky relu / tanh (ids and formulas: ppoaf_b200.h) ----
+// Each is written as torch's CUDA kernel writes it (accurate libm, float32), so NaN and +-Inf come out where torch's do.
+// SiLU, GELU and Mish cannot recover act'(z) from their output: the update's forward stores it (act_fwd_grad).
+// The three helpers are called, not inlined, so each epilogue carries one call site instead of eight functions.
+__host__ __device__ __forceinline__ bool act_stores_derivative(int act) {
+    return act >= PPOAF_ACT_SILU && act <= PPOAF_ACT_MISH;
+}
+constexpr float kSeluScale = 1.0507009873554804934193349852946f;
+constexpr float kSeluScaleAlpha = float(1.0507009873554804934193349852946 * 1.6732632423543772848170429916717);
+constexpr float kSqrtHalf = 0.70710678118654752440f;
+constexpr float kInvSqrt2Pi = 0.39894228040143267794f;
+constexpr float kGeluTanhBeta = 0.79788456080286535588f;     // sqrt(2 / pi)
+constexpr float kGeluTanhKappa = 0.044715f;
+
+static __device__ __noinline__ float act_fwd_ext(float x, int act) {
+    switch (act) {
+        case PPOAF_ACT_ELU: return x > 0.f ? x : expm1f(x);
+        case PPOAF_ACT_SELU: return x > 0.f ? kSeluScale * x : kSeluScaleAlpha * expm1f(x);
+        case PPOAF_ACT_SIGMOID: return 1.f / (1.f + expf(-x));
+        case PPOAF_ACT_SOFTPLUS: return x > 20.f ? x : log1pf(expf(x));
+        case PPOAF_ACT_SILU: return x / (1.f + expf(-x));
+        case PPOAF_ACT_GELU: return 0.5f * x * (1.f + erff(x * kSqrtHalf));
+        case PPOAF_ACT_GELU_TANH: return 0.5f * x * (1.f + tanhf(kGeluTanhBeta * (x + kGeluTanhKappa * (x * x * x))));
+        case PPOAF_ACT_MISH: return x * tanhf(log1pf(expf(x)));
+        default: return x;
+    }
+}
+// act'(z) from the output y (ids 4-7; torch's elu_backward / sigmoid_backward / softplus_backward in terms of y)
+static __device__ __noinline__ float act_bwd_ext(float y, int act) {
+    switch (act) {
+        case PPOAF_ACT_ELU: return y > 0.f ? 1.f : y + 1.f;
+        case PPOAF_ACT_SELU: return y > 0.f ? kSeluScale : y + kSeluScaleAlpha;
+        case PPOAF_ACT_SIGMOID: return y * (1.f - y);
+        case PPOAF_ACT_SOFTPLUS: return -expm1f(-y);
+        default: return y;                          // ids 8-11: y is the stored act'(z)
+    }
+}
+// ids 8-11: the output (.x) and act'(z) (.y) at once (torch's silu_backward, gelu_backward and mish_backward formulas)
+static __device__ __noinline__ float2 act_fwd_grad(float x, int act) {
+    switch (act) {
+        case PPOAF_ACT_SILU: {
+            const float e = 1.f + expf(-x), s = 1.f / e;
+            return make_float2(x / e, s * (1.f + x * (1.f - s)));
+        }
+        case PPOAF_ACT_GELU: {
+            const float cdf = 0.5f * (1.f + erff(x * kSqrtHalf));
+            return make_float2(x * cdf, cdf + x * (expf(-0.5f * x * x) * kInvSqrt2Pi));
+        }
+        case PPOAF_ACT_GELU_TANH: {
+            const float x2 = x * x;
+            const float t = tanhf(kGeluTanhBeta * (x + kGeluTanhKappa * (x2 * x)));
+            const float left = 0.5f * x, right = 1.f + t;
+            return make_float2(left * right,
+                               0.5f * right + left * (1.f - t * t) * kGeluTanhBeta * (1.f + 3.f * kGeluTanhKappa * x2));
+        }
+        default: {                                  // PPOAF_ACT_MISH
+            const float t = tanhf(log1pf(expf(x))), s = 1.f / (1.f + expf(-x));
+            return make_float2(x * t, t + x * s * (1.f - t * t));
+        }
+    }
+}
+
+// EXT = false: the grouped GEMM's kernel for ids 0-3, which must not carry the code of the others (mlp.cuh)
+template <bool EXT = true>
 __device__ __forceinline__ void act_fwd4(float (&o)[4], int act) {
     if (act == PPOAF_ACT_TANH) {
 #pragma unroll
@@ -127,8 +191,13 @@ __device__ __forceinline__ void act_fwd4(float (&o)[4], int act) {
     } else if (act == PPOAF_ACT_LEAKY_RELU) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) o[j] = o[j] > 0.f ? o[j] : 0.01f * o[j];
+    } else if (EXT && act >= PPOAF_ACT_ELU) {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) o[j] = act_fwd_ext(o[j], act);
     }
 }
+// y: the activation output of the layer (ids 1-7) or its stored act'(z) (ids 8-11)
+template <bool EXT = true>
 __device__ __forceinline__ void act_bwd4(float (&o)[4], const float (&y)[4], int act) {
     if (act == PPOAF_ACT_TANH) {
 #pragma unroll
@@ -139,6 +208,9 @@ __device__ __forceinline__ void act_bwd4(float (&o)[4], const float (&y)[4], int
     } else if (act == PPOAF_ACT_LEAKY_RELU) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) o[j] = y[j] > 0.f ? o[j] : 0.01f * o[j];
+    } else if (EXT && act >= PPOAF_ACT_ELU) {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) o[j] *= act_bwd_ext(y[j], act);
     }
 }
 

@@ -1025,6 +1025,7 @@ static const char* unsupported_reason(const ppoaf_update_cfg* cfg) {
     if (La != Lc) return "actor and critic depths differ";
     if (La < 2) return "networks without a hidden layer";
     if (cfg->actor.activation != cfg->critic.activation) return "actor and critic activations differ";
+    if (act_stores_derivative(cfg->actor.activation)) return "activation needs a stored derivative";
     if (!loss_head_fusable(cfg->actor.dims[La], cfg->actor.dims[La - 1], cfg->critic.dims[Lc - 1], cfg->vf_clip_enabled))
         return "head layers are not fusable (hidden width > 256 or not a multiple of 4, > 24 actor outputs, or value clipping)";
     if (cfg->act_dim > kMaxAct || cfg->actor.dims[La] > kMaxAct) return "action width out of range";

@@ -17,12 +17,12 @@ struct GemmGroup {
     ~GemmGroup();
     GemmGroup(const GemmGroup&) = delete;
     GemmGroup& operator=(const GemmGroup&) = delete;
-    // Y[rows, out] = act(X[idx][rows, in] W^T + b)
+    // Y[rows, out] = act(X[idx][rows, in] W^T + b); dact (FFMA tiles, act_stores_derivative ids): act'(z) [rows, out]
     // w_static / x_static: the operand is not written by the launch that precedes this one in the stream, so the
     // FFMA kernel may stage it before its programmatic-dependency wait (see common.cuh, PDL)
     void add_forward(const float* X, int ldx, const int64_t* idx, const float* W, const float* b, float* Y, int rows,
-                     int in, int out, int act, bool w_static = false);
-    // dX[rows, in] = (dZ[rows, out] W[out, in]) * act'(Xact[rows, in])
+                     int in, int out, int act, bool w_static = false, float* dact = nullptr);
+    // dX[rows, in] = (dZ[rows, out] W[out, in]) * act'(Xact[rows, in]); act_stores_derivative ids: Xact is act'(z)
     void add_backward_x(const float* dZ, const float* W, const float* Xact, float* dX, int rows, int in, int out, int act);
     // dW[out, in] = dZ[rows, out]^T X[idx][rows, in]; db[out] = column sums of dZ; sq_out[tile] = tile sum of squares
     // returns the number of sum-of-squares slots (tiles) this problem writes
@@ -80,6 +80,8 @@ struct LossArgs {
     const float* b_critic;       // [1]
     float* dz_actor;             // [batch, Ha]  dL/d(pre-activation of the layer below the head)
     float* dz_critic;            // [batch, Hc]
+    const float* dact_actor;     // act_stores_derivative ids: act'(z) below the heads, [batch, Ha] / [batch, Hc]; else null
+    const float* dact_critic;
     int Ha, Hc, act;
     int n_mirror;                // peer copies of d_log_std (push exchange)
     long long mirror_delta[PPOAF_MAX_MIRROR];

@@ -67,7 +67,8 @@ __device__ __forceinline__ void loss_epilogue(const LossArgs& a, const double* s
     *a.ticket = 0u;  // ready for the next launch
 }
 
-template <bool FUSED>
+// DACT (FUSED only): the heads' dX is multiplied by the stored act'(z) of the layer below (act_stores_derivative ids)
+template <bool FUSED, bool DACT>
 __global__ void __launch_bounds__(kLossThreads) ppo_loss_kernel(const LossArgs a) {
     extern __shared__ __align__(16) float s_dyn[];      // FUSED: HeadSmem
     __shared__ float s_sd[kMaxAct], s_dsd[kMaxAct];
@@ -186,7 +187,20 @@ __global__ void __launch_bounds__(kLossThreads) ppo_loss_kernel(const LossArgs a
     const float bad_any = group_max(bad_value);
     sc[LS_BAD_VALUE] = (live && gl == 0) ? bad_any : 0.f;
 
-    if constexpr (FUSED) head_backward(a, hs, ha, hc, sdp, dv1, inv_b, live, gl, live ? i : 0);
+    if constexpr (FUSED) {
+        if constexpr (DACT) {   // the factors of the dz rows: the stored act'(z), not a function of the activations
+                                //   (actor and critic share the activation here)
+            const float* dra = a.dact_actor + int64_t(live ? i : 0) * a.Ha + 4 * gl;
+            const float* drc = a.dact_critic + int64_t(live ? i : 0) * a.Hc + 4 * gl;
+#pragma unroll
+            for (int c = 0; c < kFusedMaxChunks; ++c) {
+                const int col = 4 * (gl + kG * c);
+                ha[c] = (col < a.Ha && live) ? *reinterpret_cast<const float4*>(dra + 4 * kG * c) : make_float4(0.f, 0.f, 0.f, 0.f);
+                hc[c] = (col < a.Hc && live) ? *reinterpret_cast<const float4*>(drc + 4 * kG * c) : make_float4(0.f, 0.f, 0.f, 0.f);
+            }
+        }
+        head_backward(a, hs, ha, hc, sdp, dv1, inv_b, live, gl, live ? i : 0);
+    }
 
     LOSS_STAMP(5);
     // ---------------- CTA partials; the last CTA to finish folds them ----------------
@@ -505,9 +519,12 @@ int launch_ppo_loss(const LossArgs& a, cudaStream_t s) {
             PPOAF_CHECK_ARG(loss_head_fusable(a.pred_dim, a.Ha, a.Hc, a.vf_clip_enabled), "ppo loss: head layers are not fusable");
             const size_t smem = sizeof(float) * size_t((a.pred_dim + kPB - 1) / kPB * kPB * (a.Ha + 4) + a.Hc + ((a.pred_dim + 1 + 3) & ~3) +
                                                        2 * kSamplesPerBlock * kFusedPredLd);
-            launch_chain(ppo_loss_kernel<true>, dim3(blocks), dim3(kLossThreads), smem, s, a);
+            if (a.dact_actor)
+                launch_chain(ppo_loss_kernel<true, true>, dim3(blocks), dim3(kLossThreads), smem, s, a);
+            else
+                launch_chain(ppo_loss_kernel<true, false>, dim3(blocks), dim3(kLossThreads), smem, s, a);
         } else {
-            launch_chain(ppo_loss_kernel<false>, dim3(blocks), dim3(kLossThreads), 0, s, a);
+            launch_chain(ppo_loss_kernel<false, false>, dim3(blocks), dim3(kLossThreads), 0, s, a);
         }
         PPOAF_CHECK_LAUNCH("ppo_loss_kernel");
         wsel_at = size_t(blocks) * kPartialStride;

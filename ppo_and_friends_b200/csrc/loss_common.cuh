@@ -384,7 +384,8 @@ __device__ __forceinline__ float head_forward(const LossArgs& a, const HeadSmem&
 }
 
 // Head layers, backward: dX of the two head layers (dL/d actor outputs in dpred, dL/d value dv * inv_b) times the
-// activation derivative of the layer below, stored to row `row` of dz_actor / dz_critic
+// activation derivative of the layer below, stored to row `row` of dz_actor / dz_critic.  ha / hc: that layer's
+// activations, or its stored act'(z) for act_stores_derivative ids (act_bwd4)
 __device__ __forceinline__ void head_backward(const LossArgs& a, const HeadSmem& s, const float4 (&ha)[kFusedMaxChunks],
                                               const float4 (&hc)[kFusedMaxChunks], const float* dpred, float dv,
                                               float inv_b, bool live, int gl, int64_t row) {

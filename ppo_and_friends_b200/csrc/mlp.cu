@@ -16,6 +16,7 @@ static bool g_gemm_configured = false;
 void configure_gemm_kernels() {
     g_gemm_configured = true;
     cudaFuncSetAttribute(grouped_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kGemmSmemBytes));
+    cudaFuncSetAttribute(grouped_gemm_ext_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kGemmSmemBytes));
     cudaFuncSetAttribute(umma::umma_grouped_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                          int(umma::kUmmaSmemBytes));
 }
@@ -37,13 +38,13 @@ static GemmProblem* next_problem(GemmGroup* grp, int M, int N) {
 }
 
 void GemmGroup::add_forward(const float* X, int ldx, const int64_t* idx, const float* W, const float* b, float* Y,
-                            int rows, int in, int out, int act, bool w_static) {
+                            int rows, int in, int out, int act, bool w_static, float* dact) {
     GemmProblem* g = next_problem(this, rows, out);
     g->b_static = w_static ? 1 : 0;
     g->A = X; g->lda = ldx; g->B = W; g->ldb = in; g->C = Y; g->ldc = out;
     g->M = rows; g->N = out; g->K = in;
-    g->idxA = idx; g->bias = b; g->act = act;
-    g->flavour = EPI_FWD * 4 + (vec4_ok(X, ldx, in) ? 2 : 0) + (vec4_ok(W, in, in) ? 1 : 0);
+    g->idxA = idx; g->bias = b; g->act = act; g->dact = dact;
+    g->flavour = (dact ? EPI_FWD_DACT : EPI_FWD) * 4 + (vec4_ok(X, ldx, in) ? 2 : 0) + (vec4_ok(W, in, in) ? 1 : 0);
 }
 
 void GemmGroup::add_backward_x(const float* dZ, const float* W, const float* Xact, float* dX, int rows, int in,
@@ -80,11 +81,16 @@ int GemmGroup::launch(const int32_t* cursor, int cursor_stride, cudaStream_t s, 
     for (int q = 0; q < n_mirror && q < PPOAF_MAX_MIRROR; ++q) args->mirror.delta[q] = mirror_delta[q];
     if (backend == GEMM_BACKEND_TCGEN05) {
         for (int i = 0; i < args->n_problems; ++i)
-            PPOAF_CHECK_ARG(args->p[i].flavour >> 2 == EPI_FWD, "GemmGroup::launch: the tcgen05 tiles run forward problems only");
+            PPOAF_CHECK_ARG(args->p[i].flavour >> 2 == EPI_FWD,
+                            "GemmGroup::launch: the tcgen05 tiles run forward problems without a stored derivative only");
         launch_chain(umma::umma_grouped_gemm_kernel, dim3(n_tiles), dim3(umma::kUThreads + 32), umma::kUmmaSmemBytes, s, *args);
         PPOAF_CHECK_LAUNCH("umma_grouped_gemm_kernel");
     } else {
-        launch_chain(grouped_gemm_kernel, dim3(n_tiles), dim3(kThreads), kGemmSmemBytes, s, *args);
+        bool ext = false;                 // activation ids 4-11 run on the kernel that carries their code
+        for (int i = 0; i < args->n_problems; ++i)
+            ext |= args->p[i].act >= PPOAF_ACT_ELU || args->p[i].flavour >> 2 == EPI_FWD_DACT;
+        launch_chain(ext ? grouped_gemm_ext_kernel : grouped_gemm_kernel, dim3(n_tiles), dim3(kThreads), kGemmSmemBytes, s,
+                     *args);
         PPOAF_CHECK_LAUNCH("grouped_gemm_kernel");
     }
     return 0;
@@ -146,8 +152,8 @@ int check_mlp_desc(const ppoaf_mlp_desc* net, const char* who) {
     PPOAF_CHECK_ARG(net != nullptr, "%s: null mlp desc", who);
     PPOAF_CHECK_ARG(net->n_layers >= 1 && net->n_layers <= PPOAF_MAX_LAYERS, "%s: n_layers out of range", who);
     for (int l = 0; l <= net->n_layers; ++l) PPOAF_CHECK_ARG(net->dims[l] > 0, "%s: dims[%d] must be > 0", who, l);
-    PPOAF_CHECK_ARG(net->activation >= PPOAF_ACT_IDENTITY && net->activation <= PPOAF_ACT_TANH,
-                    "%s: unknown activation", who);
+    PPOAF_CHECK_ARG(net->activation >= PPOAF_ACT_IDENTITY && net->activation < PPOAF_ACT_COUNT,
+                    "%s: unknown activation id %d", who, net->activation);
     return 0;
 }
 

@@ -33,27 +33,35 @@ __device__ __forceinline__ float act_fwd(float x, int act) {
         case PPOAF_ACT_RELU: return x > 0.f ? x : 0.f;
         case PPOAF_ACT_LEAKY_RELU: return x > 0.f ? x : 0.01f * x;
         case PPOAF_ACT_TANH: return tanhf(x);
-        default: return x;
+        case PPOAF_ACT_IDENTITY: return x;
+        default: return act_fwd_ext(x, act);
     }
 }
-// derivative expressed through the activation OUTPUT y (sign(y) == sign(x) for relu / leaky relu)
+// derivative expressed through the activation OUTPUT y (sign(y) == sign(x) for relu / leaky relu); ids 8-11 (stored
+// derivative) pass act'(z) itself as y
 __device__ __forceinline__ float act_bwd_from_out(float y, int act) {
     switch (act) {
         case PPOAF_ACT_RELU: return y > 0.f ? 1.f : 0.f;
         case PPOAF_ACT_LEAKY_RELU: return y > 0.f ? 1.f : 0.01f;
         case PPOAF_ACT_TANH: return 1.f - y * y;
-        default: return 1.f;
+        case PPOAF_ACT_IDENTITY: return 1.f;
+        default: return act_bwd_ext(y, act);
     }
 }
 
-enum { EPI_FWD = 0, EPI_BWD_X = 1, EPI_BWD_W = 2 };
+// EPI_FWD_DACT: EPI_FWD that also stores act'(z) to GemmProblem::dact (act_stores_derivative ids, FFMA tiles only)
+enum { EPI_FWD = 0, EPI_BWD_X = 1, EPI_BWD_W = 2, EPI_FWD_DACT = 3 };
 constexpr int kMaxGroup = 6;
 
 struct GemmProblem {
     const float* A; const float* B; float* C;
     const float* bias;              // EPI_FWD: bias[n]
-    const float* aux;               // EPI_BWD_X: activation output of the layer below, aux[m*ldaux + n]
-    float* dbias;                   // EPI_BWD_W: dbias[m] = sum_r A(m, r)
+    const float* aux;               // EPI_BWD_X: activation output of the layer below, aux[m*ldaux + n] (its stored
+                                    //   act'(z) for act_stores_derivative ids)
+    union {                         // (one slot: the struct, and the launches' parameter blocks, keep their size)
+        float* dact;                // EPI_FWD_DACT: act'(z) out, dact[m*ldc + n]
+        float* dbias;               // EPI_BWD_W: dbias[m] = sum_r A(m, r)
+    };
     double* sq_out;                 // EPI_BWD_W: sq_out[tile] = sum of squares of this tile of dW (+ db), or null
     const int64_t* idxA;            // optional row indirection on A's row index
     const int64_t* idxB;            // optional row indirection on B's row index
@@ -199,7 +207,8 @@ __device__ __forceinline__ float act_fwd_fast(float x, int act) {
         case PPOAF_ACT_RELU: return x > 0.f ? x : 0.f;
         case PPOAF_ACT_LEAKY_RELU: return x > 0.f ? x : 0.01f * x;
         case PPOAF_ACT_TANH: return fast_tanh(x);
-        default: return x;
+        case PPOAF_ACT_IDENTITY: return x;
+        default: return act_fwd_ext(x, act);
     }
 }
 
@@ -249,7 +258,8 @@ __device__ __forceinline__ float4 load4_guarded(const float* p, int remaining, b
     return v;
 }
 
-template <bool A_RC, bool B_RC, int VA, int VB, int EPI>
+// EXT: the epilogues also take activation ids 4-11 (grouped_gemm_ext_kernel)
+template <bool A_RC, bool B_RC, int VA, int VB, int EPI, bool EXT>
 __device__ __forceinline__ void gemm_tile(const GemmProblem& g, int tile, const int32_t* cursor, int cursor_stride,
                                           const MirrorSet& mir, float* smem, uint64_t* bars, int* s_idx) {
     const int tid = threadIdx.x;
@@ -350,7 +360,7 @@ __device__ __forceinline__ void gemm_tile(const GemmProblem& g, int tile, const 
     const int r = tid >> 4, c4 = (tid & 15) * 4;
     const int m = m0 + r, n = n0 + c4;
     float4 epi = make_float4(0.f, 0.f, 0.f, 0.f);
-    if constexpr (EPI == EPI_FWD) {
+    if constexpr (EPI == EPI_FWD || EPI == EPI_FWD_DACT) {
         if (n < g.N) epi = load4_guarded(g.bias + n, g.N - n, reinterpret_cast<uintptr_t>(g.bias) % 16 == 0);
     }
     if constexpr (EPI == EPI_BWD_X) {
@@ -382,6 +392,7 @@ __device__ __forceinline__ void gemm_tile(const GemmProblem& g, int tile, const 
     PPOAF_STAMP(6);
 
     float sq = 0.f;
+    float d[4];                                // EPI_FWD_DACT: act'(z) of the four outputs
     if (m < g.M && n < g.N) {
         float4 sum = make_float4(0.f, 0.f, 0.f, 0.f);
         const float* rp = red + r * kRedLd + c4;
@@ -395,9 +406,16 @@ __device__ __forceinline__ void gemm_tile(const GemmProblem& g, int tile, const 
         if constexpr (EPI == EPI_FWD) {
 #pragma unroll
             for (int j = 0; j < 4; ++j) o[j] += e[j];
-            act_fwd4(o, g.act);
+            act_fwd4<EXT>(o, g.act);
         }
-        if constexpr (EPI == EPI_BWD_X) act_bwd4(o, e, g.act);
+        if constexpr (EPI == EPI_FWD_DACT) {
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const float2 yd = act_fwd_grad(o[j] + e[j], g.act);
+                o[j] = yd.x; d[j] = yd.y;
+            }
+        }
+        if constexpr (EPI == EPI_BWD_X) act_bwd4<EXT>(o, e, g.act);
         if constexpr (EPI == EPI_BWD_W) {
 #pragma unroll
             for (int j = 0; j < 4; ++j)
@@ -415,6 +433,16 @@ __device__ __forceinline__ void gemm_tile(const GemmProblem& g, int tile, const 
                     crow[n + j] = o[j];
                     if constexpr (EPI == EPI_BWD_W) mirror_store(mir, crow + n + j, o[j]);
                 }
+        }
+        if constexpr (EPI == EPI_FWD_DACT) {   // same row pitch as C
+            float* drow = g.dact + int64_t(m) * g.ldc;
+            if (g.ldc % 4 == 0 && reinterpret_cast<uintptr_t>(g.dact) % 16 == 0 && n + 3 < g.N) {
+                *reinterpret_cast<float4*>(drow + n) = make_float4(d[0], d[1], d[2], d[3]);
+            } else {
+#pragma unroll
+                for (int j = 0; j < 4; ++j)
+                    if (n + j < g.N) drow[n + j] = d[j];
+            }
         }
         if constexpr (EPI == EPI_BWD_W) {
             if (n0 == 0 && c4 == 0 && g.dbias) {
@@ -445,7 +473,12 @@ __device__ __forceinline__ void gemm_tile(const GemmProblem& g, int tile, const 
 }
 
 #ifndef PPOAF_HELPERS_ONLY   // fused_step.cu reuses the helpers above; the kernel itself lives in mlp.cu's translation unit
-__global__ void __launch_bounds__(kThreads) grouped_gemm_kernel(const GroupedGemmArgs args) {
+// Two kernels of one body.  grouped_gemm_kernel takes activation ids 0-3 only; grouped_gemm_ext_kernel takes every id
+// and the EPI_FWD_DACT epilogue.  The code of ids 4-11 in the first kernel (one call site per epilogue and four more
+// tile instantiations) cost the Tanh C4 benchmark 0.8 % on a B200 at 1000 W, so GemmGroup::launch picks the second
+// kernel only for launches that need it.
+template <bool EXT>
+__device__ __forceinline__ void grouped_gemm_body(const GroupedGemmArgs& args) {
     extern __shared__ __align__(16) float smem[];
     __shared__ __align__(8) uint64_t s_bars[kLoadGroups];
     __shared__ int s_idx[2 * kKRound];
@@ -461,7 +494,7 @@ __global__ void __launch_bounds__(kThreads) grouped_gemm_kernel(const GroupedGem
         if (i < args.n_problems && int(blockIdx.x) >= args.p[i].tile_begin) p = i;
     const GemmProblem& g = args.p[p];
     const int tile = int(blockIdx.x) - g.tile_begin;
-#define PPOAF_TILE(ARC, BRC, VA, VB, E) gemm_tile<ARC, BRC, VA, VB, E>(g, tile, args.cursor, args.cursor_stride, args.mirror, smem, s_bars, s_idx)
+#define PPOAF_TILE(ARC, BRC, VA, VB, E) gemm_tile<ARC, BRC, VA, VB, E, EXT>(g, tile, args.cursor, args.cursor_stride, args.mirror, smem, s_bars, s_idx)
 #ifdef PPOAF_GEMM_REPEAT   // debug: run the tile twice, the stamps of the second (warm instruction cache) pass survive
 #pragma unroll 1
     for (int rep = 0; rep < 2; ++rep) {
@@ -473,6 +506,10 @@ __global__ void __launch_bounds__(kThreads) grouped_gemm_kernel(const GroupedGem
         case EPI_FWD * 4 + 2: PPOAF_TILE(true, true, 4, 1, EPI_FWD); break;
         case EPI_FWD * 4 + 1: PPOAF_TILE(true, true, 1, 4, EPI_FWD); break;
         case EPI_FWD * 4 + 0: PPOAF_TILE(true, true, 1, 1, EPI_FWD); break;
+        case EPI_FWD_DACT * 4 + 3: if constexpr (EXT) { PPOAF_TILE(true, true, 4, 4, EPI_FWD_DACT); } break;
+        case EPI_FWD_DACT * 4 + 2: if constexpr (EXT) { PPOAF_TILE(true, true, 4, 1, EPI_FWD_DACT); } break;
+        case EPI_FWD_DACT * 4 + 1: if constexpr (EXT) { PPOAF_TILE(true, true, 1, 4, EPI_FWD_DACT); } break;
+        case EPI_FWD_DACT * 4 + 0: if constexpr (EXT) { PPOAF_TILE(true, true, 1, 1, EPI_FWD_DACT); } break;
         case EPI_BWD_X * 4 + 3: PPOAF_TILE(true, false, 4, 4, EPI_BWD_X); break;
         case EPI_BWD_X * 4 + 2: PPOAF_TILE(true, false, 4, 1, EPI_BWD_X); break;
         case EPI_BWD_X * 4 + 1: PPOAF_TILE(true, false, 1, 4, EPI_BWD_X); break;
@@ -487,6 +524,8 @@ __global__ void __launch_bounds__(kThreads) grouped_gemm_kernel(const GroupedGem
 #endif
 #undef PPOAF_TILE
 }
+__global__ void __launch_bounds__(kThreads) grouped_gemm_kernel(const GroupedGemmArgs args) { grouped_gemm_body<false>(args); }
+__global__ void __launch_bounds__(kThreads) grouped_gemm_ext_kernel(const GroupedGemmArgs args) { grouped_gemm_body<true>(args); }
 #endif  // PPOAF_HELPERS_ONLY
 
 }  // namespace ppoaf

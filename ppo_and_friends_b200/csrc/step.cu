@@ -50,6 +50,7 @@ int sm_count() {
 struct NetScratch {
     float* act[PPOAF_MAX_LAYERS + 1];  // act[l] = output of layer l-1 (act[0] unused: the input is gathered)
     float* dz[PPOAF_MAX_LAYERS + 1];   // dz[l]  = gradient w.r.t. the pre-activation of layer l-1's output
+    float* dact[PPOAF_MAX_LAYERS + 1]; // dact[l] = act'(z) of hidden layer l-1's output (act_stores_derivative ids), or null
 };
 struct StepScratch {
     NetScratch actor, critic;
@@ -92,6 +93,14 @@ static void carve(const ppoaf_update_cfg* cfg, int max_batch, char* base, StepSc
             ns[k]->act[l] = reinterpret_cast<float*>(take(size_t(max_batch) * nets[k]->dims[l] * sizeof(float)));
             ns[k]->dz[l] = reinterpret_cast<float*>(take(rows * nets[k]->dims[l] * sizeof(float)));
         }
+    }
+    // act'(z) of every hidden layer, for activations whose derivative cannot be recovered from their output: carved
+    // last, so every other buffer (and the workspace of the other activations) keeps its offset
+    for (int k = 0; k < 2; ++k) {
+        const bool stored = act_stores_derivative(nets[k]->activation);
+        for (int l = 0; l <= PPOAF_MAX_LAYERS; ++l) ns[k]->dact[l] = nullptr;
+        for (int l = 1; stored && l < nets[k]->n_layers; ++l)
+            ns[k]->dact[l] = reinterpret_cast<float*>(take(size_t(max_batch) * nets[k]->dims[l] * sizeof(float)));
     }
     out->total = off;
 }
@@ -233,7 +242,7 @@ extern "C" int ppoaf_ppo_minibatch_grads(const ppoaf_update_cfg* cfg, const ppoa
             grp.add_forward(first ? x0[k] : ns[k]->act[l], net[k]->dims[l], first ? b->perm : nullptr,
                             par[k] + off[k][2 * l], par[k] + off[k][2 * l + 1], ns[k]->act[l + 1], rows,
                             net[k]->dims[l], net[k]->dims[l + 1], last ? PPOAF_ACT_IDENTITY : net[k]->activation,
-                            /*w_static=*/l > 0);
+                            /*w_static=*/l > 0, last ? nullptr : ns[k]->dact[l + 1]);
         }
         PPOAF_STEP_LIMIT();
         if (grp.launch(b->mb_cursor, b->batch_size, s)) return 2;
@@ -289,6 +298,8 @@ extern "C" int ppoaf_ppo_minibatch_grads(const ppoaf_update_cfg* cfg, const ppoa
         a.b_critic = par[1] + off[1][2 * (L[1] - 1) + 1];
         a.dz_actor = sc.actor.dz[L[0] - 1];
         a.dz_critic = sc.critic.dz[L[1] - 1];
+        a.dact_actor = sc.actor.dact[L[0] - 1];
+        a.dact_critic = sc.critic.dact[L[1] - 1];
         a.Ha = cfg->actor.dims[L[0] - 1];
         a.Hc = cfg->critic.dims[L[1] - 1];
         a.act = cfg->actor.activation;
@@ -317,8 +328,8 @@ extern "C" int ppoaf_ppo_minibatch_grads(const ppoaf_update_cfg* cfg, const ppoa
                                              grd[k] + off[k][2 * l + 1], rows, net[k]->dims[l], net[k]->dims[l + 1],
                                              sq[k] + sq_used[k], /*x_static=*/!first);
             if (!first)
-                grp.add_backward_x(ns[k]->dz[l + 1], par[k] + off[k][2 * l], ns[k]->act[l], ns[k]->dz[l], rows,
-                                   net[k]->dims[l], net[k]->dims[l + 1], net[k]->activation);
+                grp.add_backward_x(ns[k]->dz[l + 1], par[k] + off[k][2 * l], ns[k]->dact[l] ? ns[k]->dact[l] : ns[k]->act[l],
+                                   ns[k]->dz[l], rows, net[k]->dims[l], net[k]->dims[l + 1], net[k]->activation);
         }
         PPOAF_STEP_LIMIT();
         if (grp.launch(b->mb_cursor, b->batch_size, s, b->n_mirror, b->mirror_delta)) return 2;

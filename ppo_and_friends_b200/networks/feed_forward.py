@@ -19,21 +19,36 @@ from torch import nn
 
 from .. import _lib, ops
 
-_ACT_NAMES = {nn.ReLU: "relu", nn.LeakyReLU: "leaky_relu", nn.Tanh: "tanh", nn.Identity: "identity"}
+_ACT_NAMES = {nn.ReLU: "relu", nn.LeakyReLU: "leaky_relu", nn.Tanh: "tanh", nn.Identity: "identity", nn.ELU: "elu",
+              nn.CELU: "elu", nn.SELU: "selu", nn.Sigmoid: "sigmoid", nn.Softplus: "softplus", nn.SiLU: "silu",
+              nn.Mish: "mish"}
+_SUPPORTED = ("ReLU, LeakyReLU(0.01), Tanh, ELU(alpha=1), CELU(alpha=1), SELU, Sigmoid, Softplus(beta=1, threshold=20), "
+              "SiLU, GELU('none' or 'tanh'), Mish")
 
 
 def activation_name(activation):
-    """Map a torch activation instance (the reference passes module instances) or a string."""
+    """Map a torch activation instance (the reference passes module instances) or a string.  The kernels carry no
+    activation parameter, so a module whose parameter differs from the one value they implement is refused."""
     if isinstance(activation, str):
         if activation not in _lib.ACT_IDS:
             raise ValueError(f"unsupported activation {activation}")
         return activation
+    if isinstance(activation, nn.GELU):
+        if activation.approximate not in ("none", "tanh"):
+            raise ValueError(f"GELU approximate={activation.approximate!r} is not supported (supported: 'none', 'tanh')")
+        return "gelu" if activation.approximate == "none" else "gelu_tanh"
     for cls, name in _ACT_NAMES.items():
         if isinstance(activation, cls):
             if cls is nn.LeakyReLU and abs(activation.negative_slope - 0.01) > 1e-12:
                 raise ValueError("LeakyReLU slope other than 0.01 is not supported by the CUDA path")
+            if cls in (nn.ELU, nn.CELU) and activation.alpha != 1.0:
+                raise ValueError(f"{cls.__name__} alpha={activation.alpha} is not supported by the CUDA path "
+                                 "(supported: alpha=1.0)")
+            if cls is nn.Softplus and (activation.beta != 1.0 or activation.threshold != 20.0):
+                raise ValueError(f"Softplus beta={activation.beta}, threshold={activation.threshold} is not supported "
+                                 "by the CUDA path (supported: beta=1.0, threshold=20.0)")
             return name
-    raise ValueError(f"unsupported activation {activation!r} (supported: ReLU, LeakyReLU(0.01), Tanh)")
+    raise ValueError(f"unsupported activation {activation!r} (supported: {_SUPPORTED})")
 
 
 def hidden_sizes(hidden_size, hidden_depth):
